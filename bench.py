@@ -15,6 +15,9 @@ accumulators) over one batch of 2^20 synthetic observations per GPU at one SNR o
              NMSE per SNR all-reduced once per sweep -- the curve the driver's 1/2/4/8 scaling run records
   cpu_baseline  the reference's own CPU implementation on the host cores (see --impl reference), bounded sample
 
+`--dump-outputs DIR` writes what the timed path computes in its last step (rank 0; see dump_outputs) as DIR/<name>.npy, for
+comparing two builds output for output: the inputs are seeded, so the same arguments give the same inputs on every run.
+
 `--impl reference` times the UNMODIFIED reference (`oracle/_ref`, vendored by oracle/build_ref.py): `Gmm_nbit.estimate_from_y`
 under the `mp.Pool(cpu_count() // 2).starmap` pattern of Bussgang_GMM.py:29-32, 282-287, plus the single-process rate and the
 numpy port (oracle) as extra figures.  Without `oracle/_ref` it times the port (`kind: "port"`).
@@ -43,6 +46,7 @@ WORKLOAD = f"Bussgang-GMM 'full' 1-bit N={N_ANT} K={N_COMP} mode=all, SNR sweep 
 C5_COMP = 256                                        # BASELINE configs[4]
 C5_GLOBAL = 1 << 23                                  # global observations per step (a stated fraction of the 1e8 of configs[4])
 REF_TASK_PILOTS = 512                                # pilots per pool task of the reference arm (prepare: 0.44 s, then ~245 est/s)
+DUMP_ROWS = 1 << 14                                  # estimates kept by --dump-outputs: 16 Ki rows of 64 complex128 = 16 MiB
 
 
 def peaks():
@@ -328,6 +332,20 @@ def pcie_peak(torch, dev, mib=256, reps=4):
     return 2 * n * reps / (time.perf_counter() - t0) / 1e9
 
 
+def dump_outputs(path, torch, model, quant, h, noise, snr, precision):
+    """The last timed step's call made once more on the same inputs, with the estimates kept (the same kernels: the timed call
+    already computes every estimate for its accumulators).  ``nmse_acc.npy`` float64 [3] holds what this one call returns, starting
+    from zero (sum |h_est - h|^2, sum |h|^2, pilots), not the timed loop's running sums; the kernels add it up with float64
+    atomics, so its last bits may depend on the order in which blocks finish.  ``h_est_sample.npy`` float64 [DUMP_ROWS, N, 2] holds
+    the real and imaginary parts of a fixed, seeded sample of rows of its estimates (the whole batch is 1 GiB)."""
+    h_est, acc = model.pipeline(quant, h, noise, 10 ** (-snr / 20), 'all', precision, want_est=True)
+    rows = np.sort(np.random.default_rng(0).choice(h_est.shape[0], min(DUMP_ROWS, h_est.shape[0]), replace=False))
+    sample = torch.view_as_real(h_est[torch.as_tensor(rows, device=h_est.device)])
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, 'nmse_acc.npy'), acc.cpu().numpy())
+    np.save(os.path.join(path, 'h_est_sample.npy'), sample.cpu().numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
@@ -340,8 +358,13 @@ def main():
     ap.add_argument('--no-e2e', action='store_true')
     ap.add_argument('--no-config5', action='store_true')
     ap.add_argument('--sustain-seconds', type=float, default=2.0)
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the outputs of the last timed step as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
+        if args.dump_outputs:
+            ap.error('--dump-outputs needs --impl b200')
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
 
@@ -552,6 +575,10 @@ def main():
     cpu = None
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         cpu = cpu_baseline_subprocess()
+
+    if args.dump_outputs and rank == 0:
+        j = (args.steps - 1) % len(SNRS)
+        dump_outputs(args.dump_outputs, torch, models[j], quant, h, noise, SNRS[j], args.precision)
 
     if rank == 0:
         nmse = {str(s): float(a[0] / max(a[2], 1) / N_ANT) for s, a in zip(SNRS, accs) if a[2] > 0}
