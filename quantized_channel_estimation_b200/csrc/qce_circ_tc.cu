@@ -27,6 +27,7 @@ namespace qce {
 namespace {
 
 constexpr int CT_P = 32;             // pilots per CTA
+constexpr int CT_NW = 8;             // warps per CTA (16 warps with 64 registers each measured 7 % slower)
 constexpr int CT_N = 256;            // bins (16 x 16)
 constexpr int CT_EP = CT_N + 8;      // pitch (halves) of the |rt|^2 operand rows: 528 B = odd multiple of 16 B (ldmatrix conflict-free)
 constexpr int CT_R_BYTES = 34816;    // operand region: E hi/lo, later log-probabilities | weight hi/lo
@@ -115,11 +116,11 @@ __device__ __forceinline__ void split_half(const float x, __half& hi, __half& lo
     lo = __float2half_rn(x - __half2float(hi));
 }
 
-// KC = K / 64.  NW warps per CTA: GEMM 1 gives each warp G1NB = K / (8 NW) blocks of 8 components, GEMM 2 G2NB = 32 / NW blocks
-// of 8 bins; the FFT phases run 512 / (32 NW) transforms per thread.
-template <int KC, int NW>
-__global__ void __launch_bounds__(32 * NW, 2) circ_tc_kernel(const CircTcArgs a) {
-    constexpr int K = 64 * KC, NT = 32 * NW, NJ = 512 / NT, KNB = K / (8 * NW), G2NB = 32 / NW, SPW = CT_P / NW;
+// KC = K / 64.  CT_NW warps per CTA: GEMM 1 gives each warp KNB = K / (8 CT_NW) blocks of 8 components, GEMM 2 G2NB = 32 / CT_NW
+// blocks of 8 bins; the FFT phases run 512 / (32 CT_NW) transforms per thread.
+template <int KC>
+__global__ void __launch_bounds__(32 * CT_NW, 2) circ_tc_kernel(const CircTcArgs a) {
+    constexpr int K = 64 * KC, NT = 32 * CT_NW, NJ = 512 / NT, KNB = K / (8 * CT_NW), G2NB = 32 / CT_NW, SPW = CT_P / CT_NW;
     static_assert(KNB >= 1 && G2NB >= 1 && NJ >= 1 && SPW >= 1, "warp split");
     constexpr int LP = K + 4;                  // pitch (floats) of the log-probability rows
     constexpr int WP = K + 8;                  // pitch (halves) of the weight operand rows
@@ -482,483 +483,6 @@ __global__ void __launch_bounds__(32 * NW, 2) circ_tc_kernel(const CircTcArgs a)
     }
 }
 
-// ================================================================================================ tcgen05 version
-// The same algorithm with the two [N x K] contractions on the 5th-generation tensor cores.  ncu on the mma.sync kernel above
-// (profiles/r01_circ_tc_final_ncu_summary.txt): L1TEX is the busiest unit (66 %), and 43 % of its traffic is operand delivery to
-// mma.sync -- every warp re-reads the whole |rt|^2 operand with ldmatrix and pulls its parameter fragments through L1.  tcgen05.mma
-// reads both operands straight from shared memory (once per MMA, not once per warp), the parameters arrive by bulk-TMA without
-// touching L1 or registers, and the accumulators live in TMEM.  Layout of the problem on the MMA (cta_group::1, M = 128):
-//     GEMM 1   D1[comp, pilot]  = P1[comp, bin]  * E[pilot, bin]^T      M = 128 components (zero rows above K), N = 64 pilots
-//     GEMM 2   D2[bin,  pilot]  = P2[bin,  comp] * W[pilot, comp]^T     2 x (M = 128 bins), N = 64 pilots
-// i.e. the PILOTS are the N dimension: the CTA tile is 32 pilots, the parameters are the A operand (streamed in 8 KB chunks = one
-// k-step, FP16 hi then lo, through a ring by one producer thread from the start of the CTA), the computed operands E = |rt|^2 and
-// W = weights are the B operand, written by the FFT / softmax threads in the canonical K-major core-matrix order (FP16 hi, lo:
-// three passes hi*hi + lo*hi + hi*lo as before).  rt itself -- 2 KB per pilot that has to survive from the forward to the inverse
-// transform -- moves out of shared memory into TMEM (tcgen05.st / ld by the thread that owns the row: 128 columns x 128 lanes x 4 B
-// = 64 KB), and the transposes between the two FFT axes go through a tile of 16 pilots that every warp uses for its own two
-// pilots, twice.  101 KB of shared memory and 256 TMEM columns per CTA: two CTAs per SM overlap each other's waits (a first
-// version with one 64-pilot CTA per SM spent 20 % of its time waiting for the two GEMMs and 17 % in exposed load latency:
-// 292 M estimates/s against 369 M of the mma.sync kernel, profiles/r02_circ_umma_v1_ncu_summary.txt).  10 warps: 8 for the
-// transforms / epilogues, one MMA issuer, one TMA producer.
-__device__ __forceinline__ int circ_bin_of(int s, int one_d);
-constexpr int CU_P = 32;                         // pilots per CTA
-constexpr int CU_CW = 8;                         // compute warps
-constexpr int CU_NT = 32 * CU_CW;                // compute threads
-constexpr int CU_THREADS = CU_NT + 64;           // + MMA issuer warp + producer warp
-constexpr int CU_XP = CT_N + 8;                  // pitch (float2) of a pilot's tile of the transposes
-constexpr int CU_XROWS = 2 * CU_CW;              // pilots in the transpose tile: two per warp (one round of the two)
-constexpr int CU_X_BYTES = CU_XROWS * CU_XP * 8; // 33792
-constexpr int CU_E_LBO = (CU_P / 8) * 128 + 16;  // K-direction core stride of the E operand (16 B of padding: the 16 row owners of a
-                                                 // pilot write cores 1 KB apart, which would all hit the same banks)
-constexpr int CU_E_COPY = 32 * CU_E_LBO;         // bytes of one copy (hi or lo) of E: 32 K-cores x (4 pilot-cores x 128 B + pad)
-constexpr int CU_R_BYTES = 2 * CU_E_COPY;        // 33792: E hi | E lo, later log-probabilities | W hi | W lo, later G
-constexpr int CU_W_LBO = (CU_P / 8) * 128;
-constexpr int CU_GP = CT_N + 4;                  // pitch (floats) of the per-bin gains G[pilot][bin]
-constexpr int CU_CHUNK = 8192;                   // one k-step of a parameter operand: [128 x 16] FP16 hi, then lo
-constexpr int CU_RING = 4;                       // dedicated ring stages (filled from the start of the CTA) ...
-constexpr int CU_STAGES = 8;                     // ... plus four in the transpose tile, which is dead between the forward and the inverse
-                                                 // transforms (with 4 stages the refill latency of the ring, ~200 clk per chunk, made
-                                                 // the two GEMMs 3 us of waiting per tile)
-constexpr int CU_SMEM = CU_X_BYTES + CU_R_BYTES + CU_RING * CU_CHUNK + 2048;
-static_assert((CU_STAGES - CU_RING) * CU_CHUNK <= CU_X_BYTES, "extra ring stages inside the transpose tile");
-constexpr int CU_TMEM_COLS = 256;                // D1 [0, 32)  D2 [32, 96)  rt [128, 256)
-static_assert(CU_P * CU_GP * 4 <= CU_R_BYTES, "G tile");
-static_assert(2 * CU_SMEM <= 227 * 1024, "two CTAs per SM");
-
-struct CircUmmaCtrl {
-    uint64_t full[CU_STAGES], empty[CU_STAGES];
-    uint64_t e_ready, w_ready, d1_full, d2_full;
-    uint32_t tmem_base, pad;
-    float invsc[CU_P], qref[CU_P];
-    double red[2];
-    int tief[CU_P];
-};
-static_assert(sizeof(CircUmmaCtrl) <= 2048, "control block");
-
-__device__ __forceinline__ void cu_sync() { asm volatile("bar.sync 1, %0;" ::"n"(CU_NT) : "memory"); }
-__device__ __forceinline__ void tmem_st32(uint32_t taddr, const float (&v)[32]) {
-    const uint32_t* u = reinterpret_cast<const uint32_t*>(v);
-    asm volatile(
-        "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
-        "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
-        "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};"
-        ::"r"(taddr), "r"(u[0]), "r"(u[1]), "r"(u[2]), "r"(u[3]), "r"(u[4]), "r"(u[5]), "r"(u[6]), "r"(u[7]), "r"(u[8]), "r"(u[9]), "r"(u[10]),
-          "r"(u[11]), "r"(u[12]), "r"(u[13]), "r"(u[14]), "r"(u[15]), "r"(u[16]), "r"(u[17]), "r"(u[18]), "r"(u[19]), "r"(u[20]), "r"(u[21]),
-          "r"(u[22]), "r"(u[23]), "r"(u[24]), "r"(u[25]), "r"(u[26]), "r"(u[27]), "r"(u[28]), "r"(u[29]), "r"(u[30]), "r"(u[31])
-        : "memory");
-}
-__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
-    uint32_t* u = reinterpret_cast<uint32_t*>(v);
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-        : "=r"(u[0]), "=r"(u[1]), "=r"(u[2]), "=r"(u[3]), "=r"(u[4]), "=r"(u[5]), "=r"(u[6]), "=r"(u[7]), "=r"(u[8]), "=r"(u[9]), "=r"(u[10]),
-          "=r"(u[11]), "=r"(u[12]), "=r"(u[13]), "=r"(u[14]), "=r"(u[15])
-        : "r"(taddr)
-        : "memory");
-}
-
-struct CircUmmaArgs {
-    CircTcArgs t;                    // the common arguments (b1 / b2 unused)
-    const unsigned char* img;        // GEMM 1 chunks [16][hi 4 KB | lo 4 KB], then GEMM 2 chunks [K / 16][2 halves][hi | lo]
-    long long* prof;                 // QCE_CIRC_PROF=1: phase time stamps of one CTA (thread 0), else null
-};
-#define CU_STAMP(i) do { if (ua.prof && tid == 0 && blockIdx.x == gridDim.x / 2) ua.prof[i] = clock64(); } while (0)
-
-template <int KC>      // K = 64 KC components
-__global__ void __launch_bounds__(CU_THREADS, 2) circ_umma_kernel(const CircUmmaArgs ua) {
-    const CircTcArgs& a = ua.t;
-    constexpr int K = 64 * KC, LP = K + 4, NJ = CU_P * 16 / CU_NT, SPW = CU_P / CU_CW;
-    static_assert(NJ == 2 && CU_XROWS * NJ == CU_P, "two rounds: a warp owns two pilots per round");
-    constexpr int N1 = CT_N / 16, N2 = 2 * (K / 16);                      // chunks of GEMM 1 / GEMM 2
-    static_assert(CU_P * LP * 4 + 2 * (K / 8) * CU_W_LBO <= CU_R_BYTES, "log-probabilities + W operand");
-    extern __shared__ __align__(1024) unsigned char smem_raw[];
-    float2* X = reinterpret_cast<float2*>(smem_raw);                       // transpose tile (16 pilots: every warp its own two)
-    unsigned char* R = smem_raw + CU_X_BYTES;
-    unsigned char* ring = R + CU_R_BYTES;
-    unsigned char* Ehi = R;
-    unsigned char* Elo = R + CU_E_COPY;
-    float* lbuf = reinterpret_cast<float*>(R);
-    unsigned char* Whi = R + CU_P * LP * 4;
-    unsigned char* Wlo = Whi + (K / 8) * CU_W_LBO;
-    float* G = reinterpret_cast<float*>(R);
-    CircUmmaCtrl* ctrl = reinterpret_cast<CircUmmaCtrl*>(ring + CU_RING * CU_CHUNK);
-    auto stage_ptr = [&](int st) { return st < CU_RING ? ring + st * CU_CHUNK : smem_raw + (st - CU_RING) * CU_CHUNK; };
-
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int64_t base = (int64_t)blockIdx.x * CU_P;
-    const int nvalid = (int)((a.B - base) < CU_P ? (a.B - base) : CU_P);
-    if (tid == 0) {
-        for (int i = 0; i < CU_STAGES; ++i) { mbar_init(smem_u32(&ctrl->full[i]), 1); mbar_init(smem_u32(&ctrl->empty[i]), 1); }
-        mbar_init(smem_u32(&ctrl->e_ready), CU_CW);
-        mbar_init(smem_u32(&ctrl->w_ready), CU_CW);
-        mbar_init(smem_u32(&ctrl->d1_full), 1);
-        mbar_init(smem_u32(&ctrl->d2_full), 1);
-        ctrl->red[0] = ctrl->red[1] = 0.0;
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == CU_CW) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&ctrl->tmem_base)), "r"(CU_TMEM_COLS) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = ctrl->tmem_base;
-    constexpr uint32_t DESC_HI = (128u >> 4) | (1u << 14);
-    constexpr uint32_t IDESC = (1u << 4) | ((uint32_t)(CU_P >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-
-    if (warp == CU_CW + 1) {
-        // ===================== producer: the parameter chunks of both GEMMs through the ring, from the start of the CTA (the first
-        // stages are in shared memory long before the forward transforms are done)
-        if (lane == 0) {
-            for (int c = 0; c < N1 + N2; ++c) {
-                const int st = c % CU_STAGES;
-                if (c == CU_RING) mbar_wait(smem_u32(&ctrl->e_ready), 0);      // the stages in the transpose tile: after the forward transforms
-                mbar_wait(smem_u32(&ctrl->empty[st]), ((c / CU_STAGES) & 1) ^ 1);
-                mbar_expect_tx(smem_u32(&ctrl->full[st]), CU_CHUNK);
-                bulk_g2s(smem_u32(stage_ptr(st)), ua.img + (size_t)c * CU_CHUNK, CU_CHUNK, smem_u32(&ctrl->full[st]));
-            }
-        }
-    } else if (warp == CU_CW) {
-        // ===================== MMA issuer
-        const bool elected = elect_one();
-        const uint32_t a_lbo = ((16u * 128u) >> 4) << 16;                 // [128 x 16] chunk: the two K-cores are 2 KB apart
-        mbar_wait(smem_u32(&ctrl->e_ready), 0);
-        tc_fence_after();
-        for (int c = 0; c < N1 + N2; ++c) {
-            if (c == N1) { mbar_wait(smem_u32(&ctrl->w_ready), 0); tc_fence_after(); }
-            const int st = c % CU_STAGES;
-            mbar_wait(smem_u32(&ctrl->full[st]), (c / CU_STAGES) & 1);
-            tc_fence_after();
-            const uint32_t st_a = (smem_u32(stage_ptr(st)) >> 4) & 0x3FFF;
-            const uint32_t a_hi = st_a | a_lbo, a_lo = (st_a + (4096 >> 4)) | a_lbo;
-            uint32_t b_hi, b_lo, d;
-            bool first;
-            if (c < N1) {
-                b_hi = (((smem_u32(Ehi) + 2 * c * CU_E_LBO) >> 4) & 0x3FFF) | ((uint32_t)(CU_E_LBO >> 4) << 16);
-                b_lo = (((smem_u32(Elo) + 2 * c * CU_E_LBO) >> 4) & 0x3FFF) | ((uint32_t)(CU_E_LBO >> 4) << 16);
-                d = tmem_base;
-                first = c == 0;
-            } else {
-                const int ks = (c - N1) >> 1, h = (c - N1) & 1;
-                b_hi = (((smem_u32(Whi) + 2 * ks * CU_W_LBO) >> 4) & 0x3FFF) | ((uint32_t)(CU_W_LBO >> 4) << 16);
-                b_lo = (((smem_u32(Wlo) + 2 * ks * CU_W_LBO) >> 4) & 0x3FFF) | ((uint32_t)(CU_W_LBO >> 4) << 16);
-                d = tmem_base + CU_P + CU_P * h;
-                first = ks == 0;
-            }
-            if (elected) {
-                umma_f16(d, a_hi, b_hi, DESC_HI, IDESC, first ? 0u : 1u);
-                umma_f16(d, a_lo, b_hi, DESC_HI, IDESC, 1u);
-                umma_f16(d, a_hi, b_lo, DESC_HI, IDESC, 1u);
-                tc_commit(smem_u32(&ctrl->empty[st]));
-                if (c == N1 - 1) tc_commit(smem_u32(&ctrl->d1_full));
-                if (c == N1 + N2 - 1) tc_commit(smem_u32(&ctrl->d2_full));
-            }
-            __syncwarp();
-        }
-        mbar_wait(smem_u32(&ctrl->d2_full), 0);      // (TMEM is released below: not before the last MMA has retired)
-    } else {
-        // ===================== compute warps
-        const uint32_t t_rt = tmem_base + ((uint32_t)((warp & 3) * 32) << 16) + 128 + 64 * (warp >> 2);
-        if (tid == 0) {      // pull the pilots of the tile one wave of CTAs ahead into L2
-            const int64_t pb = base + (int64_t)a.prefetch_dist * CU_P;
-            if (pb < a.B) {
-                const int64_t np = (a.B - pb) < CU_P ? (a.B - pb) : CU_P;
-                asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(a.r + pb * CT_N), "r"((uint32_t)(np * CT_N * sizeof(double2))) : "memory");
-                if (a.acc && a.h_true)
-                    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(a.h_true + pb * CT_N), "r"((uint32_t)(np * CT_N * sizeof(double2))) : "memory");
-            }
-        }
-        // (pl: the pilot's slot in the transpose tile; both rounds of a warp use the same two slots, which no other warp touches)
-        auto xidx = [](int pl, int ar, int b) { return pl * CU_XP + ar * 16 + ((((b >> 1) ^ (ar & 7)) << 1) | (b & 1)); };
-        const int pl = tid >> 4;
-        CU_STAMP(0);
-
-        #pragma unroll
-        for (int j = 0; j < NJ; ++j) {
-        // ---- load (coalesced) + forward FFT along the block axis
-        {
-            const int idx = tid + CU_NT * j, p = idx >> 4, b = idx & 15;
-            float2 v[16];
-            if (p < nvalid) {
-                const double2* src = a.r + ((base + p) * CT_N + b);
-                #pragma unroll
-                for (int ar = 0; ar < 16; ++ar) { const double2 d = __ldcs(src + ar * 16); v[ar] = make_float2((float)d.x, (float)d.y); }
-            } else {
-                #pragma unroll
-                for (int ar = 0; ar < 16; ++ar) v[ar] = make_float2(0.f, 0.f);
-            }
-            fft16<false>(v);
-            if (a.tw256) {
-                #pragma unroll
-                for (int ar = 1; ar < 16; ++ar) {
-                    const float2 w = __ldg(a.tw256 + ((b * ar) & 255));
-                    v[ar] = make_float2(v[ar].x * w.x - v[ar].y * w.y, v[ar].x * w.y + v[ar].y * w.x);
-                }
-            }
-            #pragma unroll
-            for (int ar = 0; ar < 16; ++ar) X[xidx(pl, ar, b)] = v[ar];
-        }
-        __syncwarp();
-        CU_STAMP(8 + 2 * j);
-
-        // ---- forward FFT along the contiguous axis; rt -> TMEM; |rt|^2 -> E operand (FP16 hi, lo, per-pilot scale)
-        {
-            const int idx = tid + CU_NT * j, p = idx >> 4, ar = idx & 15;
-            float2 v[16];
-            const float4* row = reinterpret_cast<const float4*>(X + pl * CU_XP + ar * 16);
-            #pragma unroll
-            for (int c = 0; c < 8; ++c) { const float4 q = row[c ^ (ar & 7)]; v[2 * c] = make_float2(q.x, q.y); v[2 * c + 1] = make_float2(q.z, q.w); }
-            fft16<false>(v);
-            {
-                float f[32];
-                #pragma unroll
-                for (int b = 0; b < 16; ++b) { f[2 * b] = v[b].x; f[2 * b + 1] = v[b].y; }
-                tmem_st32(t_rt + 32 * j, f);
-            }
-            float e[16], psum = 0.f, qr = 0.f;
-            #pragma unroll
-            for (int b = 0; b < 16; ++b) { e[b] = v[b].x * v[b].x + v[b].y * v[b].y; psum += e[b]; qr = fmaf(e[b], __ldg(a.ilbar + ar * 16 + b), qr); }
-            #pragma unroll
-            for (int off = 8; off > 0; off >>= 1) {
-                psum += __shfl_xor_sync(0xffffffffu, psum, off);
-                qr += __shfl_xor_sync(0xffffffffu, qr, off);
-            }
-            if (ar == 0) ctrl->qref[p] = qr;
-            int ex = 0;
-            float sc = 1.f;
-            if (psum > 0.f && psum < 3.0e38f) { frexpf(psum, &ex); sc = ldexpf(1.f, 14 - ex); }
-            if (ar == 0) ctrl->invsc[p] = 1.f / sc;
-            uint32_t hi2[8], lo2[8];
-            #pragma unroll
-            for (int c = 0; c < 8; ++c) {
-                __half h0, l0, h1, l1;
-                split_half(e[2 * c] * sc, h0, l0);
-                split_half(e[2 * c + 1] * sc, h1, l1);
-                hi2[c] = (uint32_t)__half_as_ushort(h0) | ((uint32_t)__half_as_ushort(h1) << 16);
-                lo2[c] = (uint32_t)__half_as_ushort(l0) | ((uint32_t)__half_as_ushort(l1) << 16);
-            }
-            // bins 16 ar .. 16 ar + 15 of pilot p: K-cores 2 ar and 2 ar + 1, pilot-core p / 8, row p % 8
-            const int off0 = (2 * ar) * CU_E_LBO + (p >> 3) * 128 + (p & 7) * 16;
-            *reinterpret_cast<uint4*>(Ehi + off0) = make_uint4(hi2[0], hi2[1], hi2[2], hi2[3]);
-            *reinterpret_cast<uint4*>(Ehi + off0 + CU_E_LBO) = make_uint4(hi2[4], hi2[5], hi2[6], hi2[7]);
-            *reinterpret_cast<uint4*>(Elo + off0) = make_uint4(lo2[0], lo2[1], lo2[2], lo2[3]);
-            *reinterpret_cast<uint4*>(Elo + off0 + CU_E_LBO) = make_uint4(lo2[4], lo2[5], lo2[6], lo2[7]);
-        }
-        __syncwarp();                          // the tile slots are rewritten by the next round
-        CU_STAMP(9 + 2 * j);
-        }
-        tmem_st_wait();
-        fence_proxy_async();                   // the E operand was written through the generic proxy; the MMAs read it through the async proxy
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(smem_u32(&ctrl->e_ready));
-        CU_STAMP(1);
-
-        // ---- epilogue of GEMM 1: D1[comp, pilot] -> log-probabilities (relative to q_ref and max logc, as in the mma.sync kernel)
-        mbar_wait(smem_u32(&ctrl->d1_full), 0);
-        tc_fence_after();
-        CU_STAMP(2);
-        {
-            const int q = warp & 3, cb = warp >> 2;          // TMEM lane quadrant = components 32 q .., pilots 16 cb ..
-            if (32 * q < K) {
-                float acc[16];
-                tmem_ld16(tmem_base + ((uint32_t)(q * 32) << 16) + 16 * cb, acc);
-                tmem_ld_wait();
-                const int k = 32 * q + lane;
-                const float2 lc = __ldg(a.logc2 + k);
-                #pragma unroll
-                for (int c = 0; c < 16; ++c) {
-                    const int p = 16 * cb + c;
-                    const float sp = ctrl->invsc[p] * a.inv_s1;          // a power of two: the product is exact
-                    lbuf[p * LP + k] = (lc.x - acc[c] * sp) + lc.y;
-                }
-            }
-        }
-        tc_fence_before();
-        cu_sync();
-
-        // ---- combination weights per pilot -> W operand
-        if (a.logp_out) {
-            for (int o = tid; o < nvalid * K; o += CU_NT) a.logp_out[base * K + o] = (double)lbuf[(o / K) * LP + (o % K)] + (a.logc_max - (double)ctrl->qref[o / K]);
-            cu_sync();
-        }
-        auto w_off = [](int p, int k) { return (k >> 3) * CU_W_LBO + (p >> 3) * 128 + (p & 7) * 16 + (k & 7) * 2; };
-        if (a.mode == QCE_MODE_ALL) {
-            #pragma unroll
-            for (int pp = 0; pp < SPW; ++pp) {
-                const int p = warp * SPW + pp;
-                float v[K / 32], mx = -INFINITY;
-                #pragma unroll
-                for (int j = 0; j < K / 32; ++j) { v[j] = lbuf[p * LP + lane + 32 * j]; mx = fmaxf(mx, v[j]); }
-                #pragma unroll
-                for (int off = 16; off > 0; off >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, off));
-                float sum = 0.f;
-                #pragma unroll
-                for (int j = 0; j < K / 32; ++j) { v[j] = __expf(v[j] - mx); sum += v[j]; }
-                #pragma unroll
-                for (int off = 16; off > 0; off >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, off);
-                const float inv = CT_WSCALE / sum;
-                #pragma unroll
-                for (int j = 0; j < K / 32; ++j) {
-                    __half hi, lo;
-                    split_half(v[j] * inv, hi, lo);
-                    *reinterpret_cast<__half*>(Whi + w_off(p, lane + 32 * j)) = hi;
-                    *reinterpret_cast<__half*>(Wlo + w_off(p, lane + 32 * j)) = lo;
-                }
-            }
-        } else {
-            if (tid < CU_P) {
-                bool tie = false;
-                weights_from_logp(lbuf + tid * LP, K, a.mode, a.n_top, a.rho, a.flags, &tie, a.tie_eps);
-                tie = tie && tid < nvalid;
-                ctrl->tief[tid] = tie;
-                if (tie) a.fix_buf[2 + atomicAdd(a.fix_buf, 1)] = (int)(base + tid);
-            }
-            cu_sync();
-            for (int o = tid; o < CU_P * K; o += CU_NT) {
-                const int p = o / K, k = o % K;
-                __half hi, lo;
-                split_half(lbuf[p * LP + k] * CT_WSCALE, hi, lo);
-                *reinterpret_cast<__half*>(Whi + w_off(p, k)) = hi;
-                *reinterpret_cast<__half*>(Wlo + w_off(p, k)) = lo;
-            }
-        }
-        fence_proxy_async();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(smem_u32(&ctrl->w_ready));
-        CU_STAMP(3);
-
-        if (a.h_est || a.acc) {
-            // ---- epilogue of GEMM 2: D2[bin, pilot] -> G[pilot][bin] (the log-probabilities and W are dead once the MMAs have completed)
-            mbar_wait(smem_u32(&ctrl->d2_full), 0);
-            tc_fence_after();
-            CU_STAMP(4);
-            {
-                const int q = warp & 3, h = warp >> 2;      // bins 128 h + 32 q .., all 32 pilots
-                float acc[32];
-                tmem_ld32(tmem_base + ((uint32_t)(q * 32) << 16) + CU_P + CU_P * h, acc);
-                tmem_ld_wait();
-                const float gs = a.inv_s2 / CT_WSCALE;
-                const int bin = 128 * h + 32 * q + lane;
-                #pragma unroll
-                for (int c = 0; c < 32; ++c) G[c * CU_GP + bin] = acc[c] * gs;
-            }
-            tc_fence_before();
-            cu_sync();
-            CU_STAMP(5);
-
-            float errf = 0.f, pwf = 0.f;
-            #pragma unroll
-            for (int j = 0; j < NJ; ++j) {
-            // ---- rt <- G .* rt (rt back from TMEM), inverse FFT along the contiguous axis
-            {
-                const int idx = tid + CU_NT * j, p = idx >> 4, ar = idx & 15;
-                float f[32];
-                tmem_ld32(t_rt + 32 * j, f);
-                tmem_ld_wait();
-                float2 v[16];
-                const float4* g4 = reinterpret_cast<const float4*>(G + p * CU_GP + ar * 16);
-                #pragma unroll
-                for (int c = 0; c < 4; ++c) {
-                    const float4 g = g4[c];
-                    v[4 * c] = make_float2(f[8 * c] * g.x, f[8 * c + 1] * g.x);
-                    v[4 * c + 1] = make_float2(f[8 * c + 2] * g.y, f[8 * c + 3] * g.y);
-                    v[4 * c + 2] = make_float2(f[8 * c + 4] * g.z, f[8 * c + 5] * g.z);
-                    v[4 * c + 3] = make_float2(f[8 * c + 6] * g.w, f[8 * c + 7] * g.w);
-                }
-                fft16<true>(v);
-                float4* row = reinterpret_cast<float4*>(X + pl * CU_XP + ar * 16);
-                #pragma unroll
-                for (int c = 0; c < 8; ++c) row[c ^ (ar & 7)] = make_float4(v[2 * c].x, v[2 * c].y, v[2 * c + 1].x, v[2 * c + 1].y);
-            }
-            __syncwarp();
-
-            // ---- inverse FFT along the block axis fused into the (coalesced) store, NMSE accumulators
-            {
-                const int idx = tid + CU_NT * j, p = idx >> 4, b = idx & 15;
-                float2 v[16];
-                #pragma unroll
-                for (int ar = 0; ar < 16; ++ar) v[ar] = X[xidx(pl, ar, b)];
-                if (a.tw256) {
-                    #pragma unroll
-                    for (int ar = 1; ar < 16; ++ar) {
-                        const float2 w = __ldg(a.tw256 + ((b * ar) & 255));
-                        v[ar] = make_float2(v[ar].x * w.x + v[ar].y * w.y, v[ar].y * w.x - v[ar].x * w.y);
-                    }
-                }
-                fft16<true>(v);
-                if (p < nvalid && !(a.mode != QCE_MODE_ALL && ctrl->tief[p])) {
-                    const size_t o = (size_t)(base + p) * CT_N + b;
-                    if (a.h_est) {
-                        #pragma unroll
-                        for (int ar = 0; ar < 16; ++ar) __stcs(a.h_est + o + ar * 16, make_double2((double)v[ar].x, (double)v[ar].y));
-                    }
-                    if (a.acc && a.h_true) {
-                        #pragma unroll
-                        for (int ar = 0; ar < 16; ++ar) {
-                            const double2 h = __ldcs(a.h_true + o + ar * 16);
-                            const float hx = (float)h.x, hy = (float)h.y, dx = v[ar].x - hx, dy = v[ar].y - hy;
-                            errf = fmaf(dx, dx, fmaf(dy, dy, errf));
-                            pwf = fmaf(hx, hx, fmaf(hy, hy, pwf));
-                        }
-                    }
-                }
-            }
-            __syncwarp();                      // the tile slots are rewritten by the next round
-            }
-            CU_STAMP(6);
-            if (a.acc) {
-                double err = (double)errf, pw = (double)pwf;
-                #pragma unroll
-                for (int off = 16; off > 0; off >>= 1) {
-                    err += __shfl_xor_sync(0xffffffffu, err, off);
-                    pw += __shfl_xor_sync(0xffffffffu, pw, off);
-                }
-                if (lane == 0) { atomicAdd(&ctrl->red[0], err); atomicAdd(&ctrl->red[1], pw); }
-                cu_sync();
-                if (tid == 0) {
-                    int cnt = nvalid;
-                    if (a.mode != QCE_MODE_ALL) for (int p = 0; p < nvalid; ++p) cnt -= ctrl->tief[p];
-                    atomicAdd(a.acc + 0, ctrl->red[0]); atomicAdd(a.acc + 1, ctrl->red[1]); atomicAdd(a.acc + 2, (double)cnt);
-                }
-            }
-        }
-    }
-    __syncwarp();
-    tc_fence_before();
-    __syncthreads();
-    if (warp == CU_CW) {
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(CU_TMEM_COLS) : "memory");
-    }
-}
-
-// parameter chunks of circ_umma_kernel: [128 rows x 16] FP16 in the canonical K-major core-matrix order (core (mb, kb) at
-// ((kb * 16) + mb) * 128 B), hi 4 KB then lo 4 KB per chunk.  GEMM 1 chunk ks: row = component (zero above K), column = bin
-// 16 ks + kk (storage order of the bins, see circ_bin_of), value (1 / lambda - mean over the components) * s1.  GEMM 2 chunk
-// (ks, h): row = bin 128 h + r, column = component 16 ks + kk, value gain * s2.
-__global__ void circ_umma_pack_kernel(const double* __restrict__ inv_lambda_t, const double* __restrict__ gain, const float* __restrict__ ilbar,
-                                      int K, int one_d, double s1, double s2, unsigned char* __restrict__ img) {
-    const int n1 = CT_N / 16, n2 = 2 * (K / 16);
-    const int idx = blockIdx.x * blockDim.x + threadIdx.x;             // one thread per (chunk, row, kk)
-    if (idx >= (n1 + n2) * 128 * 16) return;
-    const int c = idx / 2048, r = (idx >> 4) & 127, kk = idx & 15;
-    double x = 0.0;
-    if (c < n1) {
-        const int s = 16 * c + kk;
-        if (r < K) x = (inv_lambda_t[(size_t)circ_bin_of(s, one_d) * K + r] - (double)ilbar[s]) * s1;
-    } else {
-        const int ks = (c - n1) >> 1, h = (c - n1) & 1, s = 128 * h + r, k = 16 * ks + kk;
-        x = gain[(size_t)k * CT_N + circ_bin_of(s, one_d)] * s2;
-    }
-    const __half hi = __double2half(x), lo = __double2half(x - (double)__half2float(hi));
-    const size_t off = (size_t)c * CU_CHUNK + ((size_t)((kk >> 3) * 16 + (r >> 3)) * 64 + (r & 7) * 8 + (kk & 7)) * 2;
-    *reinterpret_cast<__half*>(img + off) = hi;
-    *reinterpret_cast<__half*>(img + off + 4096) = lo;
-}
-
 // Constant operands in mma.m16n8k16 B-fragment order.  Thread (g = lane / 4, t = lane % 4) of block (nb, ks) holds
 // b0 = {B[16 ks + 2t][8 nb + g], B[16 ks + 2t + 1][.]}, b1 = the same 8 rows further; stored as uint4 {b0 hi, b1 hi, b0 lo, b1 lo}.
 // which = 0: B[i][k] = 1 / lambda (source inv_lambda_t [N][K]),  which = 1: B[k][i] = gain (source gain [K][N]).
@@ -1033,8 +557,8 @@ bool circ_tc_shape_ok(const qce_circ_model* m) {     // block-circulant 16 x 16,
 }
 
 void circ_tc_free(qce_circ_model* m) {
-    cudaFree(m->tc_b1); cudaFree(m->tc_b2); cudaFree(m->tc_logc2); cudaFree(m->tc_ilbar); cudaFree(m->tc_tw); cudaFree(m->tc_umma);
-    m->tc_b1 = m->tc_b2 = m->tc_logc2 = m->tc_ilbar = m->tc_tw = m->tc_umma = nullptr;
+    cudaFree(m->tc_b1); cudaFree(m->tc_b2); cudaFree(m->tc_logc2); cudaFree(m->tc_ilbar); cudaFree(m->tc_tw);
+    m->tc_b1 = m->tc_b2 = m->tc_logc2 = m->tc_ilbar = m->tc_tw = nullptr;
     m->tc_ready = false;
 }
 
@@ -1054,7 +578,6 @@ qce_status circ_tc_pack(qce_circ_model* m, cudaStream_t s) {
         QCE_CUDA_TRY(cudaMalloc(&m->tc_b2, frag_bytes));
         QCE_CUDA_TRY(cudaMalloc(&m->tc_logc2, K * sizeof(float2)));
         QCE_CUDA_TRY(cudaMalloc(&m->tc_ilbar, N * sizeof(float)));
-        QCE_CUDA_TRY(cudaMalloc(&m->tc_umma, (size_t)(CT_N / 16 + 2 * (K / 16)) * CU_CHUNK));
     }
     const int one_d = m->n1 == 1;
     if (one_d && !m->tc_tw) {
@@ -1069,12 +592,6 @@ qce_status circ_tc_pack(qce_circ_model* m, cudaStream_t s) {
     QCE_CHECK_LAUNCH("circ_tc_pack_kernel");
     circ_tc_pack_kernel<<<(total + 255) / 256, 256, 0, s>>>(m->gain, nullptr, (int)K, (int)N, s2, (uint4*)m->tc_b2, 0, one_d);
     QCE_CHECK_LAUNCH("circ_tc_pack_kernel");
-    {
-        const int n_elem = (int)(CT_N / 16 + 2 * (K / 16)) * 128 * 16;
-        circ_umma_pack_kernel<<<(n_elem + 255) / 256, 256, 0, s>>>(m->inv_lambda_t, m->gain, (const float*)m->tc_ilbar, (int)K, one_d, s1, s2,
-                                                                  (unsigned char*)m->tc_umma);
-        QCE_CHECK_LAUNCH("circ_umma_pack_kernel");
-    }
     {
         double* h_logc = (double*)malloc(K * sizeof(double));
         if (!h_logc || cudaMemcpyAsync(h_logc, m->logc, K * sizeof(double), cudaMemcpyDeviceToHost, s) != cudaSuccess ||
@@ -1116,20 +633,11 @@ static qce_status circ_fix_list(cudaStream_t s, int64_t rows, int** out) {
 }
 
 template <int KC>
-static qce_status launch_circ_umma_k(const CircUmmaArgs& ua, cudaStream_t s) {
-    static PerDeviceOnce once;
-    if (once.first(current_device())) QCE_CUDA_TRY(cudaFuncSetAttribute(circ_umma_kernel<KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, CU_SMEM));
-    circ_umma_kernel<KC><<<(unsigned)((ua.t.B + CU_P - 1) / CU_P), CU_THREADS, CU_SMEM, s>>>(ua);
-    QCE_CHECK_LAUNCH("circ_umma_kernel");
-    return QCE_OK;
-}
-
-template <int KC, int NW>
 static qce_status launch_circ_tc_k(const CircTcArgs& a, cudaStream_t s) {
     constexpr size_t SMEM = CT_P * CT_XP * sizeof(float2) + CT_R_BYTES + 512;
     static PerDeviceOnce once;
-    if (once.first(current_device())) QCE_CUDA_TRY(cudaFuncSetAttribute(circ_tc_kernel<KC, NW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM));
-    circ_tc_kernel<KC, NW><<<(unsigned)((a.B + CT_P - 1) / CT_P), 32 * NW, SMEM, s>>>(a);
+    if (once.first(current_device())) QCE_CUDA_TRY(cudaFuncSetAttribute(circ_tc_kernel<KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM));
+    circ_tc_kernel<KC><<<(unsigned)((a.B + CT_P - 1) / CT_P), 32 * CT_NW, SMEM, s>>>(a);
     QCE_CHECK_LAUNCH("circ_tc_kernel");
     return QCE_OK;
 }
@@ -1161,32 +669,7 @@ qce_status launch_circ_tc(const qce_circ_model* m, cudaStream_t s, const double*
         qce_status st = circ_fix_list(s, B, &a.fix_buf);
         if (st) return st;
     }
-    const int nw = (getenv("QCE_CIRC_NW") && atoi(getenv("QCE_CIRC_NW")) == 16) ? 16 : 8;      // 16 warps x 64 registers measured 7 % slower
-    qce_status st;
-    // QCE_CIRC_UMMA=1: the tcgen05 version.  Parity-green (same tests), L1TEX load 66 % -> 42 %, but 8-10 % slower than the mma.sync
-    // kernel at config 3 (340 vs 369 M estimates/s, profiles/r02_circ_umma_ab.jsonl): with 32-pilot tiles the 256 KB of parameter
-    // chunks per tile arrive at ~500 clk per 8 KB chunk, and the two GEMMs are a third of the tile's time.  The default stays mma.sync.
-    const bool umma = getenv("QCE_CIRC_UMMA") && atoi(getenv("QCE_CIRC_UMMA")) == 1;
-    if (umma) {
-        CircUmmaArgs ua;
-        ua.t = a;
-        ua.img = (const unsigned char*)m->tc_umma;
-        static long long* prof_dev = nullptr;       // (device memory: a managed buffer page-faults on the first stamp and stalls the CTA)
-        long long prof[16] = {};
-        const bool want_prof = getenv("QCE_CIRC_PROF") != nullptr;
-        if (want_prof && !prof_dev) cudaMalloc(&prof_dev, sizeof(prof));
-        ua.prof = want_prof ? prof_dev : nullptr;
-        st = m->n_comp == 64 ? launch_circ_umma_k<1>(ua, s) : launch_circ_umma_k<2>(ua, s);
-        if (want_prof && st == QCE_OK) {
-            cudaStreamSynchronize(s);
-            cudaMemcpy(prof, prof_dev, sizeof(prof), cudaMemcpyDeviceToHost);
-            fprintf(stderr, "[qce circ prof] clk: load+fft %lld | wait gemm1 %lld | epi1+softmax %lld | wait gemm2 %lld | epi2 %lld | inverse+store %lld\n",
-                    prof[1] - prof[0], prof[2] - prof[1], prof[3] - prof[2], prof[4] - prof[3], prof[5] - prof[4], prof[6] - prof[5]);
-            fprintf(stderr, "[qce circ prof]      round 0: load+fft1 %lld fft2+E %lld | round 1: load+fft1 %lld fft2+E %lld | st wait + fence %lld\n",
-                    prof[8] - prof[0], prof[9] - prof[8], prof[10] - prof[9], prof[11] - prof[10], prof[1] - prof[11]);
-        }
-    } else if (nw == 8) st = m->n_comp == 64 ? launch_circ_tc_k<1, 8>(a, s) : launch_circ_tc_k<2, 8>(a, s);
-    else st = m->n_comp == 64 ? launch_circ_tc_k<1, 8>(a, s) : launch_circ_tc_k<2, 16>(a, s);
+    const qce_status st = m->n_comp == 64 ? launch_circ_tc_k<1>(a, s) : launch_circ_tc_k<2>(a, s);
     if (st || mode == QCE_MODE_ALL || !(h_est || acc)) return st;
     return launch_circ_rows(m, s, r, a.fix_buf + 2, a.fix_buf, B, mode, n_top, rho, h_est, h_true, acc);
 }

@@ -103,7 +103,6 @@ struct qce_circ_model {
     void* tc_logc2 = nullptr;
     void* tc_ilbar = nullptr;         // [N] float: mean over the components of 1 / lambda
     void* tc_tw = nullptr;            // [256] float2 twiddles of the plain-circulant (one-dimensional) variant
-    void* tc_umma = nullptr;          // parameter chunks of the tcgen05 version (canonical K-major core-matrix order, FP16 hi / lo)
     double tc_logc_max = 0.0;
     float tc_inv_s1 = 0.f, tc_inv_s2 = 0.f;
     bool tc_ready = false;

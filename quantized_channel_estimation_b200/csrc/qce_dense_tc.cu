@@ -106,7 +106,6 @@ struct TcCtrl {
     uint64_t a_full, a_free;
     uint32_t tmem_base;
     uint32_t pad;
-    uint64_t fmt_done;       // PRO: the eight epilogue warps have written their shares of the next work unit's pilot tiles
 };
 static_assert(sizeof(TcCtrl) <= 1024, "control block");
 
@@ -148,99 +147,11 @@ __device__ __forceinline__ void tc_issue_chunk(const int q, const uint32_t d_til
     }
 }
 
-// In-kernel prologue (PRO): observe (A = I) + quantise + format the pilots straight into the tile image the bulk copies read, same
-// arithmetic as tc_format_kernel<true, ., false>.  One ITEM = one 128-byte core matrix = 8 pilots x 4 complex, one element per lane;
-// item i of a work unit of NTILES tiles: pair = i / kbs -> (tile, 8-row block), K-core kb = i % kbs.  The loads of an item are issued
-// early (fmt_load) and consumed late (fmt_store) so that their latency hides behind the epilogue work in between.  Rows that are not
-// on the grid are flagged by an atomicOr on the (zero-initialised) flag bytes.
-struct FmtItem { double2 h, w; float2 hf; };
-
-template <bool H_C64>
-__device__ __forceinline__ void fmt_load(const TcArgs& a, int64_t first_tile, int KD, int item, int lane, FmtItem& it) {
-    const int kbs = KD / 8, No = KD / 2;
-    const int pair = item / kbs, kb = item - pair * kbs;
-    const int64_t g = (first_tile + pair / (TILE_M / 8)) * TILE_M + (pair % (TILE_M / 8)) * 8 + (lane & 7);
-    const size_t e = (size_t)(g < a.B ? g : 0) * No + kb * 4 + (lane >> 3);
-    // volatile asm: the compiler must not sink these loads down to their use (it does, to save registers, and then every component
-    // of the epilogue eats a full memory latency)
-    if (H_C64) asm volatile("ld.global.cg.v2.f32 {%0, %1}, [%2];" : "=f"(it.hf.x), "=f"(it.hf.y) : "l"(reinterpret_cast<const float2*>(a.obs_h) + e));
-    else asm volatile("ld.global.cg.v2.f64 {%0, %1}, [%2];" : "=d"(it.h.x), "=d"(it.h.y) : "l"(reinterpret_cast<const double2*>(a.obs_h) + e));
-    asm volatile("ld.global.cg.v2.f64 {%0, %1}, [%2];" : "=d"(it.w.x), "=d"(it.w.y) : "l"(a.obs_noise + e));
-}
-
-// double -> float through the integer pipe (round half up on the magnitude; FP32-normal range, else the hardware conversion): the
-// FP64 / conversion pipes crawl while the tensor pipe is saturated, and this runs inside the estimate kernel's epilogue warps
-__device__ __forceinline__ float fmt_d2f(const double x) {
-    const uint32_t hi = (uint32_t)__double2hiint(x), lo = (uint32_t)__double2loint(x);
-    const uint32_t e = (hi >> 20) & 0x7ffu;
-    if (e - 897u < 253u) return __uint_as_float(((hi & 0x80000000u) | ((e - 896u) << 23) | ((hi & 0xfffffu) << 3) | (lo >> 29)) + ((lo >> 28) & 1u));
-    return (float)x;
-}
-
-// sign(h + s n) exactly as the float64 reference computes it (1-bit quantiser).  The rounded double sum has the sign of the exact sum
-// h + fl(s n); an FP32 evaluation decides it whenever |y| is not within 2^-19 of cancellation (relative to |h| + |s n|, 30x the FP32
-// error bound), which leaves ~1e-6 of the elements (and every NaN / infinity) to the FP64 path.
-__device__ __forceinline__ float fmt_sign1(const double h, const float hf, const double n, const double s, const float sf) {
-    const float p = sf * fmt_d2f(n);
-    const float y = hf + p;
-    if (fabsf(y) > 1.9e-6f * (fabsf(hf) + fabsf(p))) return y > 0.f ? 1.f : -1.f;      // false for NaN
-    const double yd = __dadd_rn(h, __dmul_rn(s, n));
-    return (yd > 0.0) ? 1.f : ((yd < 0.0) ? -1.f : ((yd == 0.0) ? 0.f : __int_as_float(0x7fc00000)));
-}
-
-template <bool H_C64>
-__device__ __forceinline__ void fmt_store(const TcArgs& a, int64_t first_tile, int KD, int item, int lane, const FmtItem& it) {
-    const int kbs = KD / 8;
-    const int pair = item / kbs, kb = item - pair * kbs;
-    const int64_t tile = first_tile + pair / (TILE_M / 8);
-    const int mb = pair % (TILE_M / 8);
-    const int64_t g = tile * TILE_M + mb * 8 + (lane & 7);
-    float qr = 0.f, qi = 0.f;
-    if (g < a.B) {       // 1-bit quantiser (the host launches the fused prologue for n_bits = 1 only)
-        const float sf = (float)a.obs_noise_scale_f;
-        if (H_C64) {
-            qr = fmt_sign1((double)it.hf.x, it.hf.x, it.w.x, a.obs_noise_scale, sf);
-            qi = fmt_sign1((double)it.hf.y, it.hf.y, it.w.y, a.obs_noise_scale, sf);
-        } else {
-            qr = fmt_sign1(it.h.x, fmt_d2f(it.h.x), it.w.x, a.obs_noise_scale, sf);
-            qi = fmt_sign1(it.h.y, fmt_d2f(it.h.y), it.w.y, a.obs_noise_scale, sf);
-        }
-    }
-    if (!(qr == qr && qi == qi)) {     // NaN data: flag the row (its estimate becomes NaN)
-        const int64_t fr = tile * TILE_M + mb * 8 + (lane & 7);      // (the flag buffer is padded to whole units)
-        const unsigned old = atomicOr(reinterpret_cast<unsigned int*>(const_cast<unsigned char*>(a.bad)) + (fr >> 2), 1u << (8 * (int)(fr & 3)));
-        if (((old >> (8 * (int)(fr & 3))) & 0xffu) == 0u && fr < a.B) a.fix_idx[atomicAdd(a.fix_cnt, 1)] = (int)fr;      // first flag of this row
-        qr = qi = 0.f;
-    }
-    unsigned char* tile_img = reinterpret_cast<unsigned char*>(const_cast<__half*>(a.a_img)) + (size_t)tile * TILE_M * KD * 2;
-    *reinterpret_cast<__half2*>(tile_img + (size_t)(kb * (TILE_M / 8) + mb) * 128 + (lane & 7) * 16 + (lane >> 3) * 4) = __floats2half2_rn(qr, qi);
-}
-
-// pull the (h, noise) rows of one work unit of this CTA into L2 (two bulk prefetches): the small per-item loads of the in-kernel
-// formatter then hit L2 instead of fetching DRAM in 32-byte pieces spread over the whole unit (measured: 2x read amplification)
-__device__ __forceinline__ void fmt_prefetch_unit(const TcArgs& a, int64_t first_tile, int ntiles, int KD) {
-    const int No = KD / 2;
-    const int64_t r0 = first_tile * TILE_M;
-    if (r0 >= a.B) return;
-    const int64_t rows = (a.B - r0) < (int64_t)ntiles * TILE_M ? (a.B - r0) : (int64_t)ntiles * TILE_M;
-    const size_t hsz = a.obs_h_c64 ? 8 : 16;
-    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"((const char*)a.obs_h + (size_t)r0 * No * hsz), "r"((uint32_t)(rows * No * hsz)) : "memory");
-    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"((const char*)a.obs_noise + (size_t)r0 * No * 16), "r"((uint32_t)(rows * No * 16)) : "memory");
-}
-
-// a whole share of a work unit at once (the first unit of a CTA, formatted by the eight epilogue warps before the pipeline starts)
-template <bool H_C64>
-__device__ __forceinline__ void fmt_items(const TcArgs& a, int64_t first_tile, int KD, int item0, int n_items, int lane) {
-    for (int i = 0; i < n_items; i += 4) {
-        FmtItem it[4];
-        #pragma unroll
-        for (int j = 0; j < 4; ++j) if (i + j < n_items) fmt_load<H_C64>(a, first_tile, KD, item0 + i + j, lane, it[j]);
-        #pragma unroll
-        for (int j = 0; j < 4; ++j) if (i + j < n_items) fmt_store<H_C64>(a, first_tile, KD, item0 + i + j, lane, it[j]);
-    }
-}
-
 __device__ __forceinline__ void tie_append(const unsigned char* bad, int* tie_buf, int64_t chunk_row);
+
+// fused 'all' epilogue: a warp skips the LMMSE row of a component whose un-normalised weight is below this for all of its 32 pilots
+// (the normaliser is >= 1, so the dropped terms are < TC_SKIP_THRESH each); measured: no effect on the speed up to 1e-9
+constexpr float TC_SKIP_THRESH = 1e-30f;
 
 // hi_a + lo_a > hi_b + lo_b, exactly (the FP64 sums of FP32 pairs are exact)
 __device__ __noinline__ bool pair_greater_f64(float hi_a, float lo_a, float hi_b, float lo_b) {
@@ -252,9 +163,7 @@ __device__ __noinline__ bool pair_greater_f64(float hi_a, float lo_a, float hi_b
 // cumulative-probability modes run 1 -> select -> 2) or, with TcArgs::unit_comp, the single component of each work unit of pilots
 // regrouped by label (top-1 on large batches: 1 -> bucket -> 2)
 // KDC = n_obs / 16 (reduction length 32 KDC); NCHZ = 0 (no whitening columns: an H-part launch) or KDC; NCHH = H columns / 32
-// PRO = true: fused prologue -- no formatter launch, the kernel builds its own pilot tiles from (h, noise): the epilogue warps format
-// the first work unit of the CTA, warp 2 every further one while the tensor pipe works on the previous.
-template <int KDC, int NCHZ, int NCHH, bool OFFS, int CG, int EPI, int ORDER, int AC, bool PRO = false>
+template <int KDC, int NCHZ, int NCHH, bool OFFS, int CG, int EPI, int ORDER, int AC>
 __global__ void __launch_bounds__(NUM_THREADS, 1) dense_tc_kernel(const TcArgs a) {
     constexpr int NZ = 32 * NCHZ, NH = 32 * NCHH;
     constexpr int ACCB = tc_accb(EPI, 32 * KDC, NZ, NH, ORDER, AC);
@@ -274,17 +183,13 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) dense_tc_kernel(const TcArgs a
     // work unit: CG * TILES tiles (256 pilots per CTA); the cluster (CG CTAs) walks the units round-robin
     const uint32_t rank = (CG == 2) ? cluster_ctarank() : 0u;
     int64_t n_units = (a.B + CG * NTILES * TILE_M - 1) / (CG * NTILES * TILE_M);
-    // regrouped pilots (slot -> pilot through perm): one component per work unit (bucketed top-1, pair mode), or -- listed -- the
-    // components some pilot of the unit has a non-zero weight for (top-n / cumulative: pilots grouped by their best component share
-    // most of their selections)
-    const bool listed = (EPI == 2) && a.unit_list != nullptr;
-    const bool bucket = (EPI == 2) && (a.unit_comp != nullptr || listed);
+    // regrouped pilots (slot -> pilot through perm): one component per work unit (bucketed top-1, pair mode)
+    const bool bucket = (EPI == 2) && a.unit_comp != nullptr;
     if (bucket) n_units = __ldg(a.n_units_dev);
-    // components of a unit: (first, count) and, when listed, the list
-    auto unit_comps = [&](int64_t unit, int& kb, int& nk, const int*& ul) {
-        kb = 0; nk = a.K; ul = nullptr;
-        if (listed) { nk = __ldg(a.unit_nk + unit); ul = a.unit_list + unit * a.K; }
-        else if (bucket) { kb = __ldg(a.unit_comp + unit); nk = 1; }
+    // components of a unit: (first, count)
+    auto unit_comps = [&](int64_t unit, int& kb, int& nk) {
+        kb = 0; nk = a.K;
+        if (bucket) { kb = __ldg(a.unit_comp + unit); nk = 1; }
     };
     const int64_t unit0 = blockIdx.x / CG, unit_step = gridDim.x / CG;
     // the SM-pair variant is only launched for triangular Linv (the common, Cholesky case): its offsets are compile-time
@@ -300,7 +205,6 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) dense_tc_kernel(const TcArgs a
         }
         mbar_init(smem_u32(&ctrl->a_full), full_count);
         mbar_init(smem_u32(&ctrl->a_free), 1);
-        mbar_init(smem_u32(&ctrl->fmt_done), 8);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == 2) {
@@ -329,10 +233,9 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) dense_tc_kernel(const TcArgs a
             constexpr size_t COMP_STRIDE = COMP_BYTES * CG;      // CG=2: [k][rank]
             for (int64_t unit = unit0; unit < n_units; unit += unit_step) {
                 int kb, nk;
-                const int* ul;
-                unit_comps(unit, kb, nk, ul);
+                unit_comps(unit, kb, nk);
                 for (int ki = 0; ki < nk; ++ki) {
-                    const int k = ul ? __ldg(ul + ki) : kb + ki;
+                    const int k = kb + ki;
                     const unsigned char* comp = img + (size_t)k * COMP_STRIDE;
                     #pragma unroll
                     for (int q = 0; q < Cfg::NCHUNK; ++q) {
@@ -346,16 +249,10 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) dense_tc_kernel(const TcArgs a
             }
         } else if (warp == 3 && lane == 0) {
             // ===================== pilot-tile producer: the two pre-formatted 128-pilot tiles of each unit, one bulk copy each
-            uint32_t fph = 0, n_done = 0;
+            uint32_t fph = 0;
             for (int64_t unit = unit0; unit < n_units; unit += unit_step) {
                 mbar_wait(smem_u32(&ctrl->a_free), fph ^ 1);      // all MMAs of the previous unit have read the tiles
                 fph ^= 1;
-                if (PRO) {     // the tiles of this unit must have been written (generic proxy) before the bulk copy (async proxy) reads them
-                    mbar_wait(smem_u32(&ctrl->fmt_done), n_done & 1u);      // (a spin on a shared-memory counter here starved the epilogue
-                    ++n_done;                                               //  warps that share this warp's scheduler)
-                    __threadfence();
-                    asm volatile("fence.proxy.async;" ::: "memory");
-                }
                 mbar_expect_tx(smem_u32(&ctrl->a_full), NTILES * Cfg::A_TILE_BYTES);
                 #pragma unroll
                 for (int t = 0; t < NTILES; ++t)
@@ -384,7 +281,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) dense_tc_kernel(const TcArgs a
                 a_phase ^= 1;
                 tc_fence_after();
                 w_a += QCE_CLK() - ca;
-                const int nk = listed ? __ldg(a.unit_nk + unit) : (bucket ? 1 : a.K);
+                const int nk = bucket ? 1 : a.K;
                 for (int k = 0; k < nk; ++k) {
                     if (ORDER == 0) {
                     #pragma unroll
@@ -460,7 +357,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) dense_tc_kernel(const TcArgs a
                 mbar_wait(smem_u32(&ctrl->a_full), a_phase);
                 a_phase ^= 1;
                 mbar_arrive_cluster(smem_u32(&ctrl->a_full), 0);
-                const int nk = listed ? __ldg(a.unit_nk + unit) : (bucket ? 1 : a.K);
+                const int nk = bucket ? 1 : a.K;
                 for (int k = 0; k < nk; ++k) {
                     #pragma unroll
                     for (int q = 0; q < Cfg::NCHUNK; ++q) {
@@ -482,18 +379,6 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) dense_tc_kernel(const TcArgs a
         uint32_t fph = 0;                              // parity of acc_full (one bit per accumulator buffer of this tile)
         uint32_t accn = 0;                             // components drained so far (ACCB = 2: buffer = accn & 1)
         const int N = a.N;
-        // PRO: items of a work unit per epilogue warp, and how they are spread over the components of the previous unit
-        constexpr int FMT_IPW = NTILES * (TILE_M / 8) * (Cfg::KD / 8) / 8;
-        const int fmt_slot = warp - 4;
-        const int fmt_every = a.K / FMT_IPW;      // one item every fmt_every components (the host only launches PRO when FMT_IPW divides K)
-        if (PRO && unit0 < n_units) {      // the eight epilogue warps share the first work unit of this CTA
-            if (a.obs_h_c64) fmt_items<true>(a, (unit0 * CG + rank) * NTILES, Cfg::KD, fmt_slot * FMT_IPW, FMT_IPW, lane);
-            else fmt_items<false>(a, (unit0 * CG + rank) * NTILES, Cfg::KD, fmt_slot * FMT_IPW, FMT_IPW, lane);
-            __threadfence();
-            asm volatile("fence.proxy.async;" ::: "memory");
-            __syncwarp();
-            if (lane == 0) mbar_arrive(smem_u32(&ctrl->fmt_done));
-        }
         double err = 0.0, pw = 0.0, cnt = 0.0;     // cnt also gates the atomics (rows handled by this thread)
         long long w_acc = 0, c_z = 0, c_h = 0, c_pro = 0, c_ld = 0;
 
@@ -515,43 +400,31 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) dense_tc_kernel(const TcArgs a
             int64_t src = tile_base + row;
             bool valid = src < a.B;
             int kb, nk;
-            const int* ul;
-            unit_comps(unit, kb, nk, ul);
+            unit_comps(unit, kb, nk);
             if (bucket) {
                 src = __ldg(a.perm + tile_base + row);
                 valid = src >= 0;
             }
-            int k_n = (ul && nk > 0) ? __ldg(ul) : kb;     // the component of the next iteration (its scalars are fetched one ahead)
+            int k_n = kb;                              // the component of the next iteration (its scalars are fetched one ahead)
             float zs_n = __ldg(a.zscale + k_n), hs_n = __ldg(a.hscale + k_n);
             float2 lc_n = __ldg(a.logc2 + k_n);
             const int64_t grow = valid ? src : 0;     // rows past the end read row 0, never write
             float w_n = 0.f;
             if (EPI == 2) {
-                if (listed) w_n = valid ? __ldg(a.w_in + grow * a.K + k_n) : 0.f;
-                else if (bucket) w_n = valid ? (a.slot_w ? __ldg(a.slot_w + tile_base + row) : 1.f) : 0.f;
+                if (bucket) w_n = valid ? (a.slot_w ? __ldg(a.slot_w + tile_base + row) : 1.f) : 0.f;
                 else w_n = __ldg(a.w_in + grow * a.K);
             }
-            const bool fmt_next = PRO && (unit + unit_step < n_units);
-            const int64_t fmt_tile0 = ((unit + unit_step) * CG + rank) * NTILES;
-            if (fmt_next && fmt_slot == 0 && lane == 0) fmt_prefetch_unit(a, fmt_tile0, NTILES, Cfg::KD);
             for (int ki = 0; ki < nk; ++ki) {
                 const int k = k_n;
-                // PRO: this warp's share of the NEXT unit's pilot tiles: loads issued here, consumed after the accumulator is released
-                FmtItem fit;
-                const bool fmt_now = fmt_next && (k % fmt_every == 0);
-                const int fmt_item = fmt_slot * FMT_IPW + k / fmt_every;
-                if (PRO && fmt_now) {
-                    if (a.obs_h_c64) fmt_load<true>(a, fmt_tile0, Cfg::KD, fmt_item, lane, fit); else fmt_load<false>(a, fmt_tile0, Cfg::KD, fmt_item, lane, fit);
-                }
                 // per-component scalars were fetched one iteration ahead (their L2 latency would otherwise sit on the
                 // critical path between "accumulator ready" and "accumulator released")
                 const float zs = zs_n, hs = hs_n;
                 const float2 lc = lc_n;
                 const float w_k = w_n;
                 if (ki + 1 < nk) {
-                    k_n = ul ? __ldg(ul + ki + 1) : k + 1;
+                    k_n = k + 1;
                     zs_n = __ldg(a.zscale + k_n); hs_n = __ldg(a.hscale + k_n); lc_n = __ldg(a.logc2 + k_n);
-                    if (EPI == 2) w_n = (listed && !valid) ? 0.f : __ldg(a.w_in + grow * a.K + k_n);
+                    if (EPI == 2) w_n = __ldg(a.w_in + grow * a.K + k_n);
                 }
                 // ---- whitened residual -> quadratic form
                 c0 = QCE_CLK();
@@ -673,7 +546,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) dense_tc_kernel(const TcArgs a
                 c_z += c2 - c1;
                 // ---- LMMSE row, weighted accumulation (the first H chunk is already in registers)
                 if (EPI != 1) {
-                    const bool any = __any_sync(0xffffffffu, (EPI == 2) ? (p != 0.f) : (p > a.skip_thresh));
+                    const bool any = __any_sync(0xffffffffu, (EPI == 2) ? (p != 0.f) : (p > TC_SKIP_THRESH));
                     const float2 ph = make_float2(p * hs, p * hs);
                     #pragma unroll
                     for (int ch = 0; ch < NCHH; ++ch) {
@@ -700,14 +573,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) dense_tc_kernel(const TcArgs a
                     if (CG == 2) mbar_arrive_cluster(smem_u32(&ctrl->acc_empty[0]) + 8u * ai, 0); else mbar_arrive(smem_u32(&ctrl->acc_empty[0]) + 8u * ai);
                 }
                 }
-                if (PRO && fmt_now) { if (a.obs_h_c64) fmt_store<true>(a, fmt_tile0, Cfg::KD, fmt_item, lane, fit); else fmt_store<false>(a, fmt_tile0, Cfg::KD, fmt_item, lane, fit); }
                 c_h += QCE_CLK() - c2;
-            }
-            if (fmt_next) {             // this warp's share of the next unit is written: publish it to the tile producer
-                __threadfence();
-                asm volatile("fence.proxy.async;" ::: "memory");
-                __syncwarp();
-                if (lane == 0) mbar_arrive(smem_u32(&ctrl->fmt_done));
             }
 
             // ---- finalise: normalise, write the estimate row, NMSE accumulators (FP32 per row: FP64 stalls behind the
@@ -731,8 +597,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) dense_tc_kernel(const TcArgs a
                 if ((a.top_flags & QCE_FLAG_TOP1_EXP_ARGMAX) && fabsf(best_hi + 745.1332f) < 0.01f) tie = true;
                 if (tie) tie_append(a.bad, a.tie_buf, g);
             }
-            // (flags read here, after the last component: with the fused prologue they are written by other warps of this kernel)
-            if (EPI != 1 && valid && !hard_tie && (PRO ? __ldcg(a.bad + g) : __ldg(a.bad + g)) == 0) {
+            if (EPI != 1 && valid && !hard_tie && __ldg(a.bad + g) == 0) {
                 const float invs = (EPI == 2 || EPI == 3) ? 1.f : 1.f / ssum;
                 if (EPI == 2 && a.slot_w) {      // pair mode: this slot's weighted row is one of several addends of the pilot's estimate:
                     // vector reductions (4 floats each) into the FP32 row of the pilot; tc_pair_finish_kernel writes the estimate
@@ -1208,24 +1073,22 @@ __global__ void __launch_bounds__(256) tc_select_kernel(const float2* __restrict
 // scans (n + 1 of them for top-n), the same too-close-to-call rules.  The weight rows go back through shared memory so that the
 // global stores are coalesced.  pair_cnt != null: histogram of the selected (pilot, component) pairs with a weight above pair_thresh
 // (the count pass of the pair-bucketed combination, fused).
-// R pilots and 128 threads per block (all of them stage, R of them select).  The staging loop is latency-bound, so small tiles --
-// many blocks, many loads in flight per SM -- win: one 132 KB block of 256 pilots per SM 503 us per 2^19 pilots at K = 64, 128 pilots
-// (66 KB) 265 us, 64: 222 us, 32: 198 us.
+// SEL_ROWS pilots and 128 threads per block (all of them stage, SEL_ROWS of them select).  The staging loop is latency-bound, so
+// small tiles -- many blocks, many loads in flight per SM -- win: one 132 KB block of 256 pilots per SM 503 us per 2^19 pilots at
+// K = 64, 128 pilots (66 KB) 265 us, 64: 222 us, 32: 198 us, 16: 301 us.
 constexpr int SEL_THREADS = 128;
-template <int R>
+constexpr int SEL_ROWS = 32;
 __global__ void __launch_bounds__(SEL_THREADS) tc_select_rows_kernel(const float2* __restrict__ lp2, int64_t B, int K, int mode, int n_top, double rho, int flags,
                                                              float* __restrict__ w_out, double* __restrict__ logp_out, int* __restrict__ top_out,
                                                              const unsigned char* __restrict__ bad, int* __restrict__ tie_buf, double tie_eps0,
-                                                             const double* __restrict__ logc, double inv_nobs, int* __restrict__ pair_cnt, float pair_thresh,
-                                                             int* __restrict__ key_out) {
-    // key_out != null: also the best component of every pilot (the grouping key of the listed combination)
+                                                             const double* __restrict__ logc, double inv_nobs, int* __restrict__ pair_cnt, float pair_thresh) {
     extern __shared__ __align__(16) unsigned char sel_smem[];
-    constexpr int P = R + 1;                                   // pitch: thread = pilot reads column `pilot` of every row k
+    constexpr int P = SEL_ROWS + 1;                            // pitch: thread = pilot reads column `pilot` of every row k
     float* s_hi = reinterpret_cast<float*>(sel_smem);          // [K][P]  l_hi, later e_k = exp(l_k - max), later the weight
     float* s_lo = s_hi + (size_t)K * P;                        // [K][P]  l_lo
     int* s_cnt = reinterpret_cast<int*>(s_lo + (size_t)K * P); // [K] pair histogram of this block
-    const int64_t row0 = (int64_t)blockIdx.x * R;
-    const int nrow = (int)((B - row0) < R ? (B - row0) : R);
+    const int64_t row0 = (int64_t)blockIdx.x * SEL_ROWS;
+    const int nrow = (int)((B - row0) < SEL_ROWS ? (B - row0) : SEL_ROWS);
     {
         const float2* src = lp2 + row0 * K;
         const int n = nrow * K;
@@ -1266,7 +1129,6 @@ __global__ void __launch_bounds__(SEL_THREADS) tc_select_rows_kernel(const float
         }
         const float m_lo = s_lo[amax * P + r];
         const double mx = (double)m_hi + (double)m_lo;
-        if (key_out) key_out[row0 + r] = amax;
         double tie_eps = tie_eps0;
         if (logc) tie_eps *= fmax(1.0, (__ldg(logc + amax) - mx) * inv_nobs);
         const float epsf = (float)tie_eps;
@@ -1508,44 +1370,6 @@ __global__ void __launch_bounds__(256) tc_bucket_gather_kernel(const unsigned ch
     for (int c = threadIdx.x / TILE_M; c < copies * kbs; c += 256 / TILE_M) {
         const uint4 v = src >= 0 ? __ldg(reinterpret_cast<const uint4*>(from + (size_t)c * TILE_M * 16)) : make_uint4(0u, 0u, 0u, 0u);
         *reinterpret_cast<uint4*>(to + (size_t)c * TILE_M * 16) = v;
-    }
-}
-
-// ---- listed combination: which components does a work unit of regrouped pilots need?  One block per unit; the slots' weight rows are
-// OR-ed into a K-bit mask in shared memory, the set bits become the unit's component list (ascending).
-__global__ void __launch_bounds__(256) tc_unit_list_kernel(const float* __restrict__ w, const int* __restrict__ perm, const int* __restrict__ n_units,
-                                                           int unit_rows, int K, int* __restrict__ unit_list, int* __restrict__ unit_nk) {
-    const int u = blockIdx.x;
-    if (u >= __ldg(n_units)) return;
-    __shared__ unsigned s_mask[32];                 // K <= 1024
-    __shared__ int s_n;
-    if (threadIdx.x < 32) s_mask[threadIdx.x] = 0u;
-    if (threadIdx.x == 0) s_n = 0;
-    __syncthreads();
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    for (int sl = warp; sl < unit_rows; sl += 8) {              // a warp per slot, lanes over the components (coalesced weight rows)
-        const int b = __ldg(perm + (size_t)u * unit_rows + sl);
-        if (b < 0) continue;
-        for (int k0 = 0; k0 < K; k0 += 32) {
-            const int k = k0 + lane;
-            const bool on = k < K && w[(size_t)b * K + k] != 0.f;       // (NaN weights count: their pilots are answered elsewhere)
-            const unsigned m = __ballot_sync(0xffffffffu, on);
-            if (lane == 0 && m && (s_mask[k0 >> 5] | m) != s_mask[k0 >> 5]) atomicOr(&s_mask[k0 >> 5], m);
-        }
-    }
-    __syncthreads();
-    if (threadIdx.x < 32) {
-        // ascending list: word by word
-        for (int wd = 0; wd * 32 < K; ++wd) {
-            const unsigned m = s_mask[wd];
-            const bool on = (m >> lane) & 1u;
-            const unsigned bal = __ballot_sync(0xffffffffu, on);
-            if (on) unit_list[(size_t)u * K + s_n + __popc(bal & ((1u << lane) - 1u))] = wd * 32 + lane;
-            __syncwarp();
-            if (lane == 0) s_n += __popc(bal);
-            __syncwarp();
-        }
-        if (lane == 0) unit_nk[u] = s_n;
     }
 }
 
@@ -1852,11 +1676,11 @@ qce_status tc_pack_params(qce_model* m, cudaStream_t s) {
     return QCE_OK;
 }
 
-template <int KDC, int NCHZ, int NCHH, bool OFFS, int CG, int EPI, int ORDER, int AC = 1, bool PRO = false>
+template <int KDC, int NCHZ, int NCHH, bool OFFS, int CG, int EPI, int ORDER, int AC = 1>
 static qce_status launch_cfg(const TcArgs& a, cudaStream_t s) {
     using Cfg = TcCfg<32 * KDC, 32 * NCHZ, 32 * NCHH, CG, ORDER, AC, tc_accb(EPI, 32 * KDC, 32 * NCHZ, 32 * NCHH, ORDER, AC)>;
     static PerDeviceOnce once;
-    auto kern = dense_tc_kernel<KDC, NCHZ, NCHH, OFFS, CG, EPI, ORDER, AC, PRO>;
+    auto kern = dense_tc_kernel<KDC, NCHZ, NCHH, OFFS, CG, EPI, ORDER, AC>;
     const int dev = current_device();
     if (once.first(dev)) QCE_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
     int sms = 148;
@@ -1931,26 +1755,23 @@ static void tc_fill_args(const qce_model* m, const TileScratch* ts, int64_t B, d
     a.prof = nullptr;
     a.h_stride = 2 * m->n_ant; a.h_col0 = 0; a.count_rows = 1;
     a.wide_io = (reinterpret_cast<uintptr_t>(h_est) % 32 == 0 && reinterpret_cast<uintptr_t>(h_true) % 32 == 0 && m->n_ant % 4 == 0) ? 1 : 0;
-    const char* th = getenv("QCE_TC_SKIP");                 // tuning knob (read per launch); measured: no effect up to 1e-9
-    a.skip_thresh = th ? (float)atof(th) : 1e-30f;
-    a.unit_comp = nullptr; a.perm = nullptr; a.n_units_dev = nullptr; a.unit_list = nullptr; a.unit_nk = nullptr;
+    a.unit_comp = nullptr; a.perm = nullptr; a.n_units_dev = nullptr;
     a.slot_w = nullptr; a.run_flag = nullptr; a.run_flag_want = 0; a.pair_acc = nullptr;
     a.top_out = nullptr; a.top_flags = m->flags;
-    a.fix_cnt = ts->fix_buf; a.fix_idx = ts->fix_buf + 2; a.tie_buf = ts->tie_buf;
+    a.tie_buf = ts->tie_buf;
     a.tie_eps = (float)tc_tie_eps(m); a.inv_nobs = 1.f / (float)m->n_obs;
 }
 
 static qce_status tc_run_split(const qce_model* m, const TileScratch* ts, cudaStream_t s, int64_t B, int epi, int part, double* h_est,
                                const void* h_true, int h_true_c64, double* acc, const int* unit_comp = nullptr, const int* perm = nullptr,
                                const int* n_units_dev = nullptr, const void* bucket_img = nullptr, int* top_out = nullptr, const float* slot_w = nullptr, const int* run_flag = nullptr,
-                               int run_flag_want = 0, const int* unit_list = nullptr, const int* unit_nk = nullptr) {
+                               int run_flag_want = 0) {
     const TcParams& p = m->tc;
     TcArgs a;
     tc_fill_args(m, ts, B, h_est, h_true, h_true_c64, acc, &a);
     a.slot_w = slot_w; a.run_flag = run_flag; a.run_flag_want = run_flag_want;
     a.pair_acc = (float*)ts->tmp_est;
-    if (unit_comp || unit_list) { a.unit_comp = unit_comp; a.perm = perm; a.n_units_dev = n_units_dev; a.a_img = (const __half*)bucket_img; }
-    a.unit_list = unit_list; a.unit_nk = unit_nk;
+    if (unit_comp) { a.unit_comp = unit_comp; a.perm = perm; a.n_units_dev = n_units_dev; a.a_img = (const __half*)bucket_img; }
     a.top_out = top_out;
     a.image2 = (const unsigned char*)(epi == 1 ? p.image_z : p.image_h[part]);
     a.h_col0 = part * p.part_cols;
@@ -1992,9 +1813,8 @@ static qce_status tc_run(const qce_model* m, const TileScratch* ts, cudaStream_t
     a.prof = want_prof ? prof : nullptr;
     const bool offs = p.has_offsets;
     const int cz = m->n_obs / 16, ch = m->n_ant / 16;
-    // QCE_TC_CG=1 selects the single-CTA (cta_group::1) variant; default is the SM-pair variant
-    static const int cg_env = (getenv("QCE_TC_CG") && atoi(getenv("QCE_TC_CG")) == 1) ? 1 : 2;
-    const int cg = p.triangular ? cg_env : 1;
+    // the SM-pair (cta_group::2) variant needs a lower-triangular whitening factor; any other runs on single CTAs (cta_group::1)
+    const int cg = p.triangular ? 2 : 1;
     qce_status st = QCE_ERR_UNSUPPORTED;
     bool hit = false;
 #define QCE_TC_CASE(Z, H) if (cz == Z && ch == H) { st = launch_offs<Z, H>(a, offs, cg, p.split_a, s); hit = true; }
@@ -2038,6 +1858,9 @@ qce_status tc_format(qce_model* m, cudaStream_t s, const double* r, int64_t B) {
     return tc_format_into(m, s, r, B, &ts);
 }
 
+// pair mode: at most this many (pilot, component) pairs per pilot on average, else the dense weighted launch (a tuning constant)
+constexpr int TC_PAIR_CAP = 4;
+
 // the general path: log-probabilities -> per-mode weights -> weighted combination (three launches)
 static qce_status tc_run_modes(qce_model* m, TileScratch* ts, cudaStream_t s, int64_t B, int mode, int n_top, double rho, double* h_est,
                                double* logp_out, const void* h_true, int h_true_c64, double* acc) {
@@ -2053,21 +1876,19 @@ static qce_status tc_run_modes(qce_model* m, TileScratch* ts, cudaStream_t s, in
     // Pair mode (top-n, cumulative rho, and 'all' on the large shapes): only the (pilot, component) pairs with a weight that matters
     // are combined, regrouped by component like the top-1 labels.  'all': weights <= 1e-9 are below half an ulp of the FP32
     // accumulators the weighted launch sums them in (64 of them together still are), so dropping them changes nothing that path
-    // could represent.  When a batch has more than QCE_TC_PAIR_CAP (4) pairs per pilot on average -- a flat posterior -- the dense
+    // could represent.  When a batch has more than TC_PAIR_CAP pairs per pilot on average -- a flat posterior -- the dense
     // weighted launch runs instead; the decision is made on the device (both are enqueued, one returns at once).
     // Default: on for the large shapes (n_obs > 64: an LMMSE row block launch over all K components costs 2-4x the whitening launch),
     // off for the fused shapes, where the weighted launch is as fast (measured at config 2, profiles/r02_modes.jsonl);
     // QCE_TC_PAIRS=1 / 0 forces it on / off.
     const int pair_env = getenv("QCE_TC_PAIRS") ? atoi(getenv("QCE_TC_PAIRS")) : -1;
     const bool pair_on = pair_env < 0 ? m->tc.split : pair_env != 0;
-    const int pair_cap = getenv("QCE_TC_PAIR_CAP") ? atoi(getenv("QCE_TC_PAIR_CAP")) : 4;
-    const bool sparse_all = mode == QCE_MODE_ALL && m->tc.split && !(getenv("QCE_TC_SPARSE_ALL") && atoi(getenv("QCE_TC_SPARSE_ALL")) == 0);
-    const bool pair_mode_ok = (mode == QCE_MODE_TOPN && n_top <= pair_cap) || mode == QCE_MODE_CUMPROB || sparse_all;
-    const bool pairs = pair_on && pair_cap >= 1 && want_est && pair_mode_ok && m->n_comp >= 8 && B >= 16 * unit_rows;
+    const bool pair_mode_ok = (mode == QCE_MODE_TOPN && n_top <= TC_PAIR_CAP) || mode == QCE_MODE_CUMPROB || (mode == QCE_MODE_ALL && m->tc.split);
+    const bool pairs = pair_on && want_est && pair_mode_ok && m->n_comp >= 8 && B >= 16 * unit_rows;
     // (a selected component whose renormalised weight is below 1e-9 -- the tail of a top-n / cumulative selection at a peaked posterior
     // -- is not a pair either: it cannot change the FP32 row the pairs are added into)
     const float pair_thresh = 1e-9f;
-    if (pairs && chunk > ((int64_t)1 << 19)) chunk = (int64_t)1 << 19;      // (the regrouped pilot tiles take pair_cap x the chunk's tiles)
+    if (pairs && chunk > ((int64_t)1 << 19)) chunk = (int64_t)1 << 19;      // (the regrouped pilot tiles take TC_PAIR_CAP x the chunk's tiles)
     if (chunk > B) chunk = B;
     qce_status st = tc_scratch_aux(ts, (size_t)chunk, (size_t)m->n_comp);
     if (st) return st;
@@ -2086,26 +1907,8 @@ static qce_status tc_run_modes(qce_model* m, TileScratch* ts, cudaStream_t s, in
         b_top = (int*)ts->bidx; b_perm = b_top + chunk; b_ucomp = b_perm + cap_rows; b_cnt = b_ucomp + cap_units;
         b_off = b_cnt + m->n_comp; b_cur = b_off + m->n_comp; b_nu = b_cur + m->n_comp;
     }
-    // Listed combination (top-n / cumulative rho where the pair path does not pay, i.e. the fused shapes): the pilots are regrouped by
-    // their best component like top-1, every unit then runs only the components its pilots selected (their union over 512 pilots
-    // of one bucket is a fraction of K), with the dense weight rows -- each pilot is still answered once, no atomics.
-    // Opt-in (QCE_TC_LISTED=1): on the random-PSD mixtures of the benchmark the runner-up components of a bucket's pilots are not
-    // clustered -- the union over 512 pilots is nearly all K -- and the launch is slower than the weighted one (config 2 top-4:
-    // 3.19 vs 2.84 ms per 2^19 pilots, combine launch 1.51 vs 1.35 ms, profiles/r02_modes.jsonl); mixtures whose components have
-    // few neighbours each (angular clusters of a channel model) are where it pays.
-    const bool listed = (getenv("QCE_TC_LISTED") && atoi(getenv("QCE_TC_LISTED")) == 1) && want_est && !bucketed && !pairs &&
-                        (mode == QCE_MODE_TOPN || mode == QCE_MODE_CUMPROB) && m->n_comp >= 8 && m->n_comp <= 256 && chunk >= 4 * (int64_t)bucket_rows;
-    // (K <= 256: the grouping key comes from the thread-per-pilot selection kernel)
-    int *l_key = nullptr, *l_perm = nullptr, *l_ucomp = nullptr, *l_cnt = nullptr, *l_off = nullptr, *l_cur = nullptr, *l_nu = nullptr, *l_list = nullptr, *l_nk = nullptr;
-    if (listed) {      // key[rows] | perm[slots] | unit_comp[units] | cnt[K] off[K] cursor[K] | n_units | unit_nk[units] | unit_list[units][K]
-        st = tc_scratch_bucket(ts, (size_t)(cap_rows / TILE_M + 4) * tile_bytes,
-                               (size_t)(chunk + cap_rows + 2 * cap_units + 3 * m->n_comp + 1 + cap_units * m->n_comp));
-        if (st) return st;
-        l_key = (int*)ts->bidx; l_perm = l_key + chunk; l_ucomp = l_perm + cap_rows; l_cnt = l_ucomp + cap_units;
-        l_off = l_cnt + m->n_comp; l_cur = l_off + m->n_comp; l_nu = l_cur + m->n_comp; l_nk = l_nu + 1; l_list = l_nk + cap_units;
-    }
     // pair mode: perm[slots] | slot_w[slots] | unit_comp[units] | cnt[K] off[K] cursor[K] | n_units | dense_flag
-    const int64_t p_units = (int64_t)pair_cap * (chunk / bucket_rows) + m->n_comp + 1, p_rows = p_units * bucket_rows;
+    const int64_t p_units = (int64_t)TC_PAIR_CAP * (chunk / bucket_rows) + m->n_comp + 1, p_rows = p_units * bucket_rows;
     int *p_perm = nullptr, *p_ucomp = nullptr, *p_cnt = nullptr, *p_off = nullptr, *p_cur = nullptr, *p_nu = nullptr, *p_dense = nullptr;
     float* p_w = nullptr;
     if (pairs && !bucketed) {
@@ -2152,21 +1955,12 @@ static qce_status tc_run_modes(qce_model* m, TileScratch* ts, cudaStream_t s, in
             const unsigned char* vb = (const unsigned char*)v.bad;
             const int K = m->n_comp;
             if (K <= 256) {
-#define QCE_SEL_ROWS(R)                                                                                                                        \
-                {                                                                                                                              \
-                    const size_t sm = (size_t)2 * K * (R + 1) * sizeof(float) + (size_t)K * sizeof(int);                                      \
-                    static PerDeviceOnce once;                                                                                                 \
-                    if (once.first(current_device()))                                                                                          \
-                        QCE_CUDA_TRY(cudaFuncSetAttribute(tc_select_rows_kernel<R>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024)); \
-                    tc_select_rows_kernel<R><<<(unsigned)((nb + R - 1) / R), SEL_THREADS, sm, s>>>((const float2*)v.lp2, nb, K, mode, n_top, rho, m->flags, wts, lo, \
-                        b_top, vb, ts->tie_buf, eps, m->logc, 1.0 / m->n_obs, fused_count ? p_cnt : nullptr, pair_thresh,                     \
-                        listed ? l_key : nullptr);                                                                                             \
-                }
-                // pilots per block: the smaller the tile, the more blocks (loads in flight) per SM -- measured at K = 64, 2^19 pilots:
-                // 128 pilots 265 us, 64: 222 us, 32: 198 us (QCE_SEL_R overrides: A/B runs)
-                const int sel_r = getenv("QCE_SEL_R") ? atoi(getenv("QCE_SEL_R")) : 32;
-                if (sel_r == 16) QCE_SEL_ROWS(16) else if (sel_r == 64 && K <= 128) QCE_SEL_ROWS(64) else if (sel_r == 128 && K <= 64) QCE_SEL_ROWS(128) else QCE_SEL_ROWS(32)
-#undef QCE_SEL_ROWS
+                const size_t sm = (size_t)2 * K * (SEL_ROWS + 1) * sizeof(float) + (size_t)K * sizeof(int);
+                static PerDeviceOnce once;
+                if (once.first(current_device()))
+                    QCE_CUDA_TRY(cudaFuncSetAttribute(tc_select_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+                tc_select_rows_kernel<<<(unsigned)((nb + SEL_ROWS - 1) / SEL_ROWS), SEL_THREADS, sm, s>>>((const float2*)v.lp2, nb, K, mode, n_top, rho, m->flags,
+                    wts, lo, b_top, vb, ts->tie_buf, eps, m->logc, 1.0 / m->n_obs, fused_count ? p_cnt : nullptr, pair_thresh);
             } else {
                 tc_select_kernel<32><<<(unsigned)((nb + 7) / 8), 256, 0, s>>>((const float2*)v.lp2, nb, K, mode, n_top, rho, m->flags, wts, lo, b_top, vb, ts->tie_buf, eps, nullptr, m->logc, 1.0 / m->n_obs);
             }
@@ -2201,25 +1995,6 @@ static qce_status tc_run_modes(qce_model* m, TileScratch* ts, cudaStream_t s, in
             QCE_CHECK_LAUNCH("tc_bucket kernels");
             for (int part = 0; part < m->tc.h_parts; ++part) {
                 st = tc_run_split(m, &v, s, cap_rows, 2, part, he, ht, h_true_c64, acc, b_ucomp, b_perm, b_nu, ts->img2);
-                if (st) return st;
-            }
-            continue;
-        }
-        if (listed) {
-            const unsigned g1 = (unsigned)((nb + 1023) / 1024);
-            QCE_CUDA_TRY(cudaMemsetAsync(l_cnt, 0, m->n_comp * sizeof(int), s));
-            QCE_CUDA_TRY(cudaMemsetAsync(l_perm, 0xFF, (size_t)cap_rows * sizeof(int), s));        // -1 = padding slot
-            tc_bucket_count_kernel<<<g1, 1024, 0, s>>>(l_key, nb, m->n_comp, l_cnt);
-            tc_bucket_scan_kernel<<<1, 1024, 0, s>>>(l_cnt, m->n_comp, bucket_rows, l_off, l_cur, l_ucomp, l_nu);
-            tc_bucket_place_kernel<<<g1, 1024, 0, s>>>(l_key, nb, m->n_comp, l_off, l_cur, l_perm);
-            tc_bucket_gather_kernel<<<(unsigned)(cap_rows / TILE_M), 256, 0, s>>>((const unsigned char*)v.img, l_perm, l_nu, tiles_per_unit,
-                                                                                  2 * m->n_obs / 8, m->tc.split_a ? 2 : 1, (unsigned char*)ts->img2);
-            tc_unit_list_kernel<<<(unsigned)cap_units, 256, 0, s>>>((const float*)v.wts, l_perm, l_nu, bucket_rows, m->n_comp, l_list, l_nk);
-            QCE_CHECK_LAUNCH("listed combination: bucket / list kernels");
-            count_launch(4);
-            for (int part = 0; part < m->tc.h_parts; ++part) {
-                st = tc_run_split(m, &v, s, cap_rows, 2, part, he, ht, h_true_c64, acc, nullptr, l_perm, l_nu, ts->img2, nullptr, nullptr, nullptr, 0,
-                                  l_list, l_nk);
                 if (st) return st;
             }
             continue;
@@ -2456,31 +2231,6 @@ qce_status launch_pipeline_tc(qce_model* m, const QuantTables* qt, cudaStream_t 
     if (st) return st;
     RowSource obs_src;          // where the complex128 re-evaluation of flagged rows finds the pilots: it observes + quantises them again
     obs_src.obs_h = h; obs_src.obs_noise = noise; obs_src.obs_noise_scale = noise_scale; obs_src.obs_h_c64 = h_is_c64; obs_src.qt = *qt;
-    // Fused prologue (QCE_TC_FUSE=1): ONE launch observes, quantises, formats and estimates (mode 'all', fused shapes, 1-bit pilots,
-    // SM-pair variant, K a multiple of the items per warp): the epilogue warps build the NEXT work unit's tiles one core matrix per
-    // component.  Bit-identical results, but no faster than the formatter launch + estimate launch pair (4.78 vs 4.79 ms per 2^20
-    // pilots): the kernel is power-limited, so the formatter's energy costs the same time inside it as outside.  Default: the pair.
-    {
-        const char* fe = getenv("QCE_TC_FUSE");
-        const bool want = fe && atoi(fe) == 1;
-        const int cz = m->n_obs / 16, ch = m->n_ant / 16;
-        const int ipw = 2 * 16 * (2 * m->n_obs / 8) / 8;            // items of a work unit per epilogue warp (see FMT_IPW)
-        const bool k_ok = m->n_comp >= ipw && m->n_comp % ipw == 0;      // one item per warp every K / ipw components
-        if (want && k_ok && qt->n_bits == 1 && mode == QCE_MODE_ALL && !m->tc.split && !m->tc.split_a && m->tc.triangular && cz == ch && (cz == 4 || cz == 2)) {
-            QCE_CUDA_TRY(cudaMemsetAsync(ts->bad, 0, ts->bad_bytes, s));      // off-grid rows are flagged with atomicOr
-            TcArgs a;
-            tc_fill_args(m, ts, B, h_est, h, h_is_c64, acc, &a);
-            a.obs_h = h; a.obs_noise = (const double2*)noise; a.obs_noise_scale = noise_scale; a.obs_noise_scale_f = (float)noise_scale; a.obs_inv_scale = 1.0 / m->tc.eff_scale;
-            a.obs_h_c64 = h_is_c64; a.obs_bits = qt->n_bits; a.obs_n_thr = qt->n_thr; a.obs_thr = qt->thr; a.obs_labels = qt->labels;
-            ts->owner = m; ts->rows = B;
-            ts->src = obs_src;
-            const bool offs = m->tc.has_offsets;
-            if (cz == 4) st = offs ? launch_cfg<4, 4, 4, true, 2, 0, 0, 1, true>(a, s) : launch_cfg<4, 4, 4, false, 2, 0, 0, 1, true>(a, s);
-            else st = offs ? launch_cfg<2, 2, 2, true, 2, 0, 0, 1, true>(a, s) : launch_cfg<2, 2, 2, false, 2, 0, 0, 1, true>(a, s);
-            if (st) return st;
-            return tc_fix_rows(m, ts, s, B, mode, n_top, rho, h_est, nullptr, h, h_is_c64, acc);
-        }
-    }
     const int64_t tiles = (B + TILE_M - 1) / TILE_M;
     const size_t smem = (size_t)(m->tc.split_a ? 2 : 1) * (2 * m->n_obs / 8) * 128 + ((qt->n_bits > 1) ? (size_t)(2 * qt->n_thr + 1) * sizeof(double) : 0);
     const unsigned grid = (unsigned)(tiles * (TILE_M / 8));

@@ -33,8 +33,6 @@ struct TcArgs {
     const unsigned char* bad;  // [n_tiles * 128] rows the tensor-core path cannot answer (data not on the quantiser grid): their
                                // estimates are neither written nor accumulated here; they are on the fix list and re-evaluated
                                // completely by the complex128 kernel after the tensor-core launches
-    int* fix_idx;              // [rows] the fix list (rows of the formatted batch)
-    int* fix_cnt;              // its length (device side)
     int* tie_buf;              // EPI=1 label mode: [0] count, then the rows of this launch whose top-1 selection is too close to
     float tie_eps, inv_nobs;   // call (deciding log-likelihood gap below tie_eps nats, times q / n_obs of the best component when
                                // that exceeds one): tc_refine_kernel + the exact selection re-select them
@@ -54,26 +52,11 @@ struct TcArgs {
     int h_col0;
     int count_rows;            // add the number of rows to acc[2] (only one of the H-part launches does)
     int wide_io;               // h_est and h_true are 32-byte aligned: rows are written / read with 256-bit accesses
-    // fused prologue (PRO kernels): the kernel observes + quantises + formats its own pilot tiles into a_img / bad
-    const void* obs_h;         // [B][No] c64 / c128 channels
-    const double2* obs_noise;  // [B][No] c128
-    double obs_noise_scale, obs_inv_scale;
-    float obs_noise_scale_f;
-    int obs_h_c64, obs_bits, obs_n_thr;
-    const double* obs_thr;     // device quantiser tables (b > 1)
-    const double* obs_labels;
-    float skip_thresh;         // fused 'all' epilogue: a warp skips the LMMSE row of a component whose un-normalised weight is below
-                               // this for all of its 32 pilots (the normaliser is >= 1, so the dropped terms are < skip_thresh each)
     // bucketed top-1 combination (EPI=2, all three null otherwise): the pilots were regrouped by their selected component, work
     // unit u holds pilots of component unit_comp[u] only and runs that ONE component; slot -> pilot through perm (-1 = padding)
     const int* unit_comp;      // [*n_units_dev]
     const int* perm;           // [B] (B = slot capacity of the launch)
     const int* n_units_dev;    // number of work units actually filled (device-side: the bucket sizes are data)
-    // listed combination (EPI=2; top-n / cumulative modes at the fused shapes): the pilots are regrouped by their BEST component (perm,
-    // n_units_dev as above), unit u runs the unit_nk[u] components unit_list[u * K ..] -- those some pilot of the unit has a non-zero
-    // weight for -- with the dense weight rows w_in[pilot][k]
-    const int* unit_list;      // [units][K]
-    const int* unit_nk;        // [units]
     // pair mode of the bucketed combination (top-n / cumulative / sparse 'all'): a slot is one (pilot, component) pair with the
     // combination weight slot_w[slot]; a pilot has several slots in different units, so the weighted LMMSE rows are ADDED to the
     // pilot's (zero-initialised) FP32 row with vector reductions; tc_pair_finish_kernel turns the rows into estimates + NMSE sums

@@ -705,11 +705,10 @@ def test_tc_parameter_scales_and_extreme_snr(qce, scale, snr, nb):
 
 
 @pytest.mark.parametrize('K,N,c64', [(64, 64, True), (128, 64, False), (32, 32, True)])
-def test_tc_fused_prologue_variant(qce, K, N, c64):
-    """QCE_TC_FUSE=1: the estimate kernel builds its own pilot tiles (observe + 1-bit quantise + format in the epilogue warps, FP32
-    sign decision with an exact FP64 fallback near cancellation); results must be identical to the formatter + estimate launch pair,
-    including NaN rows and a ragged tail over several work units per CTA."""
-    import os
+def test_tc_pipeline_nan_zero_and_ragged_tail(qce, K, N, c64):
+    """The fused Monte-Carlo step (observe + 1-bit quantise + estimate) on the tensor-core path against the complex128 path on the same
+    inputs: a NaN noise entry (its row is NaN, like numpy), an element with y = 0 exactly, complex64 and complex128 channels, and a
+    ragged tail over several work units per CTA."""
     from quantized_channel_estimation_b200 import engine, precompute
     B, snr = 148 * 512 * 2 + 777, 5
     means, covs, w = orc.random_psd_gmm(K, N, seed=K + N, mean_scale=0.1)
@@ -720,25 +719,15 @@ def test_tc_fused_prologue_variant(qce, K, N, c64):
     noise = torch.view_as_complex(torch.randn((B, N, 2), generator=g, device='cuda', dtype=torch.float64)).contiguous()
     noise[5, 3] = complex(float('nan'), 0.0)
     h[B - 2, 0] = 0.0
-    noise[B - 2, 0] = 0.0                          # y = 0 exactly: np.sign gives 0, both paths must carry the value 0 (FP64 fallback)
-    est0, acc0 = model.pipeline(quant, h, noise, 10 ** (-snr / 20), 'all', 'tc', want_est=True)
-    os.environ['QCE_TC_FUSE'] = '1'
-    try:
-        l0 = _launches()
-        est1, acc1 = model.pipeline(quant, h, noise, 10 ** (-snr / 20), 'all', 'tc', want_est=True)
-        assert _launches() - l0 == 2                # one estimate launch + the complex128 launch that answers off-grid / NaN rows
-    finally:
-        del os.environ['QCE_TC_FUSE']
-    ok = ~torch.isnan(est0.real).any(dim=1)
-    assert bool(torch.isnan(est0[5].real).all()) and bool(torch.isnan(est1[5].real).all())
-    assert torch.equal(torch.isnan(est0.real), torch.isnan(est1.real))
-    assert torch.equal(est0[ok], est1[ok])
-    assert acc0[2].item() == acc1[2].item() == B
-
-
-def _launches():
-    from quantized_channel_estimation_b200 import _lib
-    return _lib.launch_count()
+    noise[B - 2, 0] = 0.0                          # y = 0 exactly: np.sign gives 0, both paths must carry the value 0
+    est, acc = model.pipeline(quant, h, noise, 10 ** (-snr / 20), 'all', 'tc', want_est=True)
+    est64, _ = model.pipeline(quant, h, noise, 10 ** (-snr / 20), 'all', 'fp64', want_est=True)
+    assert bool(torch.isnan(est[5].real).all()) and bool(torch.isfinite(est[B - 2]).all())
+    assert torch.equal(torch.isnan(est.real), torch.isnan(est64.real))
+    ok = ~torch.isnan(est64.real).any(dim=1)
+    per = (est[ok] - est64[ok]).norm(dim=1) / est64[ok].norm(dim=1).clamp(min=1e-300)
+    assert float((est[ok] - est64[ok]).norm() / est64[ok].norm()) < TOL_TC and float(per.max()) < 1e-4
+    assert acc[2].item() == B
 
 
 def test_tc_single_component_and_many_components(qce):
@@ -815,28 +804,6 @@ def test_tc_non_triangular_whitening_uses_single_cta_variant(qce):
         assert relerr(est, ref) < TOL_TC
         est64 = model.estimate(rt, 'all', 'fp64').cpu().numpy()
         assert relerr(est64, ref) < 1e-9
-
-
-def test_tc_single_cta_variant_env(qce):
-    """QCE_TC_CG=1 forces the cta_group::1 kernel (read once per process): run it in a subprocess."""
-    import os, subprocess, sys
-    code = (
-        "import numpy as np, torch, sys\n"
-        "sys.path.insert(0, %r)\n"
-        "from oracle import qce_oracle as orc\n"
-        "import quantized_channel_estimation_b200 as qce\n"
-        "K,N,B,snr=5,64,900,5\n"
-        "means,covs,w=orc.random_psd_gmm(K,N,seed=3)\n"
-        "h,noise,_=orc.sample_gmm_channels(means,covs,w,B,seed=4)\n"
-        "r=orc.get_observation_nbit(h,snr,noise,None,1)\n"
-        "m=qce.Gmm_nbit(n_components=K).set_parameters(means,covs,w,detect_structure=False); m.precision='tc'\n"
-        "est=m.estimate_from_y(torch.from_numpy(r).cuda(),snr,N,n_summands_or_proba='all').cpu().numpy()\n"
-        "ref=orc.gmm_estimate_from_y(means,covs,w,r,snr,n_summands_or_proba='all',n_bits=1)\n"
-        "print('RELERR', np.linalg.norm(est-ref)/np.linalg.norm(ref))\n") % os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    out = subprocess.run([sys.executable, '-c', code], env=dict(os.environ, QCE_TC_CG='1'), capture_output=True, text=True, timeout=300)
-    assert out.returncode == 0, out.stderr[-2000:]
-    err = float([l for l in out.stdout.splitlines() if l.startswith('RELERR')][0].split()[1])
-    assert err < TOL_TC
 
 
 @pytest.mark.gpu
@@ -1207,38 +1174,6 @@ def test_estimate_from_codes_host_path(qce, nb, qt):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize('K,blocks,mode', [(128, (16, 16), 'all'), (64, (16, 16), 3), (128, (1, 256), 0.9), (64, (1, 256), 'all')])
-def test_circulant_tcgen05_variant(qce, K, blocks, mode):
-    """QCE_CIRC_UMMA=1: the two contractions of the DFT-domain kernel on tcgen05 (TMEM accumulators, rt parked in TMEM, bulk-TMA parameter
-    ring) against the mma.sync version of the same kernel and the complex128 kernel -- ragged batch, both transform variants, K = 64 / 128."""
-    import os
-    N, B, snr, nb, qt = 256, 1000 + 17, 8, 3, 'lloyd'
-    from quantized_channel_estimation_b200 import synthetic
-    c, _, w, _ = synthetic.circulant_gmm(K, *blocks, seed=K, dense=False)
-    qz = orc.get_quantizer([snr], nb, qt)[snr]
-    g = torch.Generator(device='cuda').manual_seed(5)
-    y = torch.view_as_complex(torch.randn((B, N, 2), generator=g, device='cuda', dtype=torch.float64)) * 0.8
-    r = qce.quant(y, nb, qz[0], qz[1])
-    h = torch.view_as_complex(torch.randn((B, N, 2), generator=g, device='cuda', dtype=torch.float64))
-    m = qce.Gmm_nbit(n_components=K, covariance_type='block-circulant')
-    m.set_circulant_parameters(c, w, blocks)
-    model = m._prepared(np.eye(N), snr, nb, qt, qz)
-    os.environ['QCE_CIRC_UMMA'] = '1'
-    try:
-        e1, lp1, acc1 = model.estimate(r, mode, 'tc', want_logp=True, h_true=h)
-    finally:
-        del os.environ['QCE_CIRC_UMMA']
-    e0, lp0, acc0 = model.estimate(r, mode, 'tc', want_logp=True, h_true=h)
-    e64 = model.estimate(r, mode, 'fp64')
-    per = (e1 - e64).norm(dim=1) / e64.norm(dim=1).clamp(min=1e-300)
-    assert float((e1 - e64).norm() / e64.norm()) < TOL_TC and float(per.max()) < 1e-4
-    assert float((e1 - e0).norm() / e0.norm()) < TOL_TC
-    assert float((lp1 - lp0).abs().max()) < 2e-3
-    np.testing.assert_allclose(acc1.cpu().numpy(), acc0.cpu().numpy(), rtol=1e-4)
-    assert acc1[2].item() == B
-
-
-@pytest.mark.gpu
 def test_predict_proba_right_after_set_parameters_uses_the_trained_mixture(qce):
     """ADVICE r1: with no observation setting prepared yet, predict_proba / predict_proba_cplx are the responsibilities under the
     trained (channel-domain) mixture -- what the reference computes right after fit() -- instead of an error."""
@@ -1266,31 +1201,6 @@ def test_predict_proba_right_after_set_parameters_uses_the_trained_mixture(qce):
         m.fit(hm[:1500], zero_mean=False)
     p = m.predict_proba(hm[:200])
     assert p.shape == (200, 3) and np.allclose(p.sum(1), 1.0, atol=1e-6)
-
-
-@pytest.mark.gpu
-@pytest.mark.parametrize('mode', [2, 4, 0.9])
-def test_tc_listed_combination(qce, mode):
-    """QCE_TC_LISTED=1: top-n / cumulative rho with the pilots regrouped by their best component and every work unit running only the
-    components its pilots selected -- same estimates as the weighted launch over all K components, and the oracle's."""
-    import os
-    K, N, B, snr = 32, 64, 12000, 10
-    means, covs, w, h, noise, qz, r = _case(K, N, B, snr, 1, 'uniform', 0.1, seed=77)
-    m = qce.Gmm_nbit(n_components=K).set_parameters(means, covs, w, detect_structure=False)
-    m.precision = 'tc'
-    rt, ht = torch.from_numpy(r).cuda(), torch.from_numpy(h).cuda()
-    model = m._prepared(np.eye(N), snr, 1, 'uniform', None)
-    est0, acc0 = model.estimate(rt, mode, 'tc', h_true=ht)
-    os.environ['QCE_TC_LISTED'] = '1'
-    try:
-        est1, acc1 = model.estimate(rt, mode, 'tc', h_true=ht)
-    finally:
-        del os.environ['QCE_TC_LISTED']
-    assert torch.equal(est0, est1)                     # same weights, same accumulation order per pilot
-    np.testing.assert_allclose(acc1.cpu().numpy(), acc0.cpu().numpy(), rtol=1e-9)
-    ref = orc.gmm_estimate_from_y(means, covs, w, r[:2000], snr, n_summands_or_proba=mode, n_bits=1)
-    per = np.linalg.norm(est1[:2000].cpu().numpy() - ref, axis=1) / np.linalg.norm(ref, axis=1)
-    assert per.max() < 1e-4
 
 
 @pytest.mark.gpu
@@ -1324,7 +1234,7 @@ def test_two_gpus_in_one_process(qce):
 @pytest.mark.parametrize('K,N,nb,qt,B', [(8, 64, 1, 'uniform', 900), (6, 128, 2, 'uniform', 700), (5, 48, 3, 'lloyd', 500), (4, 40, 1, 'uniform', 300)])
 def test_tc_launch_time_knobs_do_not_change_results(qce, K, N, nb, qt, B, monkeypatch):
     """Every launch-time knob of the tensor-core path (DESIGN.md knobs table) selects another route to the SAME estimates: all pilots sent
-    through the complex128 re-selection (QCE_TC_TIE_EPS=0.5), pair-bucketed / listed / weighted combination, bucketed top-1 off -- on the
+    through the complex128 re-selection (QCE_TC_TIE_EPS=0.5), pair-bucketed / weighted combination, bucketed top-1 off -- on the
     fused shape, the split path, the three-pass path and a zero-padded shape, all four modes, with some pilots off the grid."""
     snr = 10
     means, covs, w, h, noise, qz, r = _case(K, N, B, snr, nb, qt, 0.1, seed=K)
@@ -1340,7 +1250,7 @@ def test_tc_launch_time_knobs_do_not_change_results(qce, K, N, nb, qt, B, monkey
     base = {mode: m.estimate_from_y(rt, snr, N, n_summands_or_proba=mode, **kw) for mode in modes}
     for mode in modes:
         assert relerr(base[mode].cpu().numpy(), ref[mode].cpu().numpy()) < TOL_TC
-    for knob, val in (('QCE_TC_TIE_EPS', '0.5'), ('QCE_TC_PAIRS', '1'), ('QCE_TC_PAIRS', '0'), ('QCE_TC_LISTED', '1'), ('QCE_TC_BUCKET', '0')):
+    for knob, val in (('QCE_TC_TIE_EPS', '0.5'), ('QCE_TC_PAIRS', '1'), ('QCE_TC_PAIRS', '0'), ('QCE_TC_BUCKET', '0')):
         monkeypatch.setenv(knob, val)
         for mode in modes:
             got = m.estimate_from_y(rt, snr, N, n_summands_or_proba=mode, **kw)
@@ -1442,7 +1352,7 @@ def test_batches_beyond_4_gib_dense(qce):
 
 @pytest.mark.gpu
 def test_batches_beyond_4_gib_circulant(qce):
-    """The same for the DFT-domain kernels (N = 256: 4 KiB per row -> 2^20 rows = 4 GiB), both tensor-core variants."""
+    """The same for the DFT-domain kernels (N = 256: 4 KiB per row -> 2^20 rows = 4 GiB)."""
     from quantized_channel_estimation_b200 import synthetic
     K, N, B, snr = 64, 256, (1 << 20) + (1 << 18) + 5, 10
     c, _, w, _ = synthetic.circulant_gmm(K, 16, 16, seed=2, dense=False)
@@ -1456,11 +1366,6 @@ def test_batches_beyond_4_gib_circulant(qce):
     del y
     kw = dict(n_bits=3, quantizer_type='lloyd', quantizer=qz)
     _tail_invariance(m, r, snr, N, ('all', 1, 0.9), kw, tail=3000)
-    os.environ['QCE_CIRC_UMMA'] = '1'
-    try:
-        _tail_invariance(m, r, snr, N, ('all',), kw, tail=3000)
-    finally:
-        del os.environ['QCE_CIRC_UMMA']
 
 
 @pytest.mark.gpu

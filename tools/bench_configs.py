@@ -99,7 +99,7 @@ def main():
     mf.use_structure = False
     mf.precision = 'tc'
     for tag, r in (('white-noise pilots', pilots(1 << 19, 128, 2, qz)), ('model-drawn pilots 10 dB', model_pilots(mf.covs, amps, 1 << 19, snr, 2, qz))):
-        for mode, env in (('all', {}), ('all', {'QCE_TC_SPARSE_ALL': '0'}), (1, {}), (4, {}), (0.9, {})):
+        for mode, env in (('all', {}), ('all', {'QCE_TC_PAIRS': '0'}), (1, {}), (4, {}), (0.9, {})):
             os.environ.update(env)
             ms = timeit(lambda: mf.estimate_from_y(r, snr, n_summands_or_proba=mode, n_bits=2, quantizer_type='uniform', quantizer=qz))
             for k in env:

@@ -26,7 +26,7 @@ def main():
     for prec in os.environ.get('PREC', 'tc').split(','):
         ms = timeit(lambda: model.estimate(r, 'all', prec), reps=int(os.environ.get('REPS', 5)))
         print(json.dumps(dict(config=f'C3 K={K}', precision=prec, B=B, ms=ms, est_per_s=B / ms * 1e3, gbytes_per_s=32 * 256 * B / ms / 1e6)), flush=True)
-    # interleaved A/B of launch-time knobs (QCE_CIRC_PREFETCH = tiles ahead, QCE_CIRC_NW = warps per CTA): AB="PREFETCH=0;PREFETCH=148;NW=16"
+    # interleaved A/B of launch-time knobs (QCE_CIRC_PREFETCH = tiles ahead): AB="PREFETCH=0;PREFETCH=148"
     ab = [x for x in os.environ.get('AB', '').split(';') if x]
     if ab:
         res = {x: [] for x in ab}

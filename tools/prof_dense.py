@@ -1,6 +1,7 @@
 #!/usr/bin/env python
-"""The dominant kernel alone (config 2: GMM full, 1 bit, N=64, K=64; qce_format_pilots once, then qce_estimate_formatted in a loop) with
-an interleaved in-process A/B of launch-time knobs:  AB="SKIP=1e-30;SKIP=1e-12" python tools/prof_dense.py   (QCE_TC_<KEY>=<value>)."""
+"""The dominant kernel alone (config 2: GMM full, 1 bit, N=64, K=64; qce_format_pilots once, then qce_estimate_formatted in a loop),
+optionally as an interleaved in-process A/B of launch-time knobs:  AB="<KEY>=<a>;<KEY>=<b>" python tools/prof_dense.py
+(QCE_TC_<KEY>=<value>; without AB the default route alone)."""
 import ctypes as C
 import json
 import os
@@ -25,7 +26,7 @@ def main():
     lib = _lib.load()
     stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
     out = torch.empty((B, N), dtype=torch.complex128, device='cuda')
-    ab = [x for x in os.environ.get('AB', 'SKIP=1e-12').split(';') if x]
+    ab = [x for x in os.environ.get('AB', '').split(';') if x] or ['']
     for snr in snrs:
         r = qce.get_observation_nbit(torch.from_numpy(h).cuda(), snr, n_bits=1, noise=torch.from_numpy(noise).cuda()).repeat(B >> 14, 1).contiguous()
         model = engine.DenseModel(precompute.prepare(means, covs, w, np.eye(N), snr, 1))
@@ -34,12 +35,12 @@ def main():
         res = {x: [] for x in ab}
         for _ in range(int(os.environ.get('ROUNDS', 5))):
             for x in ab:
-                for kv in x.split(','):
-                    k, v = kv.split('=')
+                kvs = [kv.split('=') for kv in x.split(',') if kv]
+                for k, v in kvs:
                     os.environ['QCE_TC_' + k] = v
                 res[x].append(timeit(run, reps=3))
-                for kv in x.split(','):
-                    os.environ.pop('QCE_TC_' + kv.split('=')[0])
+                for k, _ in kvs:
+                    os.environ.pop('QCE_TC_' + k)
         for x in ab:
             v = sorted(res[x])
             ms = v[len(v) // 2]
