@@ -287,7 +287,7 @@ static qce_status estimate_impl(qce_model* m, cudaStream_t s, const double* r, i
         return launch_dense_fp64_raw(m, s, r, B, mode, n_top, rho, h_est, logp_out, h_true, h_true_c64, acc);
     if (precision == QCE_PREC_TC) {
         if (!tc_supported(m, mode) || !m->tc.ready) {
-            set_error("tensor-core kernel does not support n_obs=%d n_ant=%d K=%d mode=%d", m->n_obs, m->n_ant, m->n_comp, mode);
+            set_error("tensor-core kernel does not support n_obs=%d n_ant=%d K=%d mode=%d%s", m->n_obs, m->n_ant, m->n_comp, mode, tc_unsupported_reason(m));
             return QCE_ERR_UNSUPPORTED;
         }
         return launch_dense_tc(m, s, r, B, mode, n_top, rho, h_est, logp_out, h_true, h_true_c64, acc);
@@ -316,7 +316,7 @@ qce_status qce_pipeline(qce_model* m, const qce_quantizer* q, void* stream, cons
     }
     if (precision == QCE_PREC_TC) {
         if (!tc_supported(m, mode) || !m->tc.ready) {
-            set_error("tensor-core kernel does not support n_obs=%d n_ant=%d K=%d mode=%d", m->n_obs, m->n_ant, m->n_comp, mode);
+            set_error("tensor-core kernel does not support n_obs=%d n_ant=%d K=%d mode=%d%s", m->n_obs, m->n_ant, m->n_comp, mode, tc_unsupported_reason(m));
             return QCE_ERR_UNSUPPORTED;
         }
         // one formatter launch (observe + quantise + FP16 tiles) and one estimate launch per 2^22 pilots

@@ -77,11 +77,11 @@ struct TcParams {
     // r / eff_scale, three tensor passes
     bool split_a = false;
     double eff_scale = 0.0;     // data_scale, or 2^-8 when split_a
-    // split path (n_obs or n_ant above 64): a whitening-only image and up to two LMMSE row-block images; the estimate runs as
-    // log-probability launch -> selection -> one launch per row block
+    // split path (n_obs or n_ant above 64): a whitening-only image and up to four LMMSE row-block images (n_ant = 256: four blocks
+    // of 128 columns); the estimate runs as log-probability launch -> selection -> one launch per row block
     bool split = false;
     void* image_z = nullptr;
-    void* image_h[2] = {nullptr, nullptr};
+    void* image_h[4] = {nullptr, nullptr, nullptr, nullptr};
     int h_parts = 0;            // number of row-block launches
     int part_cols = 0;          // real columns (of the 2 n_ant) per row block
 };
@@ -286,6 +286,7 @@ qce_status launch_pipeline_tc(qce_model* m, const QuantTables* qt, cudaStream_t 
                               const double* noise, double noise_scale, int64_t B, int mode, int n_top, double rho, double* h_est,
                               double* acc);
 bool tc_supported(const qce_model* m, int mode);
+const char* tc_unsupported_reason(const qce_model* m);      // "" or ": <why>", appended to the error message
 void tc_scratch_release(cudaStream_t s);
 // qce_mfa.cu
 qce_status launch_mfa(const qce_mfa_model* m, cudaStream_t s, const double* r, int64_t B, int mode, int n_top, double rho,

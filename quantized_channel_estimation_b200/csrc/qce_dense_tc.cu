@@ -45,6 +45,12 @@ __host__ __device__ constexpr int tc2_sub_off(int nt, int tri16, int ksps, int h
     return 16 * (s2 * nt - tri16 * (s2 * half * ksps + s2 * (s2 - 1) / 2));
 }
 __host__ __device__ constexpr int tc2_chunk_bytes(int nt, int tri16, int ksps, int half) { return tc2_sub_off(nt, tri16, ksps, half, ksps); }
+// byte offset of K-step ks's sub-block from the start of its pass image (the sub-blocks of a pass are stored in K-step order)
+__host__ __device__ constexpr int tc2_ks_off(int nt, int tri16, int ks) { return 16 * (ks * nt - tri16 * (ks * (ks - 1) / 2)); }
+// A K-step whose N' exceeds the 256 columns of one MMA (the whitening block of n_obs = 256: NT = 512) is issued as two MMAs, rows
+// [skip, 256) and [256, NT); each piece is split between the two CTAs on its own (rank 0 holds the first half of the piece's rows),
+// and the per-rank sub-block holds the first piece's rows, then the second's.  Width of the first piece:
+__host__ __device__ constexpr int tc2_piece0(int np) { return np > 256 ? np - 256 : np; }
 __host__ __device__ constexpr int tc2_rank_comp_bytes(int nt, int tri16, int ksps) {
     return 2 * (tc2_chunk_bytes(nt, tri16, ksps, 0) + tc2_chunk_bytes(nt, tri16, ksps, 1));
 }
@@ -73,13 +79,24 @@ struct TcCfg {
     static constexpr int A_TILE_BYTES = AC * A_COPY_BYTES;
     // resident pilot tiles per CTA: two (their epilogues ping-pong), or one when the (hi, lo) tile pairs of the large shapes would
     // not leave room for the operand ring (the second epilogue warpgroup then idles and the accumulator is not double-buffered)
-    static constexpr int NTILES = (AC == 2 && KD > 128) ? 1 : TILES;
+    // (n_obs = 256: one pilot tile is 128 KB, so there is one per CTA whatever AC is)
+    static constexpr int NTILES = ((AC == 2 && KD > 128) || KD > 256) ? 1 : TILES;
     static constexpr int KSPS = KD / 32;                            // K-steps (of 16) per staged chunk = half the K range
     // CG=1: a chunk is one K-half of the stacked hi (or lo) image, 4 chunks per component.
-    // CG=2: a chunk is this CTA's share of the whole hi (or lo) image (triangular layout), 2 chunks per component.
-    static constexpr int NCHUNK = (CG == 2) ? 2 : 4;
+    // CG=2: a chunk is this CTA's share of the whole hi (or lo) image (triangular layout), 2 chunks per component -- or, at KD = 512
+    // (KSLICED), of a K-slice of KSLICE K-steps: a whole pass is 132 KB (whitening) / 64 KB (row block) there, which does not fit next
+    // to the 128 KB pilot tile; a slice is at most 31 KB / 8 KB, 2 KD / (16 KSLICE) chunks per component.
+    static constexpr bool KSLICED = CG == 2 && KD > 256;
+    static constexpr int KSLICE = KSLICED ? 4 : KD / 16;            // K-steps per chunk (CG=2)
+    static constexpr int CPP = (KD / 16) / KSLICE;                  // chunks per pass (CG=2)
+    static constexpr int NCHUNK = (CG == 2) ? 2 * CPP : 4;
     static constexpr int CB0 = tc2_chunk_bytes(NT, TRI16, KSPS, 0), CB1 = tc2_chunk_bytes(NT, TRI16, KSPS, 1);
-    static constexpr int STAGE_BYTES = (CG == 2) ? (CB0 + CB1) : NT * (KD / 2) * 2;
+    static constexpr int PASS_BYTES = CB0 + CB1;                    // CG=2: this CTA's share of one pass (hi or lo)
+    // (the first K-slice of a pass is its largest)
+    static constexpr int STAGE_BYTES = (CG == 2) ? (KSLICED ? tc2_ks_off(NT, TRI16, KSLICE) : PASS_BYTES) : NT * (KD / 2) * 2;
+    // CG=2: chunk q = K-slice q % CPP of pass q / CPP, at this byte offset of the CTA's component image, this long
+    __host__ __device__ static constexpr int chunk_off(int q) { return (q / CPP) * PASS_BYTES + tc2_ks_off(NT, TRI16, (q % CPP) * KSLICE); }
+    __host__ __device__ static constexpr int chunk_bytes(int q) { return tc2_ks_off(NT, TRI16, (q % CPP + 1) * KSLICE) - tc2_ks_off(NT, TRI16, (q % CPP) * KSLICE); }
     static constexpr int CTRL_BYTES = 1024;
     static constexpr int STAGES_FIT = (SMEM_LIMIT - NTILES * A_TILE_BYTES - CTRL_BYTES) / STAGE_BYTES;
     // (more than 8 stages do not help -- the whitening-only launch waits as long for operands with 16 -- and the weighted combine
@@ -95,7 +112,8 @@ struct TcCfg {
     static_assert(NZ == 0 || NZ == KD, "the whitening block is square");
     static_assert(NT >= 32, "empty launch");
     static_assert(STAGE_BYTES % 128 == 0, "stage alignment");
-    static_assert(NT <= 256, "fused MMA N exceeds 256");
+    static_assert(NT <= 256 || (KSLICED && NH == 0 && NT <= 512), "fused MMA N exceeds 256 (wider: whitening-only K-sliced launch)");
+    static_assert(!KSLICED || (AC == 1 && ORDER == 1 && (KD / 16) % KSLICE == 0), "K-sliced chunks: on-grid pilots, chunk-major order");
     static_assert(TMEM_COLS_USED <= 512, "accumulators exceed TMEM");
 };
 
@@ -118,15 +136,28 @@ __device__ __forceinline__ void tc_issue_chunk(const int q, const uint32_t d_til
     constexpr uint32_t A_LBO = (TILE_M / 8) * 128;                              // SBO = 128 for both operands
     constexpr uint32_t DESC_HI = (128u >> 4) | (1u << 14);                      // SBO field | descriptor version 1
     constexpr uint32_t IDESC0 = (1u << 4) | ((uint32_t)((CG * TILE_M) >> 4) << 24);
-    constexpr int KS_PER_CHUNK = (CG == 2) ? 2 * KSPS : KSPS;
+    constexpr int KS_PER_CHUNK = (CG == 2) ? Cfg::KSLICE : KSPS;
     #pragma unroll
     for (int s2 = 0; s2 < KS_PER_CHUNK; ++s2) {
-        const int ks = (CG == 2) ? s2 : (q & 1) * KSPS + s2;           // K-step within the full K range
-        const bool lo_pass = (CG == 2) ? (q == 1) : (q >= 2);
+        const int ks = (CG == 2) ? (Cfg::KSLICED ? (q % Cfg::CPP) * Cfg::KSLICE + s2 : s2) : (q & 1) * KSPS + s2;      // K-step within the full K range
+        const bool lo_pass = (CG == 2) ? (q >= Cfg::CPP) : (q >= 2);
         const uint32_t skip = (uint32_t)(tri16 * ks);                   // structurally zero leading columns
         const uint32_t np = NT - skip;                                  // N' of this MMA
         const uint32_t a_lo = a_lo_t + ks * ((2 * A_LBO) >> 4);
         uint32_t b_lo;
+        if constexpr (CG == 2 && Cfg::KSLICED) {      // K-slice chunk: sub-blocks in K-step order from the slice's first
+            const int off = tc2_ks_off(NT, Cfg::TRI16, ks) - tc2_ks_off(NT, Cfg::TRI16, (q % Cfg::CPP) * Cfg::KSLICE);
+            const uint32_t n0 = (uint32_t)tc2_piece0((int)np);
+            b_lo = (b_addr_s + (uint32_t)(off >> 4)) | ((n0 >> 1) << 16);
+            const uint32_t accum = (lo_pass || ks > 0) ? 1u : 0u;
+            if (elected) {
+                umma2_f16(d_tile + skip, a_lo, b_lo, DESC_HI, IDESC0 | ((n0 >> 3) << 17), accum);
+                if (n0 != np)      // columns [256, NT): the second piece follows the first's 16 n0 bytes
+                    umma2_f16(d_tile + 256, a_lo, (b_addr_s + (uint32_t)((off + 16 * (int)n0) >> 4)) | ((256u >> 1) << 16), DESC_HI,
+                              IDESC0 | ((256u >> 3) << 17), accum);
+            }
+            continue;
+        }
         if (CG == 2) {  // per-CTA half image: sub-block of N'/2 rows, LBO = (N'/16) cores * 128 B (all immediates)
             const int half = ks / KSPS, sb = ks % KSPS;
             const int off = (half ? Cfg::CB0 : 0) + tc2_sub_off(NT, Cfg::TRI16, KSPS, half, sb);
@@ -228,7 +259,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) dense_tc_kernel(const TcArgs a
             // ===================== bulk-TMA producer: NCHUNK chunks per component through the ring
             int stage = 0;
             uint32_t phase = 0;
-            constexpr size_t COMP_BYTES = (CG == 2) ? (size_t)2 * Cfg::STAGE_BYTES : (size_t)Cfg::COMP_HALFS * 2;
+            constexpr size_t COMP_BYTES = (CG == 2) ? (size_t)2 * Cfg::PASS_BYTES : (size_t)Cfg::COMP_HALFS * 2;
             const unsigned char* img = (CG == 2) ? a.image2 + (size_t)rank * COMP_BYTES : reinterpret_cast<const unsigned char*>(a.image);
             constexpr size_t COMP_STRIDE = COMP_BYTES * CG;      // CG=2: [k][rank]
             for (int64_t unit = unit0; unit < n_units; unit += unit_step) {
@@ -240,9 +271,14 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) dense_tc_kernel(const TcArgs a
                     #pragma unroll
                     for (int q = 0; q < Cfg::NCHUNK; ++q) {
                         mbar_wait(smem_u32(&ctrl->empty[stage]), phase ^ 1);
+                        if constexpr (Cfg::KSLICED) {      // K-slices differ in length (triangular skip)
+                            mbar_expect_tx(smem_u32(&ctrl->full[stage]), Cfg::chunk_bytes(q));
+                            bulk_g2s(smem_u32(sB + stage * Cfg::STAGE_BYTES), comp + Cfg::chunk_off(q), Cfg::chunk_bytes(q), smem_u32(&ctrl->full[stage]));
+                        } else {
                         mbar_expect_tx(smem_u32(&ctrl->full[stage]), Cfg::STAGE_BYTES);
                         bulk_g2s(smem_u32(sB + stage * Cfg::STAGE_BYTES), comp + (size_t)q * Cfg::STAGE_BYTES, Cfg::STAGE_BYTES,
                                  smem_u32(&ctrl->full[stage]));
+                        }
                         if (++stage == S) { stage = 0; phase ^= 1; }
                     }
                 }
@@ -758,12 +794,15 @@ __global__ void __launch_bounds__(256) tc2_pack_kernel(const double2* __restrict
     for (int half = 0; half < 2; ++half) {
         for (int s2 = 0; s2 < ksps; ++s2) {
             const int ks = half * ksps + s2;
-            const int np = tc2_nprime(nt, tri16, ks), rows = np / 2;
-            const int n0 = tri16 * ks + rank * rows;                       // first stacked row held by this rank
+            const int np = tc2_nprime(nt, tri16, ks), w0 = tc2_piece0(np);
             __half* hi = reinterpret_cast<__half*>(base + (half ? cb0 : 0) + tc2_sub_off(nt, tri16, ksps, half, s2));
             __half* lo = reinterpret_cast<__half*>(reinterpret_cast<unsigned char*>(hi) + (cb0 + cb1));
-            for (int idx = threadIdx.x; idx < rows * 16; idx += 256) {
-                const int core = idx >> 6, within = idx & 63;              // core = kc * (rows/8) + nb
+            for (int idx = threadIdx.x; idx < np * 8; idx += 256) {
+                // MMA piece (one unless N' > 256): its width, first stacked row and the index within its per-rank block
+                const bool p1 = idx >= w0 * 8;
+                const int rows = (p1 ? np - w0 : w0) / 2, li = p1 ? idx - w0 * 8 : idx;
+                const int n0 = (p1 ? tri16 * ks + w0 : tri16 * ks) + rank * rows;      // first stacked row of the piece held by this rank
+                const int core = li >> 6, within = li & 63;                // core = kc * (rows/8) + nb
                 const int nb = core % (rows / 8), kc = core / (rows / 8);
                 const int n = n0 + nb * 8 + (within >> 3), kk = ks * 16 + kc * 8 + (within & 7);
                 const bool isz = n < nz;
@@ -1581,27 +1620,38 @@ static bool tc_instantiated(const qce_model* m) {
 }
 
 // split launches: the 2 n_ant estimate columns are produced in row blocks of at most 128 (64 packed register accumulators
-// per pilot), the 2 n_obs whitening columns by a launch of their own
+// per pilot), the 2 n_obs whitening columns by a launch of their own.  n_obs = 256: one pilot per antenna, or two pilots on 128
+// antennas (A = kron([1, j], I))
 static bool tc_split_shape(int No, int N, int* parts, int* part_cols) {
+    if (No == 256 && (N == 128 || N == 256)) { *part_cols = 128; *parts = 2 * N / 128; return true; }
     if (No == 128 && (N == 64 || N == 128)) { *part_cols = 128; *parts = 2 * N / 128; return true; }
     if (No == 96 && (N == 48 || N == 96)) { *part_cols = 96; *parts = 2 * N / 96; return true; }
     return false;
 }
 
+// n_obs = 256 with pilots off the integer grid: a (hi, lo) pilot tile pair would take 256 KB of shared memory
+static bool tc_off_grid_too_wide(const qce_model* m) { return m->n_obs > 128 && !(m->data_scale > 0.0); }
+
 bool tc_supported(const qce_model* m, int mode) {
     if (!(m->data_scale >= 0.0)) return false;
     int parts = 0, pc = 0;
-    if (tc_split_shape(m->n_obs, m->n_ant, &parts, &pc)) return !m->tc.ready || m->tc.triangular;
+    if (tc_split_shape(m->n_obs, m->n_ant, &parts, &pc)) return !tc_off_grid_too_wide(m) && (!m->tc.ready || m->tc.triangular);
     if (m->data_scale == 0.0 && m->tc.ready && !m->tc.triangular) return false;      // off-grid pilots: SM-pair variant only
     // the modes other than the fused 'all' need the SM-pair variant (triangular whitening factor)
     if (mode != QCE_MODE_ALL && m->tc.ready && !m->tc.triangular) return false;
     return tc_instantiated(m);
 }
 
+const char* tc_unsupported_reason(const qce_model* m) {
+    return tc_off_grid_too_wide(m) ? ": pilots off the integer grid (Lloyd-Max labels, unquantised data) at n_obs > 128 would need a "
+                                     "256 KB (hi, lo) pilot tile pair per CTA, more than the shared memory holds" : "";
+}
+
 void tc_free(qce_model* m) {
     TcParams& p = m->tc;
     cudaFree(p.image); cudaFree(p.image2); cudaFree(p.zoff); cudaFree(p.hoff); cudaFree(p.zscale); cudaFree(p.hscale); cudaFree(p.logc2); cudaFree(p.flags);
-    cudaFree(p.image_z); cudaFree(p.image_h[0]); cudaFree(p.image_h[1]);
+    cudaFree(p.image_z);
+    for (void* h : p.image_h) cudaFree(h);
     p = TcParams();
 }
 
@@ -1669,7 +1719,7 @@ qce_status tc_pack_params(qce_model* m, cudaStream_t s) {
         }
     } else if (p.image_z) {     // parameters replaced by a non-triangular set
         QCE_CUDA_TRY(cudaFree(p.image_z)); p.image_z = nullptr;
-        QCE_CUDA_TRY(cudaFree(p.image_h[0])); p.image_h[0] = nullptr;
+        for (void*& h : p.image_h) { QCE_CUDA_TRY(cudaFree(h)); h = nullptr; }
     }
     QCE_CUDA_TRY(cudaStreamSynchronize(s));
     p.ready = true;
@@ -1725,7 +1775,10 @@ static qce_status launch_split_ac(const TcArgs& a, bool offs, int epi, cudaStrea
 }
 template <int KDC, int NCHH>
 static qce_status launch_split(const TcArgs& a, bool offs, int epi, bool split_a, cudaStream_t s) {
-    if constexpr (KDC > 4) {
+    if constexpr (KDC > 8) {      // n_obs = 256: on-grid pilots only (tc_supported)
+        if (split_a) { set_error("tensor-core kernel: pilots off the integer grid at n_obs = %d are not supported", a.No); return QCE_ERR_UNSUPPORTED; }
+        return launch_split_ac<KDC, NCHH, 1, 1>(a, offs, epi, s);
+    } else if constexpr (KDC > 4) {
         return split_a ? launch_split_ac<KDC, NCHH, 1, 2>(a, offs, epi, s) : launch_split_ac<KDC, NCHH, 1, 1>(a, offs, epi, s);
     } else {
         return split_a ? launch_split_ac<KDC, NCHH, 0, 2>(a, offs, epi, s) : launch_split_ac<KDC, NCHH, 0, 1>(a, offs, epi, s);
@@ -1734,8 +1787,9 @@ static qce_status launch_split(const TcArgs& a, bool offs, int epi, bool split_a
 
 // Log-likelihood gap (nats) below which a hard selection is re-made in complex128.  Measured error of the DIFFERENCE of two
 // FP16-split / FP32-accumulated log-likelihoods of a pilot (profiles/r02_flip_rate.json, max over 2^16..2^18 pilots): 2.2e-5 nats
-// at n_obs = 64, 3.5e-5 at n_obs = 128 and on the three-pass (off-grid) path: the gap keeps a margin of >= 4x, and grows per pilot
-// with the quadratic form of its best component.  QCE_TC_TIE_EPS overrides (0 disables the re-evaluation: A/B runs).
+// at n_obs = 64, 3.5e-5 at n_obs = 128 and on the three-pass (off-grid) path, 6.8e-5 at n_obs = 256 (profiles/n256_flip_rate.jsonl,
+// 2^16 model-drawn pilots, K = 64): the gap (4e-4 at n_obs = 256) keeps a margin of >= 4x, and grows per pilot with the quadratic
+// form of its best component.  QCE_TC_TIE_EPS overrides (0 disables the re-evaluation: A/B runs).
 static double tc_tie_eps(const qce_model* m) {
     if (const char* e = getenv("QCE_TC_TIE_EPS")) return atof(e);
     const double scale = m->n_obs > 64 ? (double)m->n_obs / 64.0 : 1.0;
@@ -1785,7 +1839,7 @@ static qce_status tc_run_split(const qce_model* m, const TileScratch* ts, cudaSt
     qce_status st = QCE_ERR_UNSUPPORTED;
     bool hit = false;
 #define QCE_TC_SPLIT_CASE(Z, H) if (!hit && cz == Z && ch == H) { st = launch_split<Z, H>(a, p.has_offsets, epi, p.split_a, s); hit = true; }
-    QCE_TC_SPLIT_CASE(8, 4) QCE_TC_SPLIT_CASE(6, 3)
+    QCE_TC_SPLIT_CASE(16, 4) QCE_TC_SPLIT_CASE(8, 4) QCE_TC_SPLIT_CASE(6, 3)
     QCE_TC_SPLIT_CASE(4, 4) QCE_TC_SPLIT_CASE(2, 2) QCE_TC_SPLIT_CASE(1, 1) QCE_TC_SPLIT_CASE(3, 3) QCE_TC_SPLIT_CASE(4, 2) QCE_TC_SPLIT_CASE(2, 1)
 #undef QCE_TC_SPLIT_CASE
     if (!hit) {
@@ -1895,7 +1949,7 @@ static qce_status tc_run_modes(qce_model* m, TileScratch* ts, cudaStream_t s, in
     const size_t tile_bytes = (size_t)TILE_M * 2 * m->n_obs * sizeof(__half) * (m->tc.split_a ? 2 : 1);
     const size_t true_row = (size_t)m->n_ant * (h_true_c64 ? 8 : 16);
     // top-1: regroup the pilots by selected component and run ONE component per work unit (QCE_TC_BUCKET=0: weighted launch instead)
-    const int tiles_per_unit = 2 * ((m->tc.split_a && 2 * m->n_obs > 128) ? 1 : TILES);      // CG * Cfg::NTILES of the split launches
+    const int tiles_per_unit = 2 * (((m->tc.split_a && 2 * m->n_obs > 128) || 2 * m->n_obs > 256) ? 1 : TILES);      // CG * Cfg::NTILES of the split launches
     const int bucket_rows = tiles_per_unit * TILE_M;
     const bool bucket_env = !(getenv("QCE_TC_BUCKET") && atoi(getenv("QCE_TC_BUCKET")) == 0);      // read per call (A/B runs, parity test)
     const bool bucketed = bucket_env && want_est && mode == QCE_MODE_TOP1 && m->n_comp >= 4 && chunk >= 4 * (int64_t)bucket_rows;

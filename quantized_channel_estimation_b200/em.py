@@ -130,7 +130,8 @@ class _KernelEStep:
     def __init__(self, X):
         from . import engine
         self.engine, self.X, self.model = engine, X.contiguous(), None
-        self.ok = X.is_cuda and engine.tc_padded_shape(X.shape[1], X.shape[1]) is not None
+        # unquantised data (data_scale = 0): off the integer grid
+        self.ok = X.is_cuda and engine.tc_padded_shape(X.shape[1], X.shape[1], on_grid=False) is not None
 
     def log_prob(self, weights, means, covs):
         K, N = means.shape

@@ -27,24 +27,29 @@ def parse_mode(n_summands_or_proba):
     return _lib.MODE_CUMPROB, 0, float(x)
 
 
-def tc_shape_ok(n_obs, n_ant):
-    """Shapes the tensor-core kernels are instantiated for (mirrors tc_instantiated / tc_split_shape in qce_dense_tc.cu)."""
+def tc_shape_ok(n_obs, n_ant, on_grid=False):
+    """Shapes the tensor-core kernels are instantiated for (mirrors tc_instantiated / tc_split_shape / tc_supported in
+    qce_dense_tc.cu).  ``on_grid``: the pilots lie on an integer grid (``data_scale > 0``: 1 bit, or uniform b bit).  n_obs = 256
+    (one pilot per antenna on 256 antennas, or two pilots on 128) takes only such pilots; off the grid it runs on the complex128
+    kernel."""
     if n_obs % 16 or n_ant % 16:
         return False
     if n_obs <= 64 and n_ant <= 64:
         return n_obs == n_ant or (n_obs, n_ant) in ((64, 32), (32, 16))
+    if on_grid and (n_obs, n_ant) in ((256, 128), (256, 256)):
+        return True
     return (n_obs, n_ant) in ((128, 64), (128, 128), (96, 48), (96, 96))
 
 
-def tc_padded_shape(n_obs, n_ant):
+def tc_padded_shape(n_obs, n_ant, on_grid=False):
     """Smallest tensor-core shape that holds an (n_obs, n_ant) model after zero padding (None: there is none).  Padded rows / columns
     of the parameter blocks are zero, padded pilot entries are zero: they add exact zeros to the quadratic forms and produce estimate
-    entries that are cut off again."""
-    if tc_shape_ok(n_obs, n_ant):
+    entries that are cut off again.  ``on_grid`` as for ``tc_shape_ok``: only on-grid models are padded up to n_obs = 256."""
+    if tc_shape_ok(n_obs, n_ant, on_grid):
         return n_obs, n_ant
-    up = lambda x: -(-x // 16) * 16
-    cands = [(o, a) for o in (16, 32, 48, 64, 96, 128) for a in (16, 32, 48, 64, 96, 128)
-             if o >= n_obs and a >= n_ant and tc_shape_ok(o, a)]
+    sizes = (16, 32, 48, 64, 96, 128, 256)
+    cands = [(o, a) for o in sizes for a in sizes
+             if o >= n_obs and a >= n_ant and tc_shape_ok(o, a, on_grid)]
     return min(cands, key=lambda c: c[0] * (c[0] + c[1])) if cands else None
 
 
@@ -159,8 +164,9 @@ class DenseModel:
         lib = _lib.require_device()
         self.n_obs, self.n_ant, self.n_comp = int(prep['n_obs']), int(prep['n_ant']), int(prep['n_comp'])
         self.pad_obs, self.pad_ant = self.n_obs, self.n_ant          # shape of the library handle
-        if pad and not tc_shape_ok(self.n_obs, self.n_ant):
-            ps = tc_padded_shape(self.n_obs, self.n_ant)
+        on_grid = float(prep['data_scale']) > 0
+        if pad and not tc_shape_ok(self.n_obs, self.n_ant, on_grid):
+            ps = tc_padded_shape(self.n_obs, self.n_ant, on_grid)
             if ps is not None:
                 self.pad_obs, self.pad_ant = ps
         self.handle = C.c_void_p()

@@ -76,8 +76,10 @@ class Mofa:
                     A.shape == (self.D, self.D) and np.array_equal(A, np.eye(self.D)) and self._covs_are_low_rank)
         # pilots on an integer grid and a tensor-core shape: the dense tcgen05 kernels beat the complex128 Woodbury kernel
         # (config 4: 55 M vs 0.9 M estimates/s) although they do 4x the flops
-        # (off-grid pilots -- Lloyd-Max labels, unquantised data -- take three tensor passes)
-        if woodbury and self.precision != 'fp64' and engine.tc_padded_shape(A.shape[0], self.D) is not None:
+        # (off-grid pilots -- Lloyd-Max labels, unquantised data -- take three tensor passes up to D = 128; at D = 256 they have no
+        # tensor-core path and stay on the Woodbury kernel)
+        on_grid = precompute.data_scale_for(snr_dB, np.inf if nb == 'inf' else nb, quantizer_type) > 0
+        if woodbury and self.precision != 'fp64' and engine.tc_padded_shape(A.shape[0], self.D, on_grid) is not None:
             woodbury = False
         if woodbury:
             key = ('woodbury', float(snr_dB), nb, quantizer_type if nb != 'inf' else None, tables, _fingerprint(self.means),

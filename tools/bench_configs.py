@@ -1,8 +1,9 @@
 #!/usr/bin/env python
 """Throughput of the other BASELINE.json configurations (kernel time with CUDA events, inputs resident).
-Not the contract bench (bench.py); prints one JSON line per configuration."""
+Not the contract bench (bench.py); prints one JSON line per configuration.  ``--n256`` runs only the dense n_obs = 256 shape."""
 import json
 import os
+import subprocess
 import sys
 
 import numpy as np
@@ -43,8 +44,45 @@ def model_pilots(covs, w, B, snr, nb, qz, seed=0):
     return qce.get_observation_nbit(h, snr, n_bits=nb, thresholds=qz[0], cluster=qz[1], noise=noise)
 
 
+def card():
+    """Name and power limit of the card the numbers were measured on."""
+    try:
+        pl = subprocess.run(['nvidia-smi', '--query-gpu=power.limit', '--format=csv,noheader,nounits', '-i', str(torch.cuda.current_device())],
+                            capture_output=True, text=True, timeout=30).stdout.strip()
+    except (OSError, subprocess.SubprocessError):
+        pl = 'unknown'
+    return dict(gpu=torch.cuda.get_device_name(), power_limit_w=pl)
+
+
+def n256(out):
+    """Dense GMM 'full', N = 256, K = 64 (BASELINE config 3's array as a dense model): 1-bit and 2-bit uniform pilots drawn from the
+    model at 10 dB, all four modes, tensor-core path and complex128 kernel on the same pilots."""
+    snr, K, N, B = 10, 64, 256, 1 << 18
+    means, covs, w = synthetic.random_psd_gmm(K, N, seed=0)
+    m = qce.Gmm_nbit(n_components=K).set_parameters(means, covs, w, detect_structure=False)
+    info = card()
+    for nb in (1, 2):
+        qz = qce.get_quantizer([snr], nb, 'uniform')[snr] if nb > 1 else (None, None)
+        r = model_pilots(covs, w, B, snr, nb, qz)
+        for mode in ('all', 1, 4, 0.9):
+            row = dict(config=f'GMM full {nb}-bit uniform N=256 K=64 mode={mode}, model-drawn pilots 10 dB', B=B, **info)
+            for prec, reps in (('tc', 5), ('fp64', 1)):
+                m.precision = prec
+                run = lambda: m.estimate_from_y(r, snr, N, n_summands_or_proba=mode, n_bits=nb, quantizer=qz)
+                ms = timeit(run, reps)
+                row[f'{prec}_ms'] = ms
+                row[f'{prec}_est_per_s'] = B / ms * 1e3
+                row[f'{prec}_tflops_algorithmic'] = 16 * K * N * N * B / ms / 1e9
+            row['speedup'] = row['fp64_ms'] / row['tc_ms']
+            out.append(row)
+            print(json.dumps(row), flush=True)
+
+
 def main():
     out = []
+    if '--n256' in sys.argv:
+        n256(out)
+        return
     snr = 10
     # C1: GMM full, 1 bit, N=32, K=16
     means, covs, w = synthetic.random_psd_gmm(16, 32, seed=0)
@@ -123,6 +161,7 @@ def main():
                     tflops_algorithmic=16 * 64 * 128 * 128 * r.shape[0] / ms / 1e9))
     for o in out:
         print(json.dumps(o), flush=True)
+    n256(out)
 
 
 if __name__ == '__main__':

@@ -8,7 +8,8 @@ Per case and mode (top-1, top-n, cumulative rho):
   fixed          rows the tensor-core path handed to the complex128 kernel (qce_last_fix_count) and their share of the batch
   ms / ms_no_fix CUDA-event time per call with and without the re-evaluation
 and the error of the tensor-core log-likelihoods (max / rms over the competitive components) that the gap threshold has to cover.
-One JSON line per case; profiles/r02_flip_rate.json is this tool's output.
+One JSON line per case; profiles/r02_flip_rate.jsonl and profiles/n256_flip_rate.jsonl are this tool's output.
+FLIP_CASES=<substring> runs only the cases whose tag contains it.
 """
 import ctypes as C
 import json
@@ -88,6 +89,7 @@ def run_case(tag, model, r, chunk64=1 << 16):
 
 def main():
     B = int(os.environ.get('FLIP_B', 1 << 18))
+    only = os.environ.get('FLIP_CASES', '')
     dev = torch.device('cuda')
     for tag, K, N, snr, nb, qt, b in (('C2 GMM full N=64 K=64 1-bit 10 dB', 64, 64, 10, 1, 'uniform', B),
                                       ('C2 -10 dB', 64, 64, -10, 1, 'uniform', B), ('C2 30 dB', 64, 64, 30, 1, 'uniform', B),
@@ -95,7 +97,11 @@ def main():
                                       ('C1 -10 dB', 16, 32, -10, 1, 'uniform', B),
                                       ('C5 shape N=64 K=256 1-bit 10 dB', 256, 64, 10, 1, 'uniform', B // 4),
                                       ('N=128 K=64 2-bit uniform (split path)', 64, 128, 10, 2, 'uniform', B // 4),
-                                      ('N=64 K=32 3-bit Lloyd (off-grid, three passes)', 32, 64, 10, 3, 'lloyd', B // 2)):
+                                      ('N=64 K=32 3-bit Lloyd (off-grid, three passes)', 32, 64, 10, 3, 'lloyd', B // 2),
+                                      ('N=256 K=64 1-bit 10 dB (n_obs = 256 split path)', 64, 256, 10, 1, 'uniform', B // 4),
+                                      ('N=256 K=64 2-bit uniform 10 dB (n_obs = 256 split path)', 64, 256, 10, 2, 'uniform', B // 4)):
+        if only not in tag:
+            continue
         means, covs, w = synthetic.random_psd_gmm(K, N, seed=0)
         h, noise, _ = synthetic.sample_gmm_channels(means, covs, w, b, seed=1)
         qz = qce.get_quantizer([snr], nb, qt)[snr]
@@ -105,6 +111,8 @@ def main():
         del model, r
     # config 3: block-circulant 16 x 16, 3-bit Lloyd-Max, K = 128
     for tag, blocks in (('C3 block-circulant 16x16 K=128 3-bit Lloyd', (16, 16)), ('C3 plain circulant 256 K=128 3-bit Lloyd', (1, 256))):
+        if only not in tag:
+            continue
         K, N, snr, nb, qt = 128, 256, 8, 3, 'lloyd'
         c, _, w, _ = synthetic.circulant_gmm(K, *blocks, seed=K, dense=False)
         qz = qce.get_quantizer([snr], nb, qt)[snr]
