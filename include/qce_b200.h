@@ -184,6 +184,23 @@ qce_status qce_mfa_model_set_params(qce_mfa_model* m, void* stream, const double
 qce_status qce_mfa_estimate(qce_mfa_model* m, void* stream, const void* r_dev, int64_t B, int mode, int n_top, double rho,
                             void* h_est_dev, double* logp_out_dev, const void* h_true_dev, double* acc_dev);
 
+/* ---- achievable-rate lower bound (Bussgang_GMM.py:291-309, Bussgang_MFA.py:154-172) in summable form.  Per estimate row
+ * g = h_est / max(|h_est|^2, 0.1), inner = g^H B h with B the diagonal Bussgang matrix of the global model, q = Re g^H C_q g.
+ * The bound is log2(1 + |m|^2 / (v + Q / n)) with m = S1 / n, v = S2 / n - |m|^2, where S1 = sum inner, S2 = sum |inner|^2,
+ * Q = sum q: five sums that add across batches and ranks like the NMSE accumulators.  inner in FP64, q on the tensor cores
+ * (split FP16 operands, FP32 accumulation).  1 <= n_ant <= 256 (QCE_ERR_UNSUPPORTED above).  Calls from a thread whose current
+ * device is not the model's return QCE_ERR_INVALID. */
+typedef struct qce_rate_model qce_rate_model;
+qce_status qce_rate_model_create(int n_ant, qce_rate_model** out);
+void       qce_rate_model_destroy(qce_rate_model* m);
+/* buss_diag_dev c128 [N] (the diagonal of B), cq_dev c128 [N][N]; the model symmetrises, scales, splits and packs a copy
+ * (synchronises the stream once to read the range of C_q) */
+qce_status qce_rate_model_set_params(qce_rate_model* m, void* stream, const double* buss_diag_dev, const double* cq_dev);
+/* acc_dev f64[5] += { sum Re inner, sum Im inner, sum |inner|^2, sum Re g^H C_q g, B }; h_est_dev c128 [B][N]; h_true_dev
+ * c64 (h_true_c64 = 1) or c128 [B][N].  B = 0 enqueues nothing. */
+qce_status qce_rate_accumulate(qce_rate_model* m, void* stream, const void* h_est_dev, const void* h_true_dev,
+                               int h_true_c64, int64_t B, double* acc_dev);
+
 /* Host-buffer form of qce_estimate: r_host c128 [B][n_obs] -> h_est_host c128 [B][n_ant].  Copies are chunked (32 MiB, four chunks
  * in flight) and overlapped with the kernels on private streams.  The streams and staging slots come from a per-device pool: a call
  * takes a free set (or creates one) and returns it at the end, so concurrent calls -- on one model or several -- never share buffers

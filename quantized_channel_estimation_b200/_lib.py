@@ -48,6 +48,10 @@ _SIGS = {
     'qce_mfa_model_set_params': (C.c_int, [C.c_void_p] * 9),
     'qce_mfa_estimate': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_double, C.c_void_p,
                                    C.c_void_p, C.c_void_p, C.c_void_p]),
+    'qce_rate_model_create': (C.c_int, [C.c_int, C.POINTER(C.c_void_p)]),
+    'qce_rate_model_destroy': (None, [C.c_void_p]),
+    'qce_rate_model_set_params': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    'qce_rate_accumulate': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_void_p]),
     'qce_estimate_host': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_double, C.c_int,
                                     C.c_void_p]),
     'qce_circ_estimate_host': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_double, C.c_int,

@@ -462,6 +462,58 @@ qce_status qce_mfa_estimate(qce_mfa_model* m, void* stream, const void* r, int64
     return launch_mfa(m, (cudaStream_t)stream, (const double*)r, B, mode, n_top, rho, (double*)h_est, logp_out, (const double*)h_true, acc);
 }
 
+qce_status qce_rate_model_create(int n_ant, qce_rate_model** out) {
+    if (!out || n_ant < 1) { set_error("qce_rate_model_create: invalid shape"); return QCE_ERR_INVALID; }
+    if (n_ant > 256) { set_error("qce_rate_model_create: n_ant=%d not supported (at most 256)", n_ant); return QCE_ERR_UNSUPPORTED; }
+    qce_status st = require_device();
+    if (st) return st;
+    qce_rate_model* m = new qce_rate_model();
+    m->n_ant = n_ant;
+    m->n_pad = (n_ant + 15) & ~15;
+    m->device = current_device();
+    cudaError_t e = cudaMalloc(&m->buss, (size_t)n_ant * 16);
+    if (e == cudaSuccess) e = cudaMalloc(&m->frag, (size_t)m->n_pad * m->n_pad * 16);     // (2 Np)^2 halves, hi and lo
+    if (e != cudaSuccess) { set_error("qce_rate_model_create: %s", cudaGetErrorString(e)); qce_rate_model_destroy(m); return QCE_ERR_CUDA; }
+    *out = m;
+    return QCE_OK;
+}
+
+void qce_rate_model_destroy(qce_rate_model* m) {
+    if (!m) return;
+    cudaFree(m->buss); cudaFree(m->frag);
+    delete m;
+}
+
+static qce_status rate_device_check(const qce_rate_model* m, const char* fn) {
+    if (current_device() != m->device) {
+        set_error("%s: the model lives on device %d, the calling thread's current device is %d", fn, m->device, current_device());
+        return QCE_ERR_INVALID;
+    }
+    return QCE_OK;
+}
+
+qce_status qce_rate_model_set_params(qce_rate_model* m, void* stream, const double* buss_diag, const double* cq) {
+    if (!m || !buss_diag || !cq) { set_error("qce_rate_model_set_params: invalid argument"); return QCE_ERR_INVALID; }
+    qce_status st = rate_device_check(m, "qce_rate_model_set_params");
+    if (st) return st;
+    cudaStream_t s = (cudaStream_t)stream;
+    m->params_set = false;
+    QCE_CUDA_TRY(cudaMemcpyAsync(m->buss, buss_diag, (size_t)m->n_ant * 16, cudaMemcpyDeviceToDevice, s));
+    st = rate_pack(m, s, cq);
+    if (st) return st;
+    m->params_set = true;
+    return QCE_OK;
+}
+
+qce_status qce_rate_accumulate(qce_rate_model* m, void* stream, const void* h_est, const void* h_true, int h_true_c64, int64_t B,
+                               double* acc) {
+    if (!m || !m->params_set || B < 0 || (B > 0 && (!h_est || !h_true || !acc))) { set_error("qce_rate_accumulate: invalid argument"); return QCE_ERR_INVALID; }
+    qce_status st = rate_device_check(m, "qce_rate_accumulate");
+    if (st) return st;
+    if (B == 0) return QCE_OK;
+    return launch_rate(m, (cudaStream_t)stream, (const double*)h_est, h_true, h_true_c64 ? 1 : 0, B, acc);
+}
+
 qce_status qce_format_pilots(qce_model* m, void* stream, const void* r, int64_t B) {
     if (!m || !m->params_set || B < 0 || (B > 0 && !r)) { set_error("qce_format_pilots: invalid argument"); return QCE_ERR_INVALID; }
     if (!tc_supported(m, QCE_MODE_ALL) || !m->tc.ready) { set_error("qce_format_pilots: tensor-core path not available for this model"); return QCE_ERR_UNSUPPORTED; }

@@ -101,21 +101,6 @@ __device__ __forceinline__ void fft16(float2 (&v)[16]) {
     for (int i = 0; i < 16; ++i) v[i] = make_float2(o[i].x * 0.25f, o[i].y * 0.25f);
 }
 
-__device__ __forceinline__ void ldmatrix_x4(uint32_t (&r)[4], const void* smem_ptr) {
-    const uint32_t addr = (uint32_t)__cvta_generic_to_shared(smem_ptr);
-    asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0, %1, %2, %3}, [%4];"
-                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(addr));
-}
-__device__ __forceinline__ void mma16816(float (&d)[4], const uint32_t (&a)[4], const uint32_t b0, const uint32_t b1) {
-    asm("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
-                 : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-                 : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ void split_half(const float x, __half& hi, __half& lo) {
-    hi = __float2half_rn(x);
-    lo = __float2half_rn(x - __half2float(hi));
-}
-
 // KC = K / 64.  CT_NW warps per CTA: GEMM 1 gives each warp KNB = K / (8 CT_NW) blocks of 8 components, GEMM 2 G2NB = 32 / CT_NW
 // blocks of 8 bins; the FFT phases run 512 / (32 CT_NW) transforms per thread.
 template <int KC>

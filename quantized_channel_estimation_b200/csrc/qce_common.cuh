@@ -122,6 +122,16 @@ struct qce_mfa_model {
     bool params_set = false;
 };
 
+// rate lower-bound accumulators (qce_rate.cu)
+struct qce_rate_model {
+    int n_ant = 0, n_pad = 0;         // N, and N rounded up to a multiple of 16
+    int device = 0;
+    double* buss = nullptr;           // c128 [N] diagonal of the Bussgang matrix
+    void* frag = nullptr;             // [n_pad / 4][n_pad / 8][32] uint4: E (real embedding of C_q) as FP16 (hi, lo) mma fragments
+    double inv_se = 1.0;              // 2^-s of the packed E
+    bool params_set = false;
+};
+
 struct qce_model {
     int n_obs, n_ant, n_comp, flags;
     int device = 0;
@@ -302,4 +312,8 @@ qce_status launch_circ(const qce_circ_model* m, cudaStream_t s, const double* r,
                        double* h_est, double* logp_out, const double* h_true, double* acc);
 qce_status launch_circ_rows(const qce_circ_model* m, cudaStream_t s, const double* r, const int* rows, const int* n_rows_dev, int64_t max_rows,
                             int mode, int n_top, double rho, double* h_est, const double* h_true, double* acc);
+// qce_rate.cu
+qce_status rate_pack(qce_rate_model* m, cudaStream_t s, const double* cq);
+qce_status launch_rate(const qce_rate_model* m, cudaStream_t s, const double* h_est, const void* h_true, int h_true_c64, int64_t B,
+                       double* acc);
 }  // namespace qce

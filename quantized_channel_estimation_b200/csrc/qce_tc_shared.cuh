@@ -1,5 +1,5 @@
-// Shared pieces of the tensor-core estimate kernels (qce_dense_tc.cu):
-// kernel arguments, mbarrier / bulk-copy / tcgen05 PTX wrappers, pilot-tile scratch.
+// Shared pieces of the tensor-core kernels: kernel arguments, mbarrier / bulk-copy / tcgen05 PTX wrappers and pilot-tile
+// scratch of qce_dense_tc.cu; the mma.sync split-FP16 helpers of qce_circ_tc.cu and qce_rate.cu.
 #pragma once
 #include <math.h>
 #include <stdlib.h>
@@ -186,6 +186,23 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
         : "memory");
 }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+
+// ---- mma.sync helpers of the split-FP16 kernels (qce_circ_tc.cu, qce_rate.cu): an operand x is carried as hi + lo with
+// hi = fp16(x), lo = fp16(x - hi), and a product is three MMAs (hi*hi + lo*hi + hi*lo, ~22 significant bits)
+__device__ __forceinline__ void ldmatrix_x4(uint32_t (&r)[4], const void* smem_ptr) {
+    const uint32_t addr = (uint32_t)__cvta_generic_to_shared(smem_ptr);
+    asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0, %1, %2, %3}, [%4];"
+                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(addr));
+}
+__device__ __forceinline__ void mma16816(float (&d)[4], const uint32_t (&a)[4], const uint32_t b0, const uint32_t b1) {
+    asm("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
+                 : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
+                 : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
+}
+__device__ __forceinline__ void split_half(const float x, __half& hi, __half& lo) {
+    hi = __float2half_rn(x);
+    lo = __float2half_rn(x - __half2float(hi));
+}
 
 
 // Pilot-tile scratch: one buffer set per CUDA stream (calls on different streams may be in flight concurrently, e.g. the

@@ -407,6 +407,59 @@ class CircModel:
         _lib.check(lib.qce_circ_estimate_host(self.handle, r_ptr, B, mode, n_top, rho, _lib.PREC_FP64, out_ptr))
 
 
+class RateModel:
+    """Accumulators of the scripts' achievable-rate lower bound (qce_rate_model): ``utils.rate_lower_bound`` as five sums that add
+    across batches and ranks, so that the bound needs no stored estimates.  ``buss`` is the ``[N, N]`` Bussgang matrix of the global
+    model (must be diagonal), ``Cq`` the ``[N, N]`` quantisation-noise covariance ``C_r - B C B^H`` (``utils.rate_params`` builds
+    both); 1 <= N <= 256."""
+
+    def __init__(self, buss, Cq):
+        lib = _lib.require_device()
+        buss = torch.as_tensor(buss).to(torch.complex128)
+        Cq = torch.as_tensor(Cq).to(torch.complex128)
+        if buss.dim() != 2 or buss.shape[0] != buss.shape[1] or Cq.shape != buss.shape:
+            raise ValueError('buss and Cq must both be [N, N]')
+        diag = torch.diagonal(buss)
+        if bool((buss - torch.diag_embed(diag)).abs().max() != 0):
+            raise ValueError('buss must be diagonal (utils.rate_lower_bound handles a full Bussgang matrix)')
+        self.n_ant = int(buss.shape[0])
+        self.handle = C.c_void_p()
+        _lib.check(lib.qce_rate_model_create(self.n_ant, C.byref(self.handle)))
+        self.device = torch.device('cuda', torch.cuda.current_device())
+        d, cq = diag.to(self.device).contiguous(), Cq.to(self.device).contiguous()
+        with torch.cuda.device(self.device):
+            _lib.check(lib.qce_rate_model_set_params(self.handle, _stream(), _ptr(d), _ptr(cq)))
+            torch.cuda.current_stream().synchronize()      # the library copied / packed them; d and cq may now be freed
+
+    def __del__(self):
+        try:
+            if getattr(self, 'handle', None) and self.handle.value:
+                _lib.load().qce_rate_model_destroy(self.handle)
+                self.handle = C.c_void_p()
+        except Exception:
+            pass
+
+    def accumulate(self, h_est, h_true, acc=None):
+        """Add ``{sum Re inner, sum Im inner, sum |inner|^2, sum Re g^H C_q g, B}`` of the estimates ``h_est [B, N]`` (CUDA, complex128)
+        and channels ``h_true [B, N]`` (CUDA, complex64 or complex128) into ``acc`` (float64 ``[5]`` on the device, zeros if None) and
+        return it.  ``utils.rate_from_accumulators(acc)`` is the bound."""
+        h_est = _as_c128_cuda(h_est, 'h_est')
+        if not (isinstance(h_true, torch.Tensor) and h_true.is_cuda):
+            raise TypeError('h_true must be a torch CUDA tensor')
+        h_c64 = h_true.dtype == torch.complex64
+        h_true = (h_true if h_c64 else h_true.to(torch.complex128)).contiguous()
+        if h_est.dim() != 2 or h_est.shape[1] != self.n_ant or h_true.shape != h_est.shape:
+            raise ValueError(f'h_est and h_true must both be [B, {self.n_ant}]')
+        if acc is None:
+            acc = torch.zeros(5, dtype=torch.float64, device=h_est.device)
+        elif not (isinstance(acc, torch.Tensor) and acc.is_cuda and acc.dtype == torch.float64 and acc.numel() == 5 and acc.is_contiguous()):
+            raise TypeError('acc must be a contiguous float64 CUDA tensor of 5 elements')
+        with torch.cuda.device(h_est.device):
+            _lib.check(_lib.load().qce_rate_accumulate(self.handle, _stream(), _ptr(h_est), _ptr(h_true), int(h_c64), h_est.shape[0],
+                                                       _ptr(acc)))
+        return acc
+
+
 class MfaModel(CircModel):
     """Woodbury-form MFA parameter set on the GPU (qce_mfa_model); A = I, n_bits > 1 or infinite resolution."""
 

@@ -20,7 +20,8 @@ def shard_range(n_total, rank, world):
 
 
 def allreduce_accumulators(acc):
-    """Sum the ``[n_snr, 3]`` float64 accumulators over all ranks (no-op without an initialised process group)."""
+    """Sum the float64 accumulators (``[n_snr, 3]``, or ``[n_snr, 8]`` with the rate sums) over all ranks (no-op without an
+    initialised process group)."""
     if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
         dist.all_reduce(acc, op=dist.ReduceOp.SUM)
     return acc
@@ -44,3 +45,19 @@ def nmse_sweep(step_fn, n_total, snrs, n_antennas, device='cpu'):
         acc[i] += torch.as_tensor(out, dtype=torch.float64, device=device)
     allreduce_accumulators(acc)
     return nmse_from_accumulators(acc, n_antennas), acc
+
+
+def nmse_rate_sweep(step_fn, n_total, snrs, n_antennas, device='cpu'):
+    """:func:`nmse_sweep` with the scripts' second number, the achievable-rate lower bound: ``step_fn(snr_index, snr_dB, lo, hi)``
+    returns the three NMSE sums followed by the five rate sums of ``engine.RateModel.accumulate``.  One all-reduce of the
+    ``[n_snr, 8]`` accumulators; returns ``(nmse [n_snr], rate [n_snr], acc [n_snr, 8])``."""
+    from .utils import rate_from_accumulators
+    rank = dist.get_rank() if dist.is_available() and dist.is_initialized() else 0
+    world = dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
+    lo, hi = shard_range(n_total, rank, world)
+    acc = torch.zeros((len(snrs), 8), dtype=torch.float64, device=device)
+    for i, snr in enumerate(snrs):
+        out = step_fn(i, snr, lo, hi)
+        acc[i] += torch.as_tensor(out, dtype=torch.float64, device=device)
+    allreduce_accumulators(acc)
+    return nmse_from_accumulators(acc[:, :3], n_antennas), rate_from_accumulators(acc[:, 3:]), acc

@@ -165,6 +165,40 @@ def rate_lower_bound(h_est, h, buss, Cq):
     return float(torch.log2(1 + num / (den1 + den2)))
 
 
+def rate_from_accumulators(acc):
+    """The bound of :func:`rate_lower_bound` from the sums ``acc [..., 5] = (sum Re inner, sum Im inner, sum |inner|^2,
+    sum Re g^H C_q g, count)`` that ``engine.RateModel.accumulate`` adds up: ``m = S1 / n``, ``v = S2 / n - |m|^2`` (np.var,
+    ddof 0), ``rate = log2(1 + |m|^2 / (v + Q / n))``.  Returns the rates over the leading dimensions (a float for ``[5]``)."""
+    a = acc.detach().cpu().numpy() if isinstance(acc, torch.Tensor) else np.asarray(acc, dtype=np.float64)
+    if a.shape[-1] != 5:
+        raise ValueError('rate accumulators must have 5 entries in the last dimension')
+    n = a[..., 4]
+    m2 = (a[..., 0] / n) ** 2 + (a[..., 1] / n) ** 2
+    rate = np.log2(1 + m2 / (a[..., 2] / n - m2 + a[..., 3] / n))
+    return float(rate) if rate.ndim == 0 else rate
+
+
+def rate_params(C, snr_dB, n_bits, quantizer_type='uniform', quantizer=None):
+    """``(buss, Cq)`` of :func:`rate_lower_bound` for the global channel covariance ``C [N, N]`` (the scripts' construction,
+    Bussgang_GMM.py:291-309): ``C_y = C + 10^(-snr/10) I``, ``buss`` the diagonal Bussgang matrix of C_y (uniform, or Lloyd-Max for
+    ``quantizer_type='lloyd'`` with ``n_bits > 1``), ``Cq = get_Cr(C_y, ...) - buss C buss^H``.  ``quantizer`` is the
+    ``(thresholds, labels, rho)`` table of ``get_quantizer``; it is looked up when omitted."""
+    from . import lloyd_max_quantizer, uniform_quantizer
+    C = np.asarray(C, dtype=complex)
+    Cy = C + 10 ** (-snr_dB / 10) * np.eye(C.shape[-1])
+    finite_multi = not _is_inf(n_bits) and n_bits > 1
+    if _is_inf(n_bits):
+        n_bits = np.inf
+    if quantizer is None and finite_multi:
+        quantizer = get_quantizer([snr_dB], n_bits, quantizer_type)[snr_dB]
+    if quantizer_type == 'lloyd' and finite_multi:
+        buss = lloyd_max_quantizer.get_Bussgang_matrix(n_bits, Cy, quantizer)
+    else:
+        buss = uniform_quantizer.get_Bussgang_matrix(snr_dB, n_bits, Cy).astype(complex)
+    Cq = uniform_quantizer.get_Cr(Cy, n_bits, snr_dB, quantizer) - buss @ C @ buss.conj().T
+    return buss, Cq
+
+
 class _RefObject:
     """Attribute bag standing in for a class of the reference's ``modules`` package while unpickling."""
 
