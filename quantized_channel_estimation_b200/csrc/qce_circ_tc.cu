@@ -302,7 +302,7 @@ __global__ void __launch_bounds__(32 * CT_NW, 2) circ_tc_kernel(const CircTcArgs
 
     // ---- combination weights per pilot
     if (a.logp_out) {
-        for (int o = tid; o < nvalid * K; o += NT) a.logp_out[base * K + o] = (double)lbuf[(o / K) * LP + (o % K)] + (a.logc_max - (double)qref[o / K]);
+        for (int o = tid; o < nvalid * K; o += NT) a.logp_out[base * K + o] = tc_logp_export((double)lbuf[(o / K) * LP + (o % K)] + (a.logc_max - (double)qref[o / K]));
         __syncthreads();
     }
     if (a.mode == QCE_MODE_ALL) {
@@ -497,7 +497,7 @@ __global__ void circ_tc_pack_kernel(const double* __restrict__ src, const float*
 
 __global__ void circ_tc_logc_kernel(const double* __restrict__ logc, int K, double logc_max, float2* __restrict__ out) {
     const int k = blockIdx.x * blockDim.x + threadIdx.x;
-    if (k < K) { const double l = logc[k] - logc_max; const float hi = (float)l; out[k] = make_float2(hi, (float)(l - (double)hi)); }
+    if (k < K) out[k] = tc_logc_pair(logc[k] - logc_max);
 }
 
 __global__ void circ_tc_ilbar_kernel(const double* __restrict__ inv_lambda_t, int N, int K, int one_d, float* __restrict__ out) {

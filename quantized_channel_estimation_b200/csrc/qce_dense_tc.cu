@@ -823,7 +823,7 @@ __global__ void tc_pack_small_kernel(const double2* __restrict__ zoff, const dou
                                      float2* __restrict__ logc2, int* __restrict__ flags) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     int nz = 0;
-    if (i < K) { const double l = logc[i]; const float hi = (float)l; logc2[i] = make_float2(hi, (float)(l - (double)hi)); }
+    if (i < K) logc2[i] = tc_logc_pair(logc[i]);
     if (i < K * No) { const double2 v = zoff[i]; zoff_f[2 * i] = (float)v.x; zoff_f[2 * i + 1] = (float)v.y; nz |= (v.x != 0.0 || v.y != 0.0); }
     if (i < K * N) { const double2 v = hoff[i]; hoff_f[2 * i] = (float)v.x; hoff_f[2 * i + 1] = (float)v.y; nz |= (v.x != 0.0 || v.y != 0.0); }
     if (nz) atomicOr(flags, 1);
@@ -1093,7 +1093,7 @@ __global__ void __launch_bounds__(256) tc_select_kernel(const float2* __restrict
             if (k < K) {
                 const float2 v = lp2[b * K + k];
                 l[i] = (double)v.x + (double)v.y;
-                if (logp_out) logp_out[b * K + k] = l[i];
+                if (logp_out) logp_out[b * K + k] = tc_logp_export(l[i]);
             }
         }
         // (re-selection of a listed pilot: its pairs leave the histogram of the pair-bucketed combination and the new ones enter)
@@ -1143,7 +1143,7 @@ __global__ void __launch_bounds__(SEL_THREADS) tc_select_rows_kernel(const float
                     const int r = i / K, k = i - r * K;
                     s_hi[k * P + r] = v[u].x;
                     s_lo[k * P + r] = v[u].y;
-                    if (logp_out) logp_out[(row0 + r) * K + k] = (double)v[u].x + (double)v[u].y;
+                    if (logp_out) logp_out[(row0 + r) * K + k] = tc_logp_export((double)v[u].x + (double)v[u].y);
                 }
             }
         }
@@ -1334,9 +1334,8 @@ __global__ void __launch_bounds__(256) tc_refine_kernel(const RefineArgs a) {
             for (int t = 0; t < REFINE_RT; ++t) if (lane == t) mine = q[t];
             if (lane < nv) {
                 const double lv = a.logc[k] - mine;
-                const float hi = (float)lv;
                 const size_t o = (size_t)s_crow[lane] * K + k;
-                a.lp2[o] = make_float2(hi, (float)(lv - (double)hi));      // 48 significant bits: ~1e-13 nats
+                a.lp2[o] = tc_logc_pair(lv);      // 48 significant bits: ~1e-13 nats
                 if (a.logp_out) a.logp_out[o] = lv;
             }
             }

@@ -21,6 +21,23 @@ constexpr int TILES = 2;
 constexpr int NUM_THREADS = 384;
 constexpr int SMEM_LIMIT = 227 * 1024;
 
+// A component of weight 0 has logc = -inf; the reference gives it responsibility 0.  The FP32 (hi, lo) pairs of the tensor-core
+// kernels cannot hold -inf: the lo part of the split and the pair subtraction l = logc - q would both be -inf - (-inf) = NaN, which
+// spreads through the softmax to every estimate of the pilot.  So the pair of such a component is the finite (TC_LOGC_ZERO_WEIGHT,
+// 0): its l_k stays at -2^100 (a quadratic form would have to reach 2^76, half an ulp there, to move it), exp(l_k - l_max) is 0,
+// and it is the maximum only if every component is.  The FP64 logc keeps -inf, and the log-probability exports map anything below
+// TC_LOGP_ZERO_WEIGHT back to -inf.
+constexpr float TC_LOGC_ZERO_WEIGHT = -0x1p100f;
+constexpr double TC_LOGP_ZERO_WEIGHT = -0x1p99;
+
+__device__ __forceinline__ float2 tc_logc_pair(double l) {
+    if (l == -INFINITY) return make_float2(TC_LOGC_ZERO_WEIGHT, 0.f);
+    const float hi = (float)l;
+    return make_float2(hi, (float)(l - (double)hi));
+}
+
+__device__ __forceinline__ double tc_logp_export(double l) { return l < TC_LOGP_ZERO_WEIGHT ? -INFINITY : l; }
+
 struct TcArgs {
     const __half* image;       // CG=1: [K][hi | lo] stacked [E(Linv); E(W)] images, canonical K-major core-matrix order
     const unsigned char* image2;  // CG=2: [K][rank][hi K0 | hi K1 | lo K0 | lo K1] per-CTA half images (see tc2_pack_kernel)
