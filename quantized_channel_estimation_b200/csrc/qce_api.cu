@@ -13,17 +13,28 @@ namespace qce {
 static thread_local char g_err[512] = "";
 std::atomic<int64_t> g_launch_count{0};
 
-// fix list (count first) of the most recent tensor-core estimate per (device, stream): qce_last_fix_count
-static std::mutex g_fix_mu;
-static std::map<std::pair<int, cudaStream_t>, const int*> g_fix_last;
-void note_fix_list(cudaStream_t s, const int* fix_buf) {
-    std::lock_guard<std::mutex> lock(g_fix_mu);
-    g_fix_last[std::make_pair(current_device(), s)] = fix_buf;
+// keyed by (device, stream): stream handles are only unique per device (the default stream is 0 everywhere)
+static std::mutex g_scratch_mu;
+static std::map<std::pair<int, cudaStream_t>, StreamScratch> g_scratch;
+StreamScratch* scratch_for(cudaStream_t s) {
+    std::lock_guard<std::mutex> lock(g_scratch_mu);
+    return &g_scratch[std::make_pair(current_device(), s)];
 }
-const int* last_fix_list(cudaStream_t s) {
-    std::lock_guard<std::mutex> lock(g_fix_mu);
-    auto it = g_fix_last.find(std::make_pair(current_device(), s));
-    return it == g_fix_last.end() ? nullptr : it->second;
+StreamScratch* scratch_find(cudaStream_t s) {
+    std::lock_guard<std::mutex> lock(g_scratch_mu);
+    auto it = g_scratch.find(std::make_pair(current_device(), s));
+    return it == g_scratch.end() ? nullptr : &it->second;
+}
+void scratch_release(cudaStream_t s) {
+    std::lock_guard<std::mutex> lock(g_scratch_mu);
+    auto it = g_scratch.find(std::make_pair(current_device(), s));
+    if (it == g_scratch.end()) return;
+    StreamScratch& e = it->second;
+    TileScratch& t = e.tc;
+    for (ScratchBuf* b : {&t.img, &t.bad, &t.lp2, &t.wts, &t.img2, &t.bidx, &t.fix, &t.tie, &t.tmp_est, &e.circ_fix, &e.pipe_r,
+                          &e.host_in, &e.host_out, &e.host_mid_in, &e.host_mid_out})
+        free_buf(*b);
+    g_scratch.erase(it);
 }
 
 void set_error(const char* fmt, ...) {
@@ -36,31 +47,23 @@ void set_error(const char* fmt, ...) {
 
 using namespace qce;
 
-struct HostCtx {                // staging of ONE host-buffer call at a time: pinned + device slots on private streams
+struct HostCtx {                // staging of ONE host-buffer call at a time: pinned slots and private streams (the device slots
+                                // are in the streams' scratch)
     static constexpr int NSLOT = 4;  // chunks in flight: keeps the H2D and the D2H copy engines busy back to back
     int device = -1;
     cudaStream_t streams[NSLOT] = {};
     cudaEvent_t done[NSLOT] = {};
-    void* pin_in[NSLOT] = {};
-    void* pin_out[NSLOT] = {};
-    void* dev_in[NSLOT] = {};
-    void* dev_out[NSLOT] = {};
-    void* dev_mid_in[NSLOT] = {};    // device-only intermediates of the compact transfer formats (decoded pilots, complex128 estimates)
-    void* dev_mid_out[NSLOT] = {};
-    size_t in_bytes = 0, out_bytes = 0, mid_in_bytes = 0, mid_out_bytes = 0, pin_in_bytes = 0, pin_out_bytes = 0;
+    ScratchBuf pin_in[NSLOT], pin_out[NSLOT];
+    HostCtx() { for (int i = 0; i < NSLOT; ++i) pin_in[i].pinned = pin_out[i].pinned = true; }
 };
 
 void host_ctx_free(HostCtx* c) {
     if (!c) return;
     for (int i = 0; i < HostCtx::NSLOT; ++i) {
-        if (c->streams[i]) { cudaStreamSynchronize(c->streams[i]); tc_scratch_release(c->streams[i]); cudaStreamDestroy(c->streams[i]); }
+        if (c->streams[i]) { cudaStreamSynchronize(c->streams[i]); scratch_release(c->streams[i]); cudaStreamDestroy(c->streams[i]); }
         if (c->done[i]) cudaEventDestroy(c->done[i]);
-        if (c->pin_in[i]) cudaFreeHost(c->pin_in[i]);
-        if (c->pin_out[i]) cudaFreeHost(c->pin_out[i]);
-        if (c->dev_in[i]) cudaFree(c->dev_in[i]);
-        if (c->dev_out[i]) cudaFree(c->dev_out[i]);
-        if (c->dev_mid_in[i]) cudaFree(c->dev_mid_in[i]);
-        if (c->dev_mid_out[i]) cudaFree(c->dev_mid_out[i]);
+        free_buf(c->pin_in[i]);
+        free_buf(c->pin_out[i]);
     }
     delete c;
 }
@@ -127,7 +130,8 @@ void qce_host_staging_release(void) {
 }
 
 int64_t qce_last_fix_count(void* stream) {
-    const int* p = last_fix_list((cudaStream_t)stream);
+    const StreamScratch* sc = scratch_find((cudaStream_t)stream);
+    const int* p = sc ? sc->last_fix : nullptr;
     if (!p) return -1;
     int n[2] = {0, 0};      // rows answered completely in complex128, near-ties re-selected in complex128
     if (cudaMemcpyAsync(n, p, sizeof(n), cudaMemcpyDeviceToHost, (cudaStream_t)stream) != cudaSuccess ||
@@ -235,7 +239,6 @@ void qce_model_destroy(qce_model* m) {
     if (m->params_ready) cudaEventDestroy(m->params_ready);
     tc_free(m);
     cudaFree(m->Linv); cudaFree(m->W); cudaFree(m->zoff); cudaFree(m->hoff); cudaFree(m->logc);
-    if (m->pipe_r) cudaFree(m->pipe_r);
     delete m;
 }
 
@@ -331,23 +334,20 @@ qce_status qce_pipeline(qce_model* m, const qce_quantizer* q, void* stream, cons
         }
         return QCE_OK;
     }
-    // quantised pilots of one chunk live in a model-owned scratch buffer (grown on first use, then reused)
+    // quantised pilots of one chunk live in the stream's scratch (grown on first use, then reused)
     const int64_t chunk_max = (int64_t)1 << 20;
-    const int64_t cap = B < chunk_max ? B : chunk_max;
-    if (cap > m->pipe_cap) {
-        if (m->pipe_r) QCE_CUDA_TRY(cudaFree(m->pipe_r));
-        m->pipe_r = nullptr; m->pipe_cap = 0;
-        QCE_CUDA_TRY(cudaMalloc(&m->pipe_r, (size_t)cap * N * 16));
-        m->pipe_cap = cap;
-    }
+    const int64_t chunk = B < chunk_max ? B : chunk_max;
+    ScratchBuf& pipe_r = scratch_for(s)->pipe_r;
+    qce_status st = grow(pipe_r, (size_t)chunk * N * 16);
+    if (st) return st;
     const size_t hstride = h_is_c64 ? 8 : 16;
-    for (int64_t b0 = 0; b0 < B; b0 += m->pipe_cap) {
-        const int64_t nb = (B - b0) < m->pipe_cap ? (B - b0) : m->pipe_cap;
+    for (int64_t b0 = 0; b0 < B; b0 += chunk) {
+        const int64_t nb = (B - b0) < chunk ? (B - b0) : chunk;
         const char* hp = (const char*)h + (size_t)b0 * N * hstride;
-        qce_status st = launch_observe_quantize(&q->t, s, hp, h_is_c64, (const double*)noise + (size_t)b0 * N * 2, noise_scale,
-                                                nb * N, nullptr, (double*)m->pipe_r, nullptr);
+        st = launch_observe_quantize(&q->t, s, hp, h_is_c64, (const double*)noise + (size_t)b0 * N * 2, noise_scale,
+                                     nb * N, nullptr, (double*)pipe_r.p, nullptr);
         if (st) return st;
-        st = estimate_impl(m, s, (const double*)m->pipe_r, nb, mode, n_top, rho, precision,
+        st = estimate_impl(m, s, (const double*)pipe_r.p, nb, mode, n_top, rho, precision,
                            h_est ? (double*)h_est + (size_t)b0 * N * 2 : nullptr, nullptr, hp, h_is_c64, acc);
         if (st) return st;
     }
@@ -549,35 +549,18 @@ static qce_status estimate_host_impl(int model_device, cudaEvent_t params_ready,
     if (mid_out_row > max_row) max_row = mid_out_row;
     int64_t chunk = (int64_t)(slot_bytes / max_row);
     if (chunk < 128) chunk = 128;
-    {
-        const size_t need_dev_in = (size_t)chunk * in_row, need_dev_out = (size_t)chunk * out_row;
-        const size_t need_mi = (size_t)chunk * mid_in_row, need_mo = (size_t)chunk * mid_out_row;
-        for (int i = 0; i < NSLOT; ++i) {
-            if (!hs->streams[i]) {
-                QCE_CUDA_TRY(cudaStreamCreateWithFlags(&hs->streams[i], cudaStreamNonBlocking));
-                QCE_CUDA_TRY(cudaEventCreateWithFlags(&hs->done[i], cudaEventDisableTiming));
-            }
-            if (hs->in_bytes < need_dev_in) {
-                if (hs->dev_in[i]) { cudaFree(hs->dev_in[i]); hs->dev_in[i] = nullptr; }
-                QCE_CUDA_TRY(cudaMalloc(&hs->dev_in[i], need_dev_in));
-            }
-            if (hs->out_bytes < need_dev_out) {
-                if (hs->dev_out[i]) { cudaFree(hs->dev_out[i]); hs->dev_out[i] = nullptr; }
-                QCE_CUDA_TRY(cudaMalloc(&hs->dev_out[i], need_dev_out));
-            }
-            if (hs->mid_in_bytes < need_mi) {
-                if (hs->dev_mid_in[i]) { cudaFree(hs->dev_mid_in[i]); hs->dev_mid_in[i] = nullptr; }
-                QCE_CUDA_TRY(cudaMalloc(&hs->dev_mid_in[i], need_mi));
-            }
-            if (hs->mid_out_bytes < need_mo) {
-                if (hs->dev_mid_out[i]) { cudaFree(hs->dev_mid_out[i]); hs->dev_mid_out[i] = nullptr; }
-                QCE_CUDA_TRY(cudaMalloc(&hs->dev_mid_out[i], need_mo));
-            }
+    StreamScratch* dev[NSLOT];         // device slots: in the scratch of the slot's stream
+    for (int i = 0; i < NSLOT; ++i) {
+        if (!hs->streams[i]) {
+            QCE_CUDA_TRY(cudaStreamCreateWithFlags(&hs->streams[i], cudaStreamNonBlocking));
+            QCE_CUDA_TRY(cudaEventCreateWithFlags(&hs->done[i], cudaEventDisableTiming));
         }
-        if (hs->in_bytes < need_dev_in) hs->in_bytes = need_dev_in;
-        if (hs->out_bytes < need_dev_out) hs->out_bytes = need_dev_out;
-        if (hs->mid_in_bytes < need_mi) hs->mid_in_bytes = need_mi;
-        if (hs->mid_out_bytes < need_mo) hs->mid_out_bytes = need_mo;
+        dev[i] = scratch_for(hs->streams[i]);
+        qce_status st = grow(dev[i]->host_in, (size_t)chunk * in_row);
+        if (!st) st = grow(dev[i]->host_out, (size_t)chunk * out_row);
+        if (!st) st = grow(dev[i]->host_mid_in, (size_t)chunk * mid_in_row);
+        if (!st) st = grow(dev[i]->host_mid_out, (size_t)chunk * mid_out_row);
+        if (st) return st;
     }
     // parameters were uploaded / packed on the caller's stream: the private streams wait for that upload (an event, not a device-wide
     // synchronisation: other streams of the process are left alone)
@@ -590,20 +573,10 @@ static qce_status estimate_host_impl(int model_device, cudaEvent_t params_ready,
     };
     const bool in_pinned = is_pinned(r_host), out_pinned = is_pinned(h_est_host);
     // pinned staging slots only where the caller's buffer is pageable (page-locked buffers are copied directly)
-    {
-        const size_t need_pi = in_pinned ? 0 : (size_t)chunk * in_row, need_po = out_pinned ? 0 : (size_t)chunk * out_row;
-        for (int i = 0; i < NSLOT; ++i) {
-            if (hs->pin_in_bytes < need_pi) {
-                if (hs->pin_in[i]) { cudaFreeHost(hs->pin_in[i]); hs->pin_in[i] = nullptr; }
-                QCE_CUDA_TRY(cudaMallocHost(&hs->pin_in[i], need_pi));
-            }
-            if (hs->pin_out_bytes < need_po) {
-                if (hs->pin_out[i]) { cudaFreeHost(hs->pin_out[i]); hs->pin_out[i] = nullptr; }
-                QCE_CUDA_TRY(cudaMallocHost(&hs->pin_out[i], need_po));
-            }
-        }
-        if (hs->pin_in_bytes < need_pi) hs->pin_in_bytes = need_pi;
-        if (hs->pin_out_bytes < need_po) hs->pin_out_bytes = need_po;
+    for (int i = 0; i < NSLOT; ++i) {
+        qce_status st = grow(hs->pin_in[i], in_pinned ? 0 : (size_t)chunk * in_row);
+        if (!st) st = grow(hs->pin_out[i], out_pinned ? 0 : (size_t)chunk * out_row);
+        if (st) return st;
     }
     int64_t pending_b0[NSLOT], pending_nb[NSLOT];
     for (int i = 0; i < NSLOT; ++i) { pending_b0[i] = -1; pending_nb[i] = 0; }
@@ -611,7 +584,7 @@ static qce_status estimate_host_impl(int model_device, cudaEvent_t params_ready,
         if (pending_b0[slot] < 0) return QCE_OK;
         QCE_CUDA_TRY(cudaEventSynchronize(hs->done[slot]));
         if (!out_pinned)
-            parallel_memcpy((char*)h_est_host + (size_t)pending_b0[slot] * out_row, hs->pin_out[slot], (size_t)pending_nb[slot] * out_row);
+            parallel_memcpy((char*)h_est_host + (size_t)pending_b0[slot] * out_row, hs->pin_out[slot].p, (size_t)pending_nb[slot] * out_row);
         pending_b0[slot] = -1;
         return QCE_OK;
     };
@@ -621,13 +594,14 @@ static qce_status estimate_host_impl(int model_device, cudaEvent_t params_ready,
         if (st) return st;
         const int64_t b0 = c * chunk, nb = (B - b0) < chunk ? (B - b0) : chunk;
         const char* src = (const char*)r_host + (size_t)b0 * in_row;
-        if (!in_pinned) { parallel_memcpy(hs->pin_in[slot], src, (size_t)nb * in_row); src = (const char*)hs->pin_in[slot]; }
+        if (!in_pinned) { parallel_memcpy(hs->pin_in[slot].p, src, (size_t)nb * in_row); src = (const char*)hs->pin_in[slot].p; }
         cudaStream_t s = hs->streams[slot];
-        QCE_CUDA_TRY(cudaMemcpyAsync(hs->dev_in[slot], src, (size_t)nb * in_row, cudaMemcpyHostToDevice, s));
-        st = run(s, (const double*)hs->dev_in[slot], nb, (double*)hs->dev_out[slot], hs->dev_mid_in[slot], hs->dev_mid_out[slot]);
+        const StreamScratch* d = dev[slot];
+        QCE_CUDA_TRY(cudaMemcpyAsync(d->host_in.p, src, (size_t)nb * in_row, cudaMemcpyHostToDevice, s));
+        st = run(s, (const double*)d->host_in.p, nb, (double*)d->host_out.p, d->host_mid_in.p, d->host_mid_out.p);
         if (st) return st;
-        void* dst = out_pinned ? (void*)((char*)h_est_host + (size_t)b0 * out_row) : hs->pin_out[slot];
-        QCE_CUDA_TRY(cudaMemcpyAsync(dst, hs->dev_out[slot], (size_t)nb * out_row, cudaMemcpyDeviceToHost, s));
+        void* dst = out_pinned ? (void*)((char*)h_est_host + (size_t)b0 * out_row) : hs->pin_out[slot].p;
+        QCE_CUDA_TRY(cudaMemcpyAsync(dst, d->host_out.p, (size_t)nb * out_row, cudaMemcpyDeviceToHost, s));
         QCE_CUDA_TRY(cudaEventRecord(hs->done[slot], s));
         pending_b0[slot] = b0; pending_nb[slot] = nb;
     }

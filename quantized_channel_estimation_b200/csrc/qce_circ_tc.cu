@@ -16,9 +16,6 @@
 // Any real-valued pilots are accepted (no grid assumption: Lloyd-Max labels, infinite resolution).
 #include <stdlib.h>
 
-#include <map>
-#include <mutex>
-
 #include "qce_common.cuh"
 #include "qce_tc_shared.cuh"
 
@@ -598,22 +595,13 @@ qce_status circ_tc_pack(qce_circ_model* m, cudaStream_t s) {
     return QCE_OK;
 }
 
-// fix list of a launch: one buffer per (device, stream), grown on demand; the count is reset in stream order
+// fix list of a launch, in the stream's scratch; the count is reset in stream order
 static qce_status circ_fix_list(cudaStream_t s, int64_t rows, int** out) {
-    struct Buf { int* p = nullptr; size_t n = 0; };
-    static std::mutex mu;
-    static std::map<std::pair<int, cudaStream_t>, Buf> bufs;
-    std::lock_guard<std::mutex> lock(mu);
-    Buf& b = bufs[std::make_pair(current_device(), s)];
-    if ((size_t)rows + 2 > b.n) {      // [0] count, [1] unused here (layout of qce_last_fix_count), then the list
-        if (b.p) QCE_CUDA_TRY(cudaFree(b.p));
-        b.p = nullptr; b.n = 0;
-        QCE_CUDA_TRY(cudaMalloc(&b.p, ((size_t)rows + 2) * sizeof(int)));
-        b.n = (size_t)rows + 2;
-    }
-    QCE_CUDA_TRY(cudaMemsetAsync(b.p, 0, 2 * sizeof(int), s));
-    note_fix_list(s, b.p);
-    *out = b.p;
+    StreamScratch* sc = scratch_for(s);
+    qce_status st = grow(sc->circ_fix, ((size_t)rows + 2) * sizeof(int));     // [0] count, [1] unused here (layout of qce_last_fix_count), then the list
+    if (st) return st;
+    QCE_CUDA_TRY(cudaMemsetAsync(sc->circ_fix.p, 0, 2 * sizeof(int), s));
+    sc->last_fix = *out = (int*)sc->circ_fix.p;
     return QCE_OK;
 }
 

@@ -12,8 +12,6 @@
 namespace qce {
 
 void set_error(const char* fmt, ...);
-void note_fix_list(cudaStream_t s, const int* fix_buf);      // qce_last_fix_count bookkeeping (qce_api.cu)
-const int* last_fix_list(cudaStream_t s);
 extern std::atomic<int64_t> g_launch_count;          // calls may come from several host threads (one per stream / device)
 inline void count_launch(int n = 1) { g_launch_count.fetch_add(n, std::memory_order_relaxed); }
 
@@ -43,6 +41,31 @@ struct PerDeviceOnce {
     bool first(int dev) { if (dev < 0 || dev >= 64) return true; if (done[dev]) return false; done[dev] = true; return true; }
 };
 inline int current_device() { int d = 0; cudaGetDevice(&d); return d; }
+
+// Grow-on-demand buffer: device memory, or page-locked host memory when `pinned`.  A plain struct: a copy aliases the buffer, and
+// only free_buf releases it.
+struct ScratchBuf {
+    void* p = nullptr;
+    size_t bytes = 0;
+    bool pinned = false;
+};
+
+// Grows only, never shrinks: a larger need frees the buffer and allocates the new size (zeroed when zero_fill).  cudaFree
+// synchronises the device, so a steady state of equal-sized calls must never get here.
+inline qce_status grow(ScratchBuf& b, size_t bytes, bool zero_fill = false) {
+    if (bytes <= b.bytes) return QCE_OK;
+    if (b.p) QCE_CUDA_TRY(b.pinned ? cudaFreeHost(b.p) : cudaFree(b.p));
+    b.p = nullptr; b.bytes = 0;
+    QCE_CUDA_TRY(b.pinned ? cudaMallocHost(&b.p, bytes) : cudaMalloc(&b.p, bytes));
+    if (zero_fill) QCE_CUDA_TRY(cudaMemset(b.p, 0, bytes));
+    b.bytes = bytes;
+    return QCE_OK;
+}
+
+inline void free_buf(ScratchBuf& b) {
+    if (b.p) { if (b.pinned) cudaFreeHost(b.p); else cudaFree(b.p); }
+    b.p = nullptr; b.bytes = 0;
+}
 
 struct QuantTables {            // device-resident quantiser tables
     int n_bits;
@@ -86,7 +109,7 @@ struct TcParams {
     int part_cols = 0;          // real columns (of the 2 n_ant) per row block
 };
 
-// host-buffer entry points: the staging sets (pinned + device slots, streams) are pooled per device (qce_api.cu); every model carries an
+// host-buffer entry points: the staging sets (private streams, pinned slots) are pooled per device (qce_api.cu); every model carries an
 // event recorded after its last parameter upload, which the staging streams wait on
 
 struct qce_circ_model {
@@ -145,9 +168,6 @@ struct qce_model {
     double data_scale = 0.0;
     bool params_set = false;
     TcParams tc;
-    // scratch for the fused pipeline (quantised pilots of one chunk)
-    void* pipe_r = nullptr;
-    int64_t pipe_cap = 0;
 };
 
 #ifdef __CUDACC__
@@ -280,6 +300,43 @@ struct RowSource {
     int obs_h_c64 = 0;
     QuantTables qt{};
 };
+
+// Pilot tiles of the dense tensor-core path (qce_dense_tc.cu), shared by all models
+struct TileScratch {
+    ScratchBuf img, bad;                   // zeroed on allocation: the last work unit reads up to 4 tiles past the batch
+    ScratchBuf lp2;                        // [rows][K] float2 log-probabilities (modes other than fused 'all')
+    ScratchBuf wts;                        // [rows][K] float weights
+    ScratchBuf img2;                       // bucketed top-1: pilot tiles regrouped by selected component
+    ScratchBuf bidx;                       // int32: top[rows] | perm[slots] | unit_comp[units] | cnt[K] off[K] cursor[K] n_units
+    const qce_model* owner = nullptr;      // model whose pilots are currently formatted here
+    int64_t rows = 0;
+    // fix list: rows of the formatted batch that are re-evaluated by the complex128 kernel after the tensor-core launches
+    // ([0] is the length, [1] counts the near-ties re-selected so far, the indices follow), and where their pilots come from
+    ScratchBuf fix;
+    RowSource src;
+    // tie list of the chunk in flight ([0] = count, then chunk rows): hard selections too close to call in FP32, re-selected in
+    // complex128 (tc_refine_kernel) before the combine launch
+    ScratchBuf tie;
+    ScratchBuf tmp_est;                    // pair mode: [chunk rows][2N] FP32 rows the (pilot, component) launches add into
+    int* fix_list() const { return (int*)fix.p; }
+    int* tie_list() const { return (int*)tie.p; }
+};
+
+// Every grow-on-demand buffer of the library, one entry per (device, stream) (qce_api.cu): calls on different streams may be in
+// flight at once (host threads on streams of their own, the private streams of the host-buffer path), so no buffer is shared
+// between streams.  An entry is used only by the calls that enqueue work on its stream; the store's mutex guards the map.
+struct StreamScratch {
+    TileScratch tc;
+    ScratchBuf circ_fix;                   // circulant tensor-core fix list: [0] count, [1] unused, then the rows
+    ScratchBuf pipe_r;                     // qce_pipeline, complex128 path: quantised pilots of one chunk
+    ScratchBuf host_in, host_out;          // device slot of a host-buffer call (private staging streams only)
+    ScratchBuf host_mid_in, host_mid_out;  // its device-only intermediates (decoded pilots, complex128 estimates)
+    const int* last_fix = nullptr;         // tc.fix or circ_fix, whichever the latest tensor-core call used: qce_last_fix_count
+};
+StreamScratch* scratch_for(cudaStream_t s);        // creates the stream's entry if it has none
+StreamScratch* scratch_find(cudaStream_t s);       // null if it has none
+void scratch_release(cudaStream_t s);              // frees the entry's buffers and erases it (the stream is about to be destroyed)
+
 qce_status launch_dense_fp64_rows(const qce_model* m, cudaStream_t s, const RowSource& src, const int* rows, const int* n_rows_dev,
                                   int64_t max_rows, int mode, int n_top, double rho, double* h_est, double* logp_out,
                                   const void* h_true, int h_true_c64, double* acc);
@@ -297,7 +354,6 @@ qce_status launch_pipeline_tc(qce_model* m, const QuantTables* qt, cudaStream_t 
                               double* acc);
 bool tc_supported(const qce_model* m, int mode);
 const char* tc_unsupported_reason(const qce_model* m);      // "" or ": <why>", appended to the error message
-void tc_scratch_release(cudaStream_t s);
 // qce_mfa.cu
 qce_status launch_mfa(const qce_mfa_model* m, cudaStream_t s, const double* r, int64_t B, int mode, int n_top, double rho,
                       double* h_est, double* logp_out, const double* h_true, double* acc);

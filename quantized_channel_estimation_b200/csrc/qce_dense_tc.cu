@@ -30,9 +30,6 @@
 // "stage free" / "accumulator ready", remote mbarrier arrives (mapa) for "peer chunk landed" / "accumulator drained".
 // The two tiles ping-pong: while the epilogue warpgroup of tile 0 drains Z|H(k), the tensor core produces
 // Z|H(k) of tile 1, and so on.
-#include <map>
-#include <mutex>
-
 #include "qce_tc_shared.cuh"
 
 namespace qce {
@@ -1514,51 +1511,19 @@ __global__ void __launch_bounds__(256) tc_pair_finish_kernel(const float2* __res
     if (lane == 0 && cnt > 0.0) { atomicAdd(acc + 0, err); atomicAdd(acc + 1, pw); atomicAdd(acc + 2, cnt); }
 }
 
-// keyed by (device, stream): stream handles are only unique per device (the default stream is 0 everywhere)
-static std::mutex g_scratch_mu;
-static std::map<std::pair<int, cudaStream_t>, TileScratch> g_scratch;
-
 static qce_status tc_scratch(const qce_model* m, cudaStream_t s, int64_t rows, TileScratch** out) {
-    std::lock_guard<std::mutex> lock(g_scratch_mu);
-    TileScratch& t = g_scratch[std::make_pair(current_device(), s)];
+    StreamScratch* sc = scratch_for(s);
+    TileScratch& t = sc->tc;
     const size_t tiles = (size_t)((rows + TILE_M - 1) / TILE_M + 4);   // the last work unit (up to 4 tiles) may reach past the end
     const size_t need_img = tiles * TILE_M * 2 * (size_t)m->n_obs * sizeof(__half) * (m->tc.split_a ? 2 : 1), need_bad = tiles * TILE_M;
-    if (need_img > t.img_bytes) {
-        if (t.img) QCE_CUDA_TRY(cudaFree(t.img));
-        t.img = nullptr; t.img_bytes = 0;
-        QCE_CUDA_TRY(cudaMalloc(&t.img, need_img));
-        QCE_CUDA_TRY(cudaMemset(t.img, 0, need_img));
-        t.img_bytes = need_img;
-    }
-    if (need_bad > t.bad_bytes) {
-        if (t.bad) QCE_CUDA_TRY(cudaFree(t.bad));
-        t.bad = nullptr; t.bad_bytes = 0;
-        QCE_CUDA_TRY(cudaMalloc(&t.bad, need_bad));
-        QCE_CUDA_TRY(cudaMemset(t.bad, 0, need_bad));
-        t.bad_bytes = need_bad;
-    }
-    const size_t need_fix = (need_bad + 2) * sizeof(int);       // [0] rows on the list, [1] near-ties re-selected so far, then the list
-    if (need_fix > t.fix_bytes) {
-        if (t.fix_buf) QCE_CUDA_TRY(cudaFree(t.fix_buf));
-        t.fix_buf = nullptr; t.fix_bytes = 0;
-        QCE_CUDA_TRY(cudaMalloc(&t.fix_buf, need_fix));
-        t.fix_bytes = need_fix;
-    }
-    QCE_CUDA_TRY(cudaMemsetAsync(t.fix_buf, 0, 2 * sizeof(int), s));      // a new batch is about to be formatted: empty fix list
-    note_fix_list(s, t.fix_buf);
+    qce_status st = grow(t.img, need_img, true);
+    if (!st) st = grow(t.bad, need_bad, true);
+    if (!st) st = grow(t.fix, (need_bad + 2) * sizeof(int));        // [0] rows on the list, [1] near-ties re-selected so far, then the list
+    if (st) return st;
+    QCE_CUDA_TRY(cudaMemsetAsync(t.fix.p, 0, 2 * sizeof(int), s));      // a new batch is about to be formatted: empty fix list
+    sc->last_fix = t.fix_list();
     *out = &t;
     return QCE_OK;
-}
-
-// a stream is about to be destroyed (the private streams of a model's host-buffer path): free its scratch
-void tc_scratch_release(cudaStream_t s) {
-    std::lock_guard<std::mutex> lock(g_scratch_mu);
-    auto it = g_scratch.find(std::make_pair(current_device(), s));
-    if (it == g_scratch.end()) return;
-    TileScratch& t = it->second;
-    cudaFree(t.img); cudaFree(t.bad); cudaFree(t.lp2); cudaFree(t.wts); cudaFree(t.img2); cudaFree(t.bidx); cudaFree(t.fix_buf); cudaFree(t.tie_buf);
-    cudaFree(t.tmp_est);
-    g_scratch.erase(it);
 }
 
 // complex128 re-evaluation of the rows on the fix list (pilots off the tensor-core grid, hard selections too close to call): they
@@ -1567,48 +1532,15 @@ void tc_scratch_release(cudaStream_t s) {
 static qce_status tc_fix_rows(const qce_model* m, const TileScratch* ts, cudaStream_t s, int64_t B, int mode, int n_top, double rho,
                               double* h_est, double* logp_out, const void* h_true, int h_true_c64, double* acc) {
     if (!h_est && !logp_out && !acc) return QCE_OK;
-    return launch_dense_fp64_rows(m, s, ts->src, ts->fix_buf + 2, ts->fix_buf, B, mode, n_top, rho, h_est, logp_out, h_true, h_true_c64, acc);
+    return launch_dense_fp64_rows(m, s, ts->src, ts->fix_list() + 2, ts->fix_list(), B, mode, n_top, rho, h_est, logp_out, h_true, h_true_c64, acc);
 }
 
+// tie list and [rows][K] log-probability / weight scratch of a chunk of `rows` pilots
 static qce_status tc_scratch_aux(TileScratch* t, size_t rows, size_t K) {
-    std::lock_guard<std::mutex> lock(g_scratch_mu);
-    if ((rows + 1) * sizeof(int) > t->tie_bytes) {
-        if (t->tie_buf) QCE_CUDA_TRY(cudaFree(t->tie_buf));
-        t->tie_buf = nullptr; t->tie_bytes = 0;
-        QCE_CUDA_TRY(cudaMalloc(&t->tie_buf, (rows + 1) * sizeof(int)));
-        t->tie_bytes = (rows + 1) * sizeof(int);
-    }
-    const size_t need_lp = rows * K * sizeof(float2), need_w = rows * K * sizeof(float);
-    if (need_lp > t->lp2_bytes) {
-        if (t->lp2) QCE_CUDA_TRY(cudaFree(t->lp2));
-        t->lp2 = nullptr; t->lp2_bytes = 0;
-        QCE_CUDA_TRY(cudaMalloc(&t->lp2, need_lp));
-        t->lp2_bytes = need_lp;
-    }
-    if (need_w > t->wts_bytes) {
-        if (t->wts) QCE_CUDA_TRY(cudaFree(t->wts));
-        t->wts = nullptr; t->wts_bytes = 0;
-        QCE_CUDA_TRY(cudaMalloc(&t->wts, need_w));
-        t->wts_bytes = need_w;
-    }
-    return QCE_OK;
-}
-
-static qce_status tc_scratch_bucket(TileScratch* t, size_t img2_bytes, size_t idx_ints) {
-    std::lock_guard<std::mutex> lock(g_scratch_mu);
-    if (img2_bytes > t->img2_bytes) {
-        if (t->img2) QCE_CUDA_TRY(cudaFree(t->img2));
-        t->img2 = nullptr; t->img2_bytes = 0;
-        QCE_CUDA_TRY(cudaMalloc(&t->img2, img2_bytes));
-        t->img2_bytes = img2_bytes;
-    }
-    if (idx_ints * sizeof(int) > t->bidx_bytes) {
-        if (t->bidx) QCE_CUDA_TRY(cudaFree(t->bidx));
-        t->bidx = nullptr; t->bidx_bytes = 0;
-        QCE_CUDA_TRY(cudaMalloc(&t->bidx, idx_ints * sizeof(int)));
-        t->bidx_bytes = idx_ints * sizeof(int);
-    }
-    return QCE_OK;
+    qce_status st = grow(t->tie, (rows + 1) * sizeof(int));
+    if (!st) st = grow(t->lp2, rows * K * sizeof(float2));
+    if (!st) st = grow(t->wts, rows * K * sizeof(float));
+    return st;
 }
 
 // fused launch (Z|H in one MMA, estimate row in registers): n_obs, n_ant <= 64
@@ -1800,9 +1732,9 @@ static void tc_fill_args(const qce_model* m, const TileScratch* ts, int64_t B, d
     const TcParams& p = m->tc;
     TcArgs& a = *out;
     a.image = (const __half*)p.image; a.image2 = (const unsigned char*)p.image2; a.zscale = p.zscale; a.hscale = p.hscale; a.zoff = p.zoff; a.hoff = p.hoff;
-    a.logc2 = (const float2*)p.logc2; a.a_img = (const __half*)ts->img; a.bad = (const unsigned char*)ts->bad;
+    a.logc2 = (const float2*)p.logc2; a.a_img = (const __half*)ts->img.p; a.bad = (const unsigned char*)ts->bad.p;
     a.h_est = (double2*)h_est; a.h_true = h_true; a.h_true_c64 = h_true_c64;
-    a.lp_out = (float2*)ts->lp2; a.w_in = (const float*)ts->wts;
+    a.lp_out = (float2*)ts->lp2.p; a.w_in = (const float*)ts->wts.p;
     a.acc = acc; a.B = B; a.K = m->n_comp; a.No = m->n_obs; a.N = m->n_ant;
     a.tri = p.triangular ? 1 : 0;
     a.prof = nullptr;
@@ -1811,7 +1743,7 @@ static void tc_fill_args(const qce_model* m, const TileScratch* ts, int64_t B, d
     a.unit_comp = nullptr; a.perm = nullptr; a.n_units_dev = nullptr;
     a.slot_w = nullptr; a.run_flag = nullptr; a.run_flag_want = 0; a.pair_acc = nullptr;
     a.top_out = nullptr; a.top_flags = m->flags;
-    a.tie_buf = ts->tie_buf;
+    a.tie_buf = ts->tie_list();
     a.tie_eps = (float)tc_tie_eps(m); a.inv_nobs = 1.f / (float)m->n_obs;
 }
 
@@ -1823,7 +1755,7 @@ static qce_status tc_run_split(const qce_model* m, const TileScratch* ts, cudaSt
     TcArgs a;
     tc_fill_args(m, ts, B, h_est, h_true, h_true_c64, acc, &a);
     a.slot_w = slot_w; a.run_flag = run_flag; a.run_flag_want = run_flag_want;
-    a.pair_acc = (float*)ts->tmp_est;
+    a.pair_acc = (float*)ts->tmp_est.p;
     if (unit_comp) { a.unit_comp = unit_comp; a.perm = perm; a.n_units_dev = n_units_dev; a.a_img = (const __half*)bucket_img; }
     a.top_out = top_out;
     a.image2 = (const unsigned char*)(epi == 1 ? p.image_z : p.image_h[part]);
@@ -1894,10 +1826,10 @@ static qce_status tc_format_into(qce_model* m, cudaStream_t s, const double* r, 
     QuantTables none{};
     if (m->tc.split_a)
         tc_format_kernel<false, false, true><<<(unsigned)(tiles * (TILE_M / 8)), 256, 2 * (size_t)(2 * m->n_obs / 8) * 128, s>>>(r, nullptr, 0.0, none, B, m->n_obs, 1.0 / m->tc.eff_scale,
-                                                                                            (__half*)ts->img, (unsigned char*)ts->bad, ts->fix_buf);
+                                                                                            (__half*)ts->img.p, (unsigned char*)ts->bad.p, ts->fix_list());
     else
         tc_format_kernel<false, false, false><<<(unsigned)(tiles * (TILE_M / 8)), 256, (size_t)(2 * m->n_obs / 8) * 128, s>>>(r, nullptr, 0.0, none, B, m->n_obs, 1.0 / m->tc.eff_scale,
-                                                                                             (__half*)ts->img, (unsigned char*)ts->bad, ts->fix_buf);
+                                                                                             (__half*)ts->img.p, (unsigned char*)ts->bad.p, ts->fix_list());
     QCE_CHECK_LAUNCH("tc_format_kernel");
     ts->owner = m; ts->rows = B;
     ts->src = RowSource();
@@ -1955,9 +1887,10 @@ static qce_status tc_run_modes(qce_model* m, TileScratch* ts, cudaStream_t s, in
     const int64_t cap_units = chunk / bucket_rows + m->n_comp + 1, cap_rows = cap_units * bucket_rows;
     int *b_top = nullptr, *b_perm = nullptr, *b_ucomp = nullptr, *b_cnt = nullptr, *b_off = nullptr, *b_cur = nullptr, *b_nu = nullptr;
     if (bucketed) {
-        st = tc_scratch_bucket(ts, (size_t)(cap_rows / TILE_M + 4) * tile_bytes, (size_t)(chunk + cap_rows + cap_units + 3 * m->n_comp + 1));
+        st = grow(ts->img2, (size_t)(cap_rows / TILE_M + 4) * tile_bytes);
+        if (!st) st = grow(ts->bidx, (size_t)(chunk + cap_rows + cap_units + 3 * m->n_comp + 1) * sizeof(int));
         if (st) return st;
-        b_top = (int*)ts->bidx; b_perm = b_top + chunk; b_ucomp = b_perm + cap_rows; b_cnt = b_ucomp + cap_units;
+        b_top = (int*)ts->bidx.p; b_perm = b_top + chunk; b_ucomp = b_perm + cap_rows; b_cnt = b_ucomp + cap_units;
         b_off = b_cnt + m->n_comp; b_cur = b_off + m->n_comp; b_nu = b_cur + m->n_comp;
     }
     // pair mode: perm[slots] | slot_w[slots] | unit_comp[units] | cnt[K] off[K] cursor[K] | n_units | dense_flag
@@ -1965,26 +1898,18 @@ static qce_status tc_run_modes(qce_model* m, TileScratch* ts, cudaStream_t s, in
     int *p_perm = nullptr, *p_ucomp = nullptr, *p_cnt = nullptr, *p_off = nullptr, *p_cur = nullptr, *p_nu = nullptr, *p_dense = nullptr;
     float* p_w = nullptr;
     if (pairs && !bucketed) {
-        st = tc_scratch_bucket(ts, (size_t)(p_rows / TILE_M + 4) * tile_bytes, (size_t)(2 * p_rows + p_units + 3 * m->n_comp + 2));
+        st = grow(ts->img2, (size_t)(p_rows / TILE_M + 4) * tile_bytes);
+        if (!st) st = grow(ts->bidx, (size_t)(2 * p_rows + p_units + 3 * m->n_comp + 2) * sizeof(int));
+        if (!st) st = grow(ts->tmp_est, (size_t)chunk * m->n_ant * 8);          // FP32 rows the pair launches add into
         if (st) return st;
-        p_perm = (int*)ts->bidx; p_w = (float*)(p_perm + p_rows); p_ucomp = p_perm + 2 * p_rows; p_cnt = p_ucomp + p_units;
+        p_perm = (int*)ts->bidx.p; p_w = (float*)(p_perm + p_rows); p_ucomp = p_perm + 2 * p_rows; p_cnt = p_ucomp + p_units;
         p_off = p_cnt + m->n_comp; p_cur = p_off + m->n_comp; p_nu = p_cur + m->n_comp; p_dense = p_nu + 1;
-        {                  // FP32 rows the pair launches add into
-            std::lock_guard<std::mutex> lock(g_scratch_mu);
-            const size_t need = (size_t)chunk * m->n_ant * 8;
-            if (need > ts->tmp_est_bytes) {
-                if (ts->tmp_est) QCE_CUDA_TRY(cudaFree(ts->tmp_est));
-                ts->tmp_est = nullptr; ts->tmp_est_bytes = 0;
-                QCE_CUDA_TRY(cudaMalloc(&ts->tmp_est, need));
-                ts->tmp_est_bytes = need;
-            }
-        }
     }
     for (int64_t b0 = 0; b0 < B; b0 += chunk) {
         const int64_t nb = (B - b0) < chunk ? (B - b0) : chunk;
         TileScratch v = *ts;                                   // view of this chunk's tiles (b0 is a multiple of the tile size)
-        v.img = (unsigned char*)ts->img + (size_t)(b0 / TILE_M) * tile_bytes;
-        v.bad = (unsigned char*)ts->bad + b0;
+        v.img.p = (unsigned char*)ts->img.p + (size_t)(b0 / TILE_M) * tile_bytes;
+        v.bad.p = (unsigned char*)ts->bad.p + b0;
         double* he = h_est ? h_est + (size_t)b0 * m->n_ant * 2 : nullptr;
         double* lo = logp_out ? logp_out + (size_t)b0 * m->n_comp : nullptr;
         const void* ht = h_true ? (const void*)((const char*)h_true + (size_t)b0 * true_row) : nullptr;
@@ -1993,7 +1918,7 @@ static qce_status tc_run_modes(qce_model* m, TileScratch* ts, cudaStream_t s, in
         // hard selections: pilots whose selection is too close to call go on the chunk's tie list (QCE_TC_TIE_EPS=0: nobody does)
         const double eps = tc_tie_eps(m);
         const bool refine = want_est && mode != QCE_MODE_ALL && eps > 0.0 && (ts->src.r || ts->src.obs_h);
-        QCE_CUDA_TRY(cudaMemsetAsync(ts->tie_buf, 0, sizeof(int), s));
+        QCE_CUDA_TRY(cudaMemsetAsync(ts->tie_list(), 0, sizeof(int), s));
         st = tc_run_split(m, &v, s, nb, 1, 0, nullptr, nullptr, 0, nullptr, nullptr, nullptr, nullptr, nullptr, label_in_kernel ? b_top : nullptr);
         if (st) return st;
         if (bucketed) {
@@ -2004,18 +1929,18 @@ static qce_status tc_run_modes(qce_model* m, TileScratch* ts, cudaStream_t s, in
         const bool fused_count = pair_chunk && m->n_comp <= 256;      // the thread-per-pilot selection counts the pairs itself
         if (pair_chunk) QCE_CUDA_TRY(cudaMemsetAsync(p_cnt, 0, m->n_comp * sizeof(int), s));
         if (!label_in_kernel) {
-            float* wts = (want_est && !bucketed) ? (float*)v.wts : nullptr;
-            const unsigned char* vb = (const unsigned char*)v.bad;
+            float* wts = (want_est && !bucketed) ? (float*)v.wts.p : nullptr;
+            const unsigned char* vb = (const unsigned char*)v.bad.p;
             const int K = m->n_comp;
             if (K <= 256) {
                 const size_t sm = (size_t)2 * K * (SEL_ROWS + 1) * sizeof(float) + (size_t)K * sizeof(int);
                 static PerDeviceOnce once;
                 if (once.first(current_device()))
                     QCE_CUDA_TRY(cudaFuncSetAttribute(tc_select_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-                tc_select_rows_kernel<<<(unsigned)((nb + SEL_ROWS - 1) / SEL_ROWS), SEL_THREADS, sm, s>>>((const float2*)v.lp2, nb, K, mode, n_top, rho, m->flags,
-                    wts, lo, b_top, vb, ts->tie_buf, eps, m->logc, 1.0 / m->n_obs, fused_count ? p_cnt : nullptr, pair_thresh);
+                tc_select_rows_kernel<<<(unsigned)((nb + SEL_ROWS - 1) / SEL_ROWS), SEL_THREADS, sm, s>>>((const float2*)v.lp2.p, nb, K, mode, n_top, rho, m->flags,
+                    wts, lo, b_top, vb, ts->tie_list(), eps, m->logc, 1.0 / m->n_obs, fused_count ? p_cnt : nullptr, pair_thresh);
             } else {
-                tc_select_kernel<32><<<(unsigned)((nb + 7) / 8), 256, 0, s>>>((const float2*)v.lp2, nb, K, mode, n_top, rho, m->flags, wts, lo, b_top, vb, ts->tie_buf, eps, nullptr, m->logc, 1.0 / m->n_obs);
+                tc_select_kernel<32><<<(unsigned)((nb + 7) / 8), 256, 0, s>>>((const float2*)v.lp2.p, nb, K, mode, n_top, rho, m->flags, wts, lo, b_top, vb, ts->tie_list(), eps, nullptr, m->logc, 1.0 / m->n_obs);
             }
             QCE_CHECK_LAUNCH("tc_select kernel");
         }
@@ -2024,54 +1949,54 @@ static qce_status tc_run_modes(qce_model* m, TileScratch* ts, cudaStream_t s, in
             RefineArgs ra;
             ra.No = m->n_obs; ra.K = m->n_comp; ra.tri = m->tc.triangular ? 1 : 0;
             ra.Linv = (const double2*)m->Linv; ra.zoff = (const double2*)m->zoff; ra.logc = m->logc;
-            ra.src = ts->src; ra.row0 = b0; ra.tie_buf = ts->tie_buf; ra.tie_total = ts->fix_buf + 1;
-            ra.lp2 = (float2*)v.lp2; ra.logp_out = lo;
+            ra.src = ts->src; ra.row0 = b0; ra.tie_buf = ts->tie_list(); ra.tie_total = ts->fix_list() + 1;
+            ra.lp2 = (float2*)v.lp2.p; ra.logp_out = lo;
             int sms = 148;
             cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, current_device());
             const size_t rsm = (size_t)REFINE_RT * m->n_obs * sizeof(double2);
             tc_refine_kernel<<<(unsigned)(4 * sms), 256, rsm, s>>>(ra);
             QCE_CHECK_LAUNCH("tc_refine_kernel");
-            float* wts = bucketed ? nullptr : (float*)v.wts;
+            float* wts = bucketed ? nullptr : (float*)v.wts.p;
             const unsigned sgrid = (unsigned)sms;
             int* pc = fused_count ? p_cnt : nullptr;
-            if (m->n_comp <= 64) tc_select_kernel<2, true><<<sgrid, 256, 0, s>>>((const float2*)v.lp2, nb, m->n_comp, mode, n_top, rho, m->flags, wts, nullptr, b_top, nullptr, nullptr, 0.0, ts->tie_buf, nullptr, 0.0, pc, pair_thresh);
-            else if (m->n_comp <= 256) tc_select_kernel<8, true><<<sgrid, 256, 0, s>>>((const float2*)v.lp2, nb, m->n_comp, mode, n_top, rho, m->flags, wts, nullptr, b_top, nullptr, nullptr, 0.0, ts->tie_buf, nullptr, 0.0, pc, pair_thresh);
-            else tc_select_kernel<32, true><<<sgrid, 256, 0, s>>>((const float2*)v.lp2, nb, m->n_comp, mode, n_top, rho, m->flags, wts, nullptr, b_top, nullptr, nullptr, 0.0, ts->tie_buf, nullptr, 0.0, pc, pair_thresh);
+            if (m->n_comp <= 64) tc_select_kernel<2, true><<<sgrid, 256, 0, s>>>((const float2*)v.lp2.p, nb, m->n_comp, mode, n_top, rho, m->flags, wts, nullptr, b_top, nullptr, nullptr, 0.0, ts->tie_list(), nullptr, 0.0, pc, pair_thresh);
+            else if (m->n_comp <= 256) tc_select_kernel<8, true><<<sgrid, 256, 0, s>>>((const float2*)v.lp2.p, nb, m->n_comp, mode, n_top, rho, m->flags, wts, nullptr, b_top, nullptr, nullptr, 0.0, ts->tie_list(), nullptr, 0.0, pc, pair_thresh);
+            else tc_select_kernel<32, true><<<sgrid, 256, 0, s>>>((const float2*)v.lp2.p, nb, m->n_comp, mode, n_top, rho, m->flags, wts, nullptr, b_top, nullptr, nullptr, 0.0, ts->tie_list(), nullptr, 0.0, pc, pair_thresh);
             QCE_CHECK_LAUNCH("tc_select_kernel(list)");
         }
         if (bucketed) {
             tc_bucket_count_kernel<<<(unsigned)((nb + 1023) / 1024), 1024, 0, s>>>(b_top, nb, m->n_comp, b_cnt);
             tc_bucket_scan_kernel<<<1, 1024, 0, s>>>(b_cnt, m->n_comp, bucket_rows, b_off, b_cur, b_ucomp, b_nu);
             tc_bucket_place_kernel<<<(unsigned)((nb + 1023) / 1024), 1024, 0, s>>>(b_top, nb, m->n_comp, b_off, b_cur, b_perm);
-            tc_bucket_gather_kernel<<<(unsigned)(cap_rows / TILE_M), 256, 0, s>>>((const unsigned char*)v.img, b_perm, b_nu, tiles_per_unit,
-                                                                                  2 * m->n_obs / 8, m->tc.split_a ? 2 : 1, (unsigned char*)ts->img2);
+            tc_bucket_gather_kernel<<<(unsigned)(cap_rows / TILE_M), 256, 0, s>>>((const unsigned char*)v.img.p, b_perm, b_nu, tiles_per_unit,
+                                                                                  2 * m->n_obs / 8, m->tc.split_a ? 2 : 1, (unsigned char*)ts->img2.p);
             QCE_CHECK_LAUNCH("tc_bucket kernels");
             for (int part = 0; part < m->tc.h_parts; ++part) {
-                st = tc_run_split(m, &v, s, cap_rows, 2, part, he, ht, h_true_c64, acc, b_ucomp, b_perm, b_nu, ts->img2);
+                st = tc_run_split(m, &v, s, cap_rows, 2, part, he, ht, h_true_c64, acc, b_ucomp, b_perm, b_nu, ts->img2.p);
                 if (st) return st;
             }
             continue;
         }
         if (pairs && !bucketed) {
             const unsigned g1 = (unsigned)((nb + 1023) / 1024);
-            const unsigned char* vb = (const unsigned char*)v.bad;
+            const unsigned char* vb = (const unsigned char*)v.bad.p;
             QCE_CUDA_TRY(cudaMemsetAsync(p_perm, 0xFF, (size_t)p_rows * sizeof(int), s));          // -1 = padding slot
-            QCE_CUDA_TRY(cudaMemsetAsync(ts->tmp_est, 0, (size_t)nb * m->n_ant * 8, s));           // the pair rows are added into zeros
-            if (!fused_count) tc_pair_count_kernel<<<g1, 1024, 0, s>>>((const float*)v.wts, vb, nb, m->n_comp, pair_thresh, p_cnt);
+            QCE_CUDA_TRY(cudaMemsetAsync(ts->tmp_est.p, 0, (size_t)nb * m->n_ant * 8, s));           // the pair rows are added into zeros
+            if (!fused_count) tc_pair_count_kernel<<<g1, 1024, 0, s>>>((const float*)v.wts.p, vb, nb, m->n_comp, pair_thresh, p_cnt);
             tc_pair_scan_kernel<<<1, 1024, 0, s>>>(p_cnt, m->n_comp, bucket_rows, (int)(p_units - 1), p_off, p_cur, p_ucomp, p_nu, p_dense);
-            tc_pair_place_kernel<<<g1, 1024, 0, s>>>((const float*)v.wts, vb, nb, m->n_comp, pair_thresh, p_off, p_cur, p_dense, p_perm, p_w);
-            tc_bucket_gather_kernel<<<(unsigned)(p_rows / TILE_M), 256, 0, s>>>((const unsigned char*)v.img, p_perm, p_nu, tiles_per_unit,
-                                                                                2 * m->n_obs / 8, m->tc.split_a ? 2 : 1, (unsigned char*)ts->img2);
+            tc_pair_place_kernel<<<g1, 1024, 0, s>>>((const float*)v.wts.p, vb, nb, m->n_comp, pair_thresh, p_off, p_cur, p_dense, p_perm, p_w);
+            tc_bucket_gather_kernel<<<(unsigned)(p_rows / TILE_M), 256, 0, s>>>((const unsigned char*)v.img.p, p_perm, p_nu, tiles_per_unit,
+                                                                                2 * m->n_obs / 8, m->tc.split_a ? 2 : 1, (unsigned char*)ts->img2.p);
             QCE_CHECK_LAUNCH("tc_pair kernels");
             count_launch(fused_count ? 2 : 3);
             for (int part = 0; part < m->tc.h_parts; ++part) {
-                st = tc_run_split(m, &v, s, p_rows, 2, part, nullptr, nullptr, 0, nullptr, p_ucomp, p_perm, p_nu, ts->img2, nullptr, p_w);
+                st = tc_run_split(m, &v, s, p_rows, 2, part, nullptr, nullptr, 0, nullptr, p_ucomp, p_perm, p_nu, ts->img2.p, nullptr, p_w);
                 if (st) return st;
             }
             {
                 int sms = 148;
                 cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, current_device());
-                tc_pair_finish_kernel<<<(unsigned)(8 * sms), 256, 0, s>>>((const float2*)ts->tmp_est, (double2*)he, ht, h_true_c64, vb, nb, m->n_ant,
+                tc_pair_finish_kernel<<<(unsigned)(8 * sms), 256, 0, s>>>((const float2*)ts->tmp_est.p, (double2*)he, ht, h_true_c64, vb, nb, m->n_ant,
                                                                           p_dense, acc);
                 QCE_CHECK_LAUNCH("tc_pair_finish_kernel");
             }
@@ -2189,7 +2114,7 @@ static qce_status tc_run_hard_top1(qce_model* m, TileScratch* ts, cudaStream_t s
     if (refine) {
         st = tc_scratch_aux(ts, (size_t)chunk, (size_t)K);                       // tie list, FP32 pairs of the listed pilots
         if (st) return st;
-        st = tc_scratch_bucket(ts, 0, (size_t)chunk);                            // exact labels of the listed pilots
+        st = grow(ts->bidx, (size_t)chunk * sizeof(int));                        // exact labels of the listed pilots
         if (st) return st;
     }
     const size_t tile_bytes = (size_t)TILE_M * 2 * m->n_obs * sizeof(__half);
@@ -2200,13 +2125,13 @@ static qce_status tc_run_hard_top1(qce_model* m, TileScratch* ts, cudaStream_t s
     for (int64_t b0 = 0; b0 < B; b0 += chunk) {
         const int64_t nb = (B - b0) < chunk ? (B - b0) : chunk;
         TileScratch v = *ts;
-        v.img = (unsigned char*)ts->img + (size_t)(b0 / TILE_M) * tile_bytes;
-        v.bad = (unsigned char*)ts->bad + b0;
+        v.img.p = (unsigned char*)ts->img.p + (size_t)(b0 / TILE_M) * tile_bytes;
+        v.bad.p = (unsigned char*)ts->bad.p + b0;
         double* he = h_est ? h_est + (size_t)b0 * m->n_ant * 2 : nullptr;
         const void* ht = h_true ? (const void*)((const char*)h_true + (size_t)b0 * true_row) : nullptr;
         TcArgs a;
         tc_fill_args(m, &v, nb, he, ht, h_true_c64, acc, &a);
-        if (refine) QCE_CUDA_TRY(cudaMemsetAsync(ts->tie_buf, 0, sizeof(int), s));
+        if (refine) QCE_CUDA_TRY(cudaMemsetAsync(ts->tie_list(), 0, sizeof(int), s));
         else a.tie_buf = nullptr;                                              // nobody is handed to the exact path: every pilot is answered here
         const bool offs = m->tc.has_offsets;
         bool hit = false;
@@ -2219,20 +2144,20 @@ static qce_status tc_run_hard_top1(qce_model* m, TileScratch* ts, cudaStream_t s
         RefineArgs ra;
         ra.No = m->n_obs; ra.K = K; ra.tri = 1;
         ra.Linv = (const double2*)m->Linv; ra.zoff = (const double2*)m->zoff; ra.logc = m->logc;
-        ra.src = ts->src; ra.row0 = b0; ra.tie_buf = ts->tie_buf; ra.tie_total = ts->fix_buf + 1;
-        ra.lp2 = (float2*)ts->lp2; ra.logp_out = nullptr;
+        ra.src = ts->src; ra.row0 = b0; ra.tie_buf = ts->tie_list(); ra.tie_total = ts->fix_list() + 1;
+        ra.lp2 = (float2*)ts->lp2.p; ra.logp_out = nullptr;
         tc_refine_kernel<<<(unsigned)(4 * sms), 256, (size_t)REFINE_RT * m->n_obs * sizeof(double2), s>>>(ra);
         QCE_CHECK_LAUNCH("tc_refine_kernel");
-        int* top = (int*)ts->bidx;
+        int* top = (int*)ts->bidx.p;
         const unsigned sgrid = (unsigned)sms;
-        if (K <= 64) tc_select_kernel<2, true><<<sgrid, 256, 0, s>>>((const float2*)ts->lp2, nb, K, QCE_MODE_TOP1, 1, 0.0, m->flags, nullptr, nullptr, top, nullptr, nullptr, 0.0, ts->tie_buf, nullptr, 0.0, nullptr, 0.f);
-        else if (K <= 256) tc_select_kernel<8, true><<<sgrid, 256, 0, s>>>((const float2*)ts->lp2, nb, K, QCE_MODE_TOP1, 1, 0.0, m->flags, nullptr, nullptr, top, nullptr, nullptr, 0.0, ts->tie_buf, nullptr, 0.0, nullptr, 0.f);
-        else tc_select_kernel<32, true><<<sgrid, 256, 0, s>>>((const float2*)ts->lp2, nb, K, QCE_MODE_TOP1, 1, 0.0, m->flags, nullptr, nullptr, top, nullptr, nullptr, 0.0, ts->tie_buf, nullptr, 0.0, nullptr, 0.f);
+        if (K <= 64) tc_select_kernel<2, true><<<sgrid, 256, 0, s>>>((const float2*)ts->lp2.p, nb, K, QCE_MODE_TOP1, 1, 0.0, m->flags, nullptr, nullptr, top, nullptr, nullptr, 0.0, ts->tie_list(), nullptr, 0.0, nullptr, 0.f);
+        else if (K <= 256) tc_select_kernel<8, true><<<sgrid, 256, 0, s>>>((const float2*)ts->lp2.p, nb, K, QCE_MODE_TOP1, 1, 0.0, m->flags, nullptr, nullptr, top, nullptr, nullptr, 0.0, ts->tie_list(), nullptr, 0.0, nullptr, 0.f);
+        else tc_select_kernel<32, true><<<sgrid, 256, 0, s>>>((const float2*)ts->lp2.p, nb, K, QCE_MODE_TOP1, 1, 0.0, m->flags, nullptr, nullptr, top, nullptr, nullptr, 0.0, ts->tie_list(), nullptr, 0.0, nullptr, 0.f);
         QCE_CHECK_LAUNCH("tc_select_kernel(list)");
         Top1RowsArgs ta;
         ta.No = m->n_obs; ta.N = m->n_ant; ta.K = K;
         ta.W = (const double2*)m->W; ta.hoff = (const double2*)m->hoff;
-        ta.src = ts->src; ta.row0 = b0; ta.tie_buf = ts->tie_buf; ta.top = top;
+        ta.src = ts->src; ta.row0 = b0; ta.tie_buf = ts->tie_list(); ta.top = top;
         ta.h_est = (double2*)he; ta.h_true = ht; ta.h_true_c64 = h_true_c64; ta.acc = acc;
         tc_top1_rows_kernel<<<(unsigned)sms, 256, (size_t)8 * m->n_obs * sizeof(double2), s>>>(ta);
         QCE_CHECK_LAUNCH("tc_top1_rows_kernel");
@@ -2242,12 +2167,8 @@ static qce_status tc_run_hard_top1(qce_model* m, TileScratch* ts, cudaStream_t s
 }
 
 qce_status tc_estimate_formatted(qce_model* m, cudaStream_t s, int64_t B, double* h_est, const void* h_true, int h_true_c64, double* acc) {
-    TileScratch* ts = nullptr;
-    {
-        std::lock_guard<std::mutex> lock(g_scratch_mu);
-        auto it = g_scratch.find(std::make_pair(current_device(), s));
-        if (it != g_scratch.end()) ts = &it->second;
-    }
+    StreamScratch* sc = scratch_find(s);
+    TileScratch* ts = sc ? &sc->tc : nullptr;
     if (!ts || ts->owner != m || B > ts->rows) {
         set_error("qce_estimate_formatted: no pilots of this model are formatted on this stream (or fewer than %lld)", (long long)B);
         return QCE_ERR_INVALID;
@@ -2289,7 +2210,7 @@ qce_status launch_pipeline_tc(qce_model* m, const QuantTables* qt, cudaStream_t 
     const unsigned grid = (unsigned)(tiles * (TILE_M / 8));
     const double inv_scale = 1.0 / m->tc.eff_scale;
 #define QCE_FMT(C64, SPL) tc_format_kernel<true, C64, SPL><<<grid, 256, smem, s>>>(h, (const double2*)noise, noise_scale, *qt, B, m->n_obs, inv_scale, \
-                                                                                 (__half*)ts->img, (unsigned char*)ts->bad, ts->fix_buf)
+                                                                                 (__half*)ts->img.p, (unsigned char*)ts->bad.p, ts->fix_list())
     if (h_is_c64) { if (m->tc.split_a) QCE_FMT(true, true); else QCE_FMT(true, false); }
     else { if (m->tc.split_a) QCE_FMT(false, true); else QCE_FMT(false, false); }
 #undef QCE_FMT

@@ -1,5 +1,5 @@
-// Shared pieces of the tensor-core kernels: kernel arguments, mbarrier / bulk-copy / tcgen05 PTX wrappers and pilot-tile
-// scratch of qce_dense_tc.cu; the mma.sync split-FP16 helpers of qce_circ_tc.cu and qce_rate.cu.
+// Shared pieces of the tensor-core kernels: kernel arguments and mbarrier / bulk-copy / tcgen05 PTX wrappers of qce_dense_tc.cu;
+// the mma.sync split-FP16 helpers of qce_circ_tc.cu and qce_rate.cu.
 #pragma once
 #include <math.h>
 #include <stdlib.h>
@@ -220,34 +220,5 @@ __device__ __forceinline__ void split_half(const float x, __half& hi, __half& lo
     hi = __float2half_rn(x);
     lo = __float2half_rn(x - __half2float(hi));
 }
-
-
-// Pilot-tile scratch: one buffer set per CUDA stream (calls on different streams may be in flight concurrently, e.g. the
-// double-buffered host path), shared by all models, grown on demand outside the steady state.
-struct TileScratch {
-    void* img = nullptr;
-    void* bad = nullptr;
-    void* lp2 = nullptr;                   // [rows][K] float2 log-probabilities (modes other than fused 'all')
-    void* wts = nullptr;                   // [rows][K] float weights
-    size_t img_bytes = 0, bad_bytes = 0, lp2_bytes = 0, wts_bytes = 0;
-    void* img2 = nullptr;                  // bucketed top-1: pilot tiles regrouped by selected component
-    void* bidx = nullptr;                  // int32: top[rows] | perm[slots] | unit_comp[units] | cnt[K] off[K] cursor[K] n_units
-    size_t img2_bytes = 0, bidx_bytes = 0;
-    const qce_model* owner = nullptr;      // model whose pilots are currently formatted here
-    int64_t rows = 0;
-    // fix list: rows of the formatted batch that are re-evaluated by the complex128 kernel after the tensor-core launches
-    // ([0] of fix_buf is the length, [1] counts the near-ties re-selected so far, the indices follow), and where their pilots come from
-    int* fix_buf = nullptr;
-    size_t fix_bytes = 0;
-    RowSource src;
-    // tie list of the chunk in flight ([0] = count, then chunk rows): hard selections too close to call in FP32, re-selected in
-    // complex128 (tc_refine_kernel) before the combine launch
-    int* tie_buf = nullptr;
-    size_t tie_bytes = 0;
-    void* tmp_est = nullptr;               // pair mode: [chunk rows][2N] FP32 rows the (pilot, component) launches add into
-    size_t tmp_est_bytes = 0;
-};
-
-
 
 }  // namespace qce
