@@ -279,6 +279,14 @@ static qce_status check_mode(int mode, int n_top, double rho, int K) {
     (void)K;
 }
 
+// the tensor-core kernels of `mode` for this model, or QCE_ERR_UNSUPPORTED and why not
+static qce_status tc_require(const qce_model* m, int mode, const char* fn) {
+    if (tc_supported(m, mode) && m->tc.ready) return QCE_OK;
+    set_error("%s: tensor-core kernel does not support n_obs=%d n_ant=%d K=%d mode=%d%s", fn, m->n_obs, m->n_ant, m->n_comp, mode,
+              tc_unsupported_reason(m));
+    return QCE_ERR_UNSUPPORTED;
+}
+
 static qce_status estimate_impl(qce_model* m, cudaStream_t s, const double* r, int64_t B, int mode, int n_top, double rho,
                                 int precision, double* h_est, double* logp_out, const void* h_true, int h_true_c64,
                                 double* acc) {
@@ -289,10 +297,8 @@ static qce_status estimate_impl(qce_model* m, cudaStream_t s, const double* r, i
     if (precision == QCE_PREC_FP64)
         return launch_dense_fp64_raw(m, s, r, B, mode, n_top, rho, h_est, logp_out, h_true, h_true_c64, acc);
     if (precision == QCE_PREC_TC) {
-        if (!tc_supported(m, mode) || !m->tc.ready) {
-            set_error("tensor-core kernel does not support n_obs=%d n_ant=%d K=%d mode=%d%s", m->n_obs, m->n_ant, m->n_comp, mode, tc_unsupported_reason(m));
-            return QCE_ERR_UNSUPPORTED;
-        }
+        st = tc_require(m, mode, "qce_estimate");
+        if (st) return st;
         return launch_dense_tc(m, s, r, B, mode, n_top, rho, h_est, logp_out, h_true, h_true_c64, acc);
     }
     set_error("unknown precision %d", precision);
@@ -318,10 +324,8 @@ qce_status qce_pipeline(qce_model* m, const qce_quantizer* q, void* stream, cons
         if (stm) return stm;
     }
     if (precision == QCE_PREC_TC) {
-        if (!tc_supported(m, mode) || !m->tc.ready) {
-            set_error("tensor-core kernel does not support n_obs=%d n_ant=%d K=%d mode=%d%s", m->n_obs, m->n_ant, m->n_comp, mode, tc_unsupported_reason(m));
-            return QCE_ERR_UNSUPPORTED;
-        }
+        qce_status st = tc_require(m, mode, "qce_pipeline");
+        if (st) return st;
         // one formatter launch (observe + quantise + FP16 tiles) and one estimate launch per 2^22 pilots
         const int64_t chunk = (int64_t)1 << 22;
         const size_t hs = h_is_c64 ? 8 : 16;
@@ -516,13 +520,15 @@ qce_status qce_rate_accumulate(qce_rate_model* m, void* stream, const void* h_es
 
 qce_status qce_format_pilots(qce_model* m, void* stream, const void* r, int64_t B) {
     if (!m || !m->params_set || B < 0 || (B > 0 && !r)) { set_error("qce_format_pilots: invalid argument"); return QCE_ERR_INVALID; }
-    if (!tc_supported(m, QCE_MODE_ALL) || !m->tc.ready) { set_error("qce_format_pilots: tensor-core path not available for this model"); return QCE_ERR_UNSUPPORTED; }
+    qce_status st = tc_require(m, QCE_MODE_ALL, "qce_format_pilots");
+    if (st) return st;
     return tc_format(m, (cudaStream_t)stream, (const double*)r, B);
 }
 
 qce_status qce_estimate_formatted(qce_model* m, void* stream, int64_t B, void* h_est, const void* h_true, double* acc) {
     if (!m || !m->params_set || B < 0) { set_error("qce_estimate_formatted: invalid argument"); return QCE_ERR_INVALID; }
-    if (!tc_supported(m, QCE_MODE_ALL) || !m->tc.ready) { set_error("qce_estimate_formatted: tensor-core path not available for this model"); return QCE_ERR_UNSUPPORTED; }
+    qce_status st = tc_require(m, QCE_MODE_ALL, "qce_estimate_formatted");
+    if (st) return st;
     return tc_estimate_formatted(m, (cudaStream_t)stream, B, (double*)h_est, h_true, 0, acc);
 }
 

@@ -1511,11 +1511,20 @@ __global__ void __launch_bounds__(256) tc_pair_finish_kernel(const float2* __res
     if (lane == 0 && cnt > 0.0) { atomicAdd(acc + 0, err); atomicAdd(acc + 1, pw); atomicAdd(acc + 2, cnt); }
 }
 
+static int sm_count() {
+    int sms = 148;
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, current_device());
+    return sms;
+}
+
+// bytes of one FP16 pilot tile: TILE_M rows of 2 n_obs halves, twice for (hi, lo) pairs of pilots off the integer grid
+static size_t tc_tile_bytes(const qce_model* m) { return (size_t)TILE_M * 2 * m->n_obs * sizeof(__half) * (m->tc.split_a ? 2 : 1); }
+
 static qce_status tc_scratch(const qce_model* m, cudaStream_t s, int64_t rows, TileScratch** out) {
     StreamScratch* sc = scratch_for(s);
     TileScratch& t = sc->tc;
     const size_t tiles = (size_t)((rows + TILE_M - 1) / TILE_M + 4);   // the last work unit (up to 4 tiles) may reach past the end
-    const size_t need_img = tiles * TILE_M * 2 * (size_t)m->n_obs * sizeof(__half) * (m->tc.split_a ? 2 : 1), need_bad = tiles * TILE_M;
+    const size_t need_img = tiles * tc_tile_bytes(m), need_bad = tiles * TILE_M;
     qce_status st = grow(t.img, need_img, true);
     if (!st) st = grow(t.bad, need_bad, true);
     if (!st) st = grow(t.fix, (need_bad + 2) * sizeof(int));        // [0] rows on the list, [1] near-ties re-selected so far, then the list
@@ -1543,21 +1552,32 @@ static qce_status tc_scratch_aux(TileScratch* t, size_t rows, size_t K) {
     return st;
 }
 
-// fused launch (Z|H in one MMA, estimate row in registers): n_obs, n_ant <= 64
+// The instantiated shapes, as X(n_obs / 16, part_cols / 32): the 2 n_obs whitening columns and one block of part_cols estimate
+// columns.  Fused shapes (n_obs, n_ant <= 64): Z|H in one MMA, estimate row in registers, part_cols = 2 n_ant; every launch family
+// is instantiated for them.
+#define QCE_TC_FUSED_SHAPES(X) X(4, 4) X(2, 2) X(1, 1) X(3, 3) X(4, 2) X(2, 1)
+// Split-only shapes: the 2 n_ant estimate columns are produced in row blocks of part_cols <= 128 (64 packed register accumulators
+// per pilot), the 2 n_obs whitening columns by a launch of their own; only the split launches are instantiated for them.  n_ant is
+// n_obs (one pilot per antenna) or n_obs / 2 (two pilots per antenna, A = kron([1, j], I)).
+#define QCE_TC_SPLIT_SHAPES(X) X(16, 4) X(8, 4) X(6, 3)
+
 static bool tc_instantiated(const qce_model* m) {
-    if (m->n_obs % 16 || m->n_ant % 16) return false;
-    const int cz = m->n_obs / 16, ch = m->n_ant / 16;
-    return (cz == ch && cz >= 1 && cz <= 4) || (cz == 4 && ch == 2) || (cz == 2 && ch == 1);
+#define QCE_TC_FUSED_HIT(Z, H) if (m->n_obs == 16 * Z && m->n_ant == 16 * H) return true;
+    QCE_TC_FUSED_SHAPES(QCE_TC_FUSED_HIT)
+#undef QCE_TC_FUSED_HIT
+    return false;
 }
 
-// split launches: the 2 n_ant estimate columns are produced in row blocks of at most 128 (64 packed register accumulators
-// per pilot), the 2 n_obs whitening columns by a launch of their own.  n_obs = 256: one pilot per antenna, or two pilots on 128
-// antennas (A = kron([1, j], I))
 static bool tc_split_shape(int No, int N, int* parts, int* part_cols) {
-    if (No == 256 && (N == 128 || N == 256)) { *part_cols = 128; *parts = 2 * N / 128; return true; }
-    if (No == 128 && (N == 64 || N == 128)) { *part_cols = 128; *parts = 2 * N / 128; return true; }
-    if (No == 96 && (N == 48 || N == 96)) { *part_cols = 96; *parts = 2 * N / 96; return true; }
+#define QCE_TC_SPLIT_HIT(Z, H) if (No == 16 * Z && (N == No || 2 * N == No)) { *part_cols = 32 * H; *parts = 2 * N / (32 * H); return true; }
+    QCE_TC_SPLIT_SHAPES(QCE_TC_SPLIT_HIT)
+#undef QCE_TC_SPLIT_HIT
     return false;
+}
+
+static qce_status tc_not_instantiated(const qce_model* m) {
+    set_error("tensor-core kernel: n_obs=%d n_ant=%d not instantiated", m->n_obs, m->n_ant);
+    return QCE_ERR_UNSUPPORTED;
 }
 
 // n_obs = 256 with pilots off the integer grid: a (hi, lo) pilot tile pair would take 256 KB of shared memory
@@ -1657,17 +1677,32 @@ qce_status tc_pack_params(qce_model* m, cudaStream_t s) {
     return QCE_OK;
 }
 
+// QCE_TC_PROF (with a -DQCE_TC_PROFILE build): per-role cycle counters of CTA 0, printed after every dense_tc_kernel launch
+static long long* tc_prof_counters(cudaStream_t s) {
+    static long long* prof = nullptr;
+    static const bool want_prof = getenv("QCE_TC_PROF") != nullptr;
+    if (!want_prof) return nullptr;
+    if (!prof) cudaMalloc(&prof, 16 * sizeof(long long));
+    cudaMemsetAsync(prof, 0, 16 * sizeof(long long), s);
+    return prof;
+}
+
+static void tc_prof_print(const TcArgs& a, int epi, cudaStream_t s) {
+    long long h[16];
+    cudaMemcpyAsync(h, a.prof, sizeof(h), cudaMemcpyDeviceToHost, s);
+    cudaStreamSynchronize(s);
+    fprintf(stderr, "[qce tc prof] epi %d B=%lld K=%d | mma: total %lld wait_acc_empty %lld wait_full %lld wait_a %lld | epi t0: wait %lld z %lld h %lld pro %lld | epi t1: wait %lld z %lld h %lld pro %lld | zld t0 %lld t1 %lld\n",
+            epi, (long long)a.B, a.K, h[0], h[1], h[2], h[3], h[4], h[5], h[6], h[7], h[8], h[9], h[10], h[11], h[12], h[13]);
+}
+
 template <int KDC, int NCHZ, int NCHH, bool OFFS, int CG, int EPI, int ORDER, int AC = 1>
-static qce_status launch_cfg(const TcArgs& a, cudaStream_t s) {
+static qce_status launch_cfg(TcArgs a, cudaStream_t s) {
     using Cfg = TcCfg<32 * KDC, 32 * NCHZ, 32 * NCHH, CG, ORDER, AC, tc_accb(EPI, 32 * KDC, 32 * NCHZ, 32 * NCHH, ORDER, AC)>;
     static PerDeviceOnce once;
     auto kern = dense_tc_kernel<KDC, NCHZ, NCHH, OFFS, CG, EPI, ORDER, AC>;
-    const int dev = current_device();
-    if (once.first(dev)) QCE_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
-    int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    if (once.first(current_device())) QCE_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
     const int64_t n_units = (a.B + CG * Cfg::NTILES * TILE_M - 1) / (CG * Cfg::NTILES * TILE_M);
-    const int64_t max_clusters = sms / CG;
+    const int64_t max_clusters = sm_count() / CG;
     const unsigned grid = (unsigned)((n_units < max_clusters ? n_units : max_clusters) * CG);
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = dim3(grid);
@@ -1681,8 +1716,10 @@ static qce_status launch_cfg(const TcArgs& a, cudaStream_t s) {
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
+    a.prof = tc_prof_counters(s);
     QCE_CUDA_TRY(cudaLaunchKernelEx(&cfg, kern, a));
     QCE_CHECK_LAUNCH("dense_tc_kernel");
+    if (a.prof) tc_prof_print(a, EPI, s);
     return QCE_OK;
 }
 
@@ -1747,100 +1784,121 @@ static void tc_fill_args(const qce_model* m, const TileScratch* ts, int64_t B, d
     a.tie_eps = (float)tc_tie_eps(m); a.inv_nobs = 1.f / (float)m->n_obs;
 }
 
-static qce_status tc_run_split(const qce_model* m, const TileScratch* ts, cudaStream_t s, int64_t B, int epi, int part, double* h_est,
-                               const void* h_true, int h_true_c64, double* acc, const int* unit_comp = nullptr, const int* perm = nullptr,
-                               const int* n_units_dev = nullptr, const void* bucket_img = nullptr, int* top_out = nullptr, const float* slot_w = nullptr, const int* run_flag = nullptr,
-                               int run_flag_want = 0) {
+// one split launch: epi 1 = the whitening columns (part 0), epi 2 = LMMSE row block `part`.  The caller fills `a` (tc_fill_args, then
+// the fields of its variant: regrouped units, pair weights, run flag, label output).
+static qce_status tc_launch_split(const qce_model* m, TcArgs a, int epi, int part, cudaStream_t s) {
     const TcParams& p = m->tc;
-    TcArgs a;
-    tc_fill_args(m, ts, B, h_est, h_true, h_true_c64, acc, &a);
-    a.slot_w = slot_w; a.run_flag = run_flag; a.run_flag_want = run_flag_want;
-    a.pair_acc = (float*)ts->tmp_est.p;
-    if (unit_comp) { a.unit_comp = unit_comp; a.perm = perm; a.n_units_dev = n_units_dev; a.a_img = (const __half*)bucket_img; }
-    a.top_out = top_out;
     a.image2 = (const unsigned char*)(epi == 1 ? p.image_z : p.image_h[part]);
     a.h_col0 = part * p.part_cols;
     a.count_rows = part == 0;
     const int cz = m->n_obs / 16, ch = p.part_cols / 32;
-    // QCE_TC_PROF (with a -DQCE_TC_PROFILE build): per-role cycle counters of CTA 0, printed per launch
-    static long long* prof = nullptr;
-    static const bool want_prof = getenv("QCE_TC_PROF") != nullptr;
-    if (want_prof && !prof) { cudaMalloc(&prof, 16 * sizeof(long long)); }
-    if (want_prof) { cudaMemsetAsync(prof, 0, 16 * sizeof(long long), s); a.prof = prof; }
-    qce_status st = QCE_ERR_UNSUPPORTED;
-    bool hit = false;
-#define QCE_TC_SPLIT_CASE(Z, H) if (!hit && cz == Z && ch == H) { st = launch_split<Z, H>(a, p.has_offsets, epi, p.split_a, s); hit = true; }
-    QCE_TC_SPLIT_CASE(16, 4) QCE_TC_SPLIT_CASE(8, 4) QCE_TC_SPLIT_CASE(6, 3)
-    QCE_TC_SPLIT_CASE(4, 4) QCE_TC_SPLIT_CASE(2, 2) QCE_TC_SPLIT_CASE(1, 1) QCE_TC_SPLIT_CASE(3, 3) QCE_TC_SPLIT_CASE(4, 2) QCE_TC_SPLIT_CASE(2, 1)
-#undef QCE_TC_SPLIT_CASE
-    if (!hit) {
-        set_error("tensor-core kernel: n_obs=%d n_ant=%d not instantiated", m->n_obs, m->n_ant);
-        return QCE_ERR_UNSUPPORTED;
-    }
-    if (want_prof && st == QCE_OK) {
-        long long h[16];
-        cudaMemcpyAsync(h, prof, sizeof(h), cudaMemcpyDeviceToHost, s);
-        cudaStreamSynchronize(s);
-        fprintf(stderr, "[qce tc prof] epi %d B=%lld K=%d | mma: total %lld wait_acc_empty %lld wait_full %lld wait_a %lld | epi t0: wait %lld z %lld h %lld | epi t1: wait %lld z %lld h %lld\n",
-                epi, (long long)B, a.K, h[0], h[1], h[2], h[3], h[4], h[5], h[6], h[8], h[9], h[10]);
-    }
-    return st;
+#define QCE_TC_SPLIT_LAUNCH(Z, H) if (cz == Z && ch == H) return launch_split<Z, H>(a, p.has_offsets, epi, p.split_a, s);
+    QCE_TC_SPLIT_SHAPES(QCE_TC_SPLIT_LAUNCH) QCE_TC_FUSED_SHAPES(QCE_TC_SPLIT_LAUNCH)
+#undef QCE_TC_SPLIT_LAUNCH
+    return tc_not_instantiated(m);
 }
 
-static qce_status tc_run(const qce_model* m, const TileScratch* ts, cudaStream_t s, int64_t B, double* h_est, const void* h_true, int h_true_c64,
-                         double* acc) {
+// the given-weights combination: every LMMSE row block
+static qce_status tc_combine_parts(const qce_model* m, const TcArgs& a, cudaStream_t s) {
+    for (int part = 0; part < m->tc.h_parts; ++part) {
+        const qce_status st = tc_launch_split(m, a, 2, part, s);
+        if (st) return st;
+    }
+    return QCE_OK;
+}
+
+// fused Z|H launch: epi 0 = 'all' (online softmax), epi 3 = hard top-1 (running argmax, SM-pair variant only)
+static qce_status tc_launch_fused(const qce_model* m, const TcArgs& a, int epi, cudaStream_t s) {
     const TcParams& p = m->tc;
-    TcArgs a;
-    tc_fill_args(m, ts, B, h_est, h_true, h_true_c64, acc, &a);
-    static long long* prof = nullptr;
-    static const bool want_prof = getenv("QCE_TC_PROF") != nullptr;
-    if (want_prof && !prof) cudaMallocManaged(&prof, 16 * sizeof(long long));
-    a.prof = want_prof ? prof : nullptr;
     const bool offs = p.has_offsets;
     const int cz = m->n_obs / 16, ch = m->n_ant / 16;
     // the SM-pair (cta_group::2) variant needs a lower-triangular whitening factor; any other runs on single CTAs (cta_group::1)
     const int cg = p.triangular ? 2 : 1;
-    qce_status st = QCE_ERR_UNSUPPORTED;
-    bool hit = false;
-#define QCE_TC_CASE(Z, H) if (cz == Z && ch == H) { st = launch_offs<Z, H>(a, offs, cg, p.split_a, s); hit = true; }
-    QCE_TC_CASE(4, 4) QCE_TC_CASE(2, 2) QCE_TC_CASE(1, 1) QCE_TC_CASE(3, 3) QCE_TC_CASE(4, 2) QCE_TC_CASE(2, 1)
-#undef QCE_TC_CASE
-    if (!hit) {
-        set_error("tensor-core kernel: n_obs=%d n_ant=%d not instantiated", m->n_obs, m->n_ant);
-        return QCE_ERR_UNSUPPORTED;
-    }
-    if (want_prof && st == QCE_OK) {
-        cudaStreamSynchronize(s);
-        fprintf(stderr, "[qce tc prof] B=%lld K=%d | mma: total %lld wait_acc_empty %lld wait_full %lld wait_a %lld | epi t0: wait %lld z %lld h %lld pro %lld | epi t1: wait %lld z %lld h %lld pro %lld | zld t0 %lld t1 %lld\n",
-                (long long)B, a.K, prof[0], prof[1], prof[2], prof[3], prof[4], prof[5], prof[6], prof[7], prof[8], prof[9], prof[10], prof[11], prof[12], prof[13]);
-    }
-    return st;
+#define QCE_TC_FUSED_LAUNCH(Z, H)                                                                                                      \
+    if (cz == Z && ch == H) return epi == 3 ? (offs ? launch_cfg<Z, Z, H, true, 2, 3, 0>(a, s) : launch_cfg<Z, Z, H, false, 2, 3, 0>(a, s)) \
+                                            : launch_offs<Z, H>(a, offs, cg, p.split_a, s);
+    QCE_TC_FUSED_SHAPES(QCE_TC_FUSED_LAUNCH)
+#undef QCE_TC_FUSED_LAUNCH
+    return tc_not_instantiated(m);
 }
 
-static qce_status tc_format_into(qce_model* m, cudaStream_t s, const double* r, int64_t B, TileScratch** out) {
-    if (!tc_instantiated(m) && !m->tc.split) { set_error("tensor-core kernel: n_obs=%d n_ant=%d not instantiated", m->n_obs, m->n_ant); return QCE_ERR_UNSUPPORTED; }
+// Formats B pilots into the stream's FP16 tile image: the complex128 values src.r, or (src.r null) the channels src.obs_h observed
+// (A = I) and quantised with src.qt on the fly.  The complex128 re-evaluation of flagged rows reads the pilots again from `src`.
+static qce_status tc_format_tiles(qce_model* m, cudaStream_t s, int64_t B, const RowSource& src, TileScratch** out) {
+    if (!tc_instantiated(m) && !m->tc.split) return tc_not_instantiated(m);
     TileScratch* ts = nullptr;
     qce_status st = tc_scratch(m, s, B, &ts);
     if (st) return st;
+    const bool observe = !src.r, split_a = m->tc.split_a;
     const int64_t tiles = (B + TILE_M - 1) / TILE_M;
-    QuantTables none{};
-    if (m->tc.split_a)
-        tc_format_kernel<false, false, true><<<(unsigned)(tiles * (TILE_M / 8)), 256, 2 * (size_t)(2 * m->n_obs / 8) * 128, s>>>(r, nullptr, 0.0, none, B, m->n_obs, 1.0 / m->tc.eff_scale,
-                                                                                            (__half*)ts->img.p, (unsigned char*)ts->bad.p, ts->fix_list());
-    else
-        tc_format_kernel<false, false, false><<<(unsigned)(tiles * (TILE_M / 8)), 256, (size_t)(2 * m->n_obs / 8) * 128, s>>>(r, nullptr, 0.0, none, B, m->n_obs, 1.0 / m->tc.eff_scale,
-                                                                                             (__half*)ts->img.p, (unsigned char*)ts->bad.p, ts->fix_list());
+    // [copies][kbs][8 rows][16 B] core matrices of a block, then the quantiser's thresholds and labels
+    const size_t smem = (size_t)(split_a ? 2 : 1) * (2 * m->n_obs / 8) * 128 +
+                        ((observe && src.qt.n_bits > 1) ? (size_t)(2 * src.qt.n_thr + 1) * sizeof(double) : 0);
+    auto kern = !observe        ? (split_a ? tc_format_kernel<false, false, true> : tc_format_kernel<false, false, false>)
+                : src.obs_h_c64 ? (split_a ? tc_format_kernel<true, true, true> : tc_format_kernel<true, true, false>)
+                                : (split_a ? tc_format_kernel<true, false, true> : tc_format_kernel<true, false, false>);
+    kern<<<(unsigned)(tiles * (TILE_M / 8)), 256, smem, s>>>(observe ? src.obs_h : src.r, (const double2*)src.obs_noise, src.obs_noise_scale,
+                                                             src.qt, B, m->n_obs, 1.0 / m->tc.eff_scale, (__half*)ts->img.p,
+                                                             (unsigned char*)ts->bad.p, ts->fix_list());
     QCE_CHECK_LAUNCH("tc_format_kernel");
     ts->owner = m; ts->rows = B;
-    ts->src = RowSource();
-    ts->src.r = r;
+    ts->src = src;
     *out = ts;
     return QCE_OK;
 }
 
 qce_status tc_format(qce_model* m, cudaStream_t s, const double* r, int64_t B) {
+    RowSource src;
+    src.r = r;
     TileScratch* ts = nullptr;
-    return tc_format_into(m, s, r, B, &ts);
+    return tc_format_tiles(m, s, B, src, &ts);
+}
+
+// Rows per chunk of the paths that keep [rows][K] scratch: whole work units, at most 2^27 / K rows (1 GiB + 0.5 GiB of
+// log-probabilities and weights) however large the batch is.  Each path clamps it to its batch.
+constexpr int64_t TC_UNIT_ROWS = 4 * TILE_M;
+static int64_t tc_chunk_rows(const qce_model* m) {
+    int64_t chunk = (((int64_t)1 << 27) / m->n_comp) / TC_UNIT_ROWS * TC_UNIT_ROWS;
+    if (const char* ce = getenv("QCE_TC_MODE_CHUNK")) chunk = atoll(ce) / TC_UNIT_ROWS * TC_UNIT_ROWS;      // test hook
+    return chunk < TC_UNIT_ROWS ? TC_UNIT_ROWS : chunk;
+}
+
+// the chunk of a formatted batch that starts at row b0 (a multiple of the tile size): a view of its pilot tiles, and its rows of the outputs
+struct TcChunk {
+    TileScratch v;
+    double* h_est;
+    double* logp;
+    const void* h_true;
+};
+
+static TcChunk tc_chunk(const qce_model* m, const TileScratch* ts, int64_t b0, double* h_est, double* logp, const void* h_true, int h_true_c64) {
+    TcChunk c{*ts, nullptr, nullptr, nullptr};
+    c.v.img.p = (unsigned char*)ts->img.p + (size_t)(b0 / TILE_M) * tc_tile_bytes(m);
+    c.v.bad.p = (unsigned char*)ts->bad.p + b0;
+    if (h_est) c.h_est = h_est + (size_t)b0 * m->n_ant * 2;
+    if (logp) c.logp = logp + (size_t)b0 * m->n_comp;
+    if (h_true) c.h_true = (const char*)h_true + (size_t)b0 * m->n_ant * (h_true_c64 ? 8 : 16);
+    return c;
+}
+
+// Near-tie re-selection of a chunk: exact log-probabilities of the pilots on its tie list (complex128), then their hard selection
+// again, overwriting their labels (`top`) and weight rows (`wts`)
+static qce_status tc_reselect_ties(const qce_model* m, const TileScratch* ts, cudaStream_t s, int64_t b0, int64_t nb, int mode, int n_top,
+                                   double rho, double* logp, float* wts, int* top, int* pair_cnt, float pair_thresh) {
+    RefineArgs ra;
+    ra.No = m->n_obs; ra.K = m->n_comp; ra.tri = m->tc.triangular ? 1 : 0;
+    ra.Linv = (const double2*)m->Linv; ra.zoff = (const double2*)m->zoff; ra.logc = m->logc;
+    ra.src = ts->src; ra.row0 = b0; ra.tie_buf = ts->tie_list(); ra.tie_total = ts->fix_list() + 1;
+    ra.lp2 = (float2*)ts->lp2.p; ra.logp_out = logp;
+    const int sms = sm_count();
+    tc_refine_kernel<<<(unsigned)(4 * sms), 256, (size_t)REFINE_RT * m->n_obs * sizeof(double2), s>>>(ra);
+    QCE_CHECK_LAUNCH("tc_refine_kernel");
+    const int K = m->n_comp;
+    auto sel = K <= 64 ? tc_select_kernel<2, true> : K <= 256 ? tc_select_kernel<8, true> : tc_select_kernel<32, true>;
+    sel<<<(unsigned)sms, 256, 0, s>>>((const float2*)ts->lp2.p, nb, K, mode, n_top, rho, m->flags, wts, nullptr, top, nullptr, nullptr, 0.0,
+                                      ts->tie_list(), nullptr, 0.0, pair_cnt, pair_thresh);
+    QCE_CHECK_LAUNCH("tc_select_kernel(list)");
+    return QCE_OK;
 }
 
 // pair mode: at most this many (pilot, component) pairs per pilot on average, else the dense weighted launch (a tuning constant)
@@ -1851,12 +1909,7 @@ static qce_status tc_run_modes(qce_model* m, TileScratch* ts, cudaStream_t s, in
                                double* logp_out, const void* h_true, int h_true_c64, double* acc) {
     if (m->n_comp > 1024) { set_error("tensor-core mode selection supports K <= 1024"); return QCE_ERR_UNSUPPORTED; }
     if (!m->tc.image_z) { set_error("tensor-core mode selection needs a lower-triangular whitening factor"); return QCE_ERR_UNSUPPORTED; }
-    // The log-probability / weight scratch is [rows][K]: walk the batch in chunks of whole work units so that it stays below
-    // 2^27 entries (1 GiB + 0.5 GiB) however large the batch is.
-    const int64_t unit_rows = 4 * TILE_M;
-    int64_t chunk = (((int64_t)1 << 27) / m->n_comp) / unit_rows * unit_rows;
-    if (const char* ce = getenv("QCE_TC_MODE_CHUNK")) chunk = atoll(ce) / unit_rows * unit_rows;      // test hook
-    if (chunk < unit_rows) chunk = unit_rows;
+    int64_t chunk = tc_chunk_rows(m);
     const bool want_est = h_est || acc;
     // Pair mode (top-n, cumulative rho, and 'all' on the large shapes): only the (pilot, component) pairs with a weight that matters
     // are combined, regrouped by component like the top-1 labels.  'all': weights <= 1e-9 are below half an ulp of the FP32
@@ -1869,7 +1922,7 @@ static qce_status tc_run_modes(qce_model* m, TileScratch* ts, cudaStream_t s, in
     const int pair_env = getenv("QCE_TC_PAIRS") ? atoi(getenv("QCE_TC_PAIRS")) : -1;
     const bool pair_on = pair_env < 0 ? m->tc.split : pair_env != 0;
     const bool pair_mode_ok = (mode == QCE_MODE_TOPN && n_top <= TC_PAIR_CAP) || mode == QCE_MODE_CUMPROB || (mode == QCE_MODE_ALL && m->tc.split);
-    const bool pairs = pair_on && want_est && pair_mode_ok && m->n_comp >= 8 && B >= 16 * unit_rows;
+    const bool pairs = pair_on && want_est && pair_mode_ok && m->n_comp >= 8 && B >= 16 * TC_UNIT_ROWS;
     // (a selected component whose renormalised weight is below 1e-9 -- the tail of a top-n / cumulative selection at a peaked posterior
     // -- is not a pair either: it cannot change the FP32 row the pairs are added into)
     const float pair_thresh = 1e-9f;
@@ -1877,8 +1930,7 @@ static qce_status tc_run_modes(qce_model* m, TileScratch* ts, cudaStream_t s, in
     if (chunk > B) chunk = B;
     qce_status st = tc_scratch_aux(ts, (size_t)chunk, (size_t)m->n_comp);
     if (st) return st;
-    const size_t tile_bytes = (size_t)TILE_M * 2 * m->n_obs * sizeof(__half) * (m->tc.split_a ? 2 : 1);
-    const size_t true_row = (size_t)m->n_ant * (h_true_c64 ? 8 : 16);
+    const size_t tile_bytes = tc_tile_bytes(m);
     // top-1: regroup the pilots by selected component and run ONE component per work unit (QCE_TC_BUCKET=0: weighted launch instead)
     const int tiles_per_unit = 2 * (((m->tc.split_a && 2 * m->n_obs > 128) || 2 * m->n_obs > 256) ? 1 : TILES);      // CG * Cfg::NTILES of the split launches
     const int bucket_rows = tiles_per_unit * TILE_M;
@@ -1907,19 +1959,23 @@ static qce_status tc_run_modes(qce_model* m, TileScratch* ts, cudaStream_t s, in
     }
     for (int64_t b0 = 0; b0 < B; b0 += chunk) {
         const int64_t nb = (B - b0) < chunk ? (B - b0) : chunk;
-        TileScratch v = *ts;                                   // view of this chunk's tiles (b0 is a multiple of the tile size)
-        v.img.p = (unsigned char*)ts->img.p + (size_t)(b0 / TILE_M) * tile_bytes;
-        v.bad.p = (unsigned char*)ts->bad.p + b0;
-        double* he = h_est ? h_est + (size_t)b0 * m->n_ant * 2 : nullptr;
-        double* lo = logp_out ? logp_out + (size_t)b0 * m->n_comp : nullptr;
-        const void* ht = h_true ? (const void*)((const char*)h_true + (size_t)b0 * true_row) : nullptr;
+        const TcChunk c = tc_chunk(m, ts, b0, h_est, logp_out, h_true, h_true_c64);
+        // arguments of a split launch over `rows` pilot rows of this chunk (or of its regrouped tiles)
+        auto args = [&](int64_t rows, double* he, const void* ht, int ht_c64, double* ac) {
+            TcArgs a;
+            tc_fill_args(m, &c.v, rows, he, ht, ht_c64, ac, &a);
+            a.pair_acc = (float*)ts->tmp_est.p;
+            return a;
+        };
         // top-1 without log-probability export: the whitening launch keeps the running argmax itself (no [rows][K] export, no selection launch)
         const bool label_in_kernel = bucketed && !logp_out;
         // hard selections: pilots whose selection is too close to call go on the chunk's tie list (QCE_TC_TIE_EPS=0: nobody does)
         const double eps = tc_tie_eps(m);
         const bool refine = want_est && mode != QCE_MODE_ALL && eps > 0.0 && (ts->src.r || ts->src.obs_h);
         QCE_CUDA_TRY(cudaMemsetAsync(ts->tie_list(), 0, sizeof(int), s));
-        st = tc_run_split(m, &v, s, nb, 1, 0, nullptr, nullptr, 0, nullptr, nullptr, nullptr, nullptr, nullptr, label_in_kernel ? b_top : nullptr);
+        TcArgs wa = args(nb, nullptr, nullptr, 0, nullptr);
+        wa.top_out = label_in_kernel ? b_top : nullptr;
+        st = tc_launch_split(m, wa, 1, 0, s);
         if (st) return st;
         if (bucketed) {
             QCE_CUDA_TRY(cudaMemsetAsync(b_cnt, 0, m->n_comp * sizeof(int), s));
@@ -1928,89 +1984,68 @@ static qce_status tc_run_modes(qce_model* m, TileScratch* ts, cudaStream_t s, in
         const bool pair_chunk = pairs && !bucketed;
         const bool fused_count = pair_chunk && m->n_comp <= 256;      // the thread-per-pilot selection counts the pairs itself
         if (pair_chunk) QCE_CUDA_TRY(cudaMemsetAsync(p_cnt, 0, m->n_comp * sizeof(int), s));
+        const unsigned char* vb = (const unsigned char*)c.v.bad.p;
         if (!label_in_kernel) {
-            float* wts = (want_est && !bucketed) ? (float*)v.wts.p : nullptr;
-            const unsigned char* vb = (const unsigned char*)v.bad.p;
+            float* wts = (want_est && !bucketed) ? (float*)c.v.wts.p : nullptr;
             const int K = m->n_comp;
             if (K <= 256) {
                 const size_t sm = (size_t)2 * K * (SEL_ROWS + 1) * sizeof(float) + (size_t)K * sizeof(int);
                 static PerDeviceOnce once;
                 if (once.first(current_device()))
                     QCE_CUDA_TRY(cudaFuncSetAttribute(tc_select_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-                tc_select_rows_kernel<<<(unsigned)((nb + SEL_ROWS - 1) / SEL_ROWS), SEL_THREADS, sm, s>>>((const float2*)v.lp2.p, nb, K, mode, n_top, rho, m->flags,
-                    wts, lo, b_top, vb, ts->tie_list(), eps, m->logc, 1.0 / m->n_obs, fused_count ? p_cnt : nullptr, pair_thresh);
+                tc_select_rows_kernel<<<(unsigned)((nb + SEL_ROWS - 1) / SEL_ROWS), SEL_THREADS, sm, s>>>((const float2*)c.v.lp2.p, nb, K, mode, n_top, rho, m->flags,
+                    wts, c.logp, b_top, vb, ts->tie_list(), eps, m->logc, 1.0 / m->n_obs, fused_count ? p_cnt : nullptr, pair_thresh);
             } else {
-                tc_select_kernel<32><<<(unsigned)((nb + 7) / 8), 256, 0, s>>>((const float2*)v.lp2.p, nb, K, mode, n_top, rho, m->flags, wts, lo, b_top, vb, ts->tie_list(), eps, nullptr, m->logc, 1.0 / m->n_obs);
+                tc_select_kernel<32><<<(unsigned)((nb + 7) / 8), 256, 0, s>>>((const float2*)c.v.lp2.p, nb, K, mode, n_top, rho, m->flags, wts, c.logp, b_top, vb, ts->tie_list(), eps, nullptr, m->logc, 1.0 / m->n_obs);
             }
             QCE_CHECK_LAUNCH("tc_select kernel");
         }
         if (!want_est) continue;
-        if (refine) {      // exact log-probabilities for the pilots on the tie list, then their selection again (weight rows / labels overwritten)
-            RefineArgs ra;
-            ra.No = m->n_obs; ra.K = m->n_comp; ra.tri = m->tc.triangular ? 1 : 0;
-            ra.Linv = (const double2*)m->Linv; ra.zoff = (const double2*)m->zoff; ra.logc = m->logc;
-            ra.src = ts->src; ra.row0 = b0; ra.tie_buf = ts->tie_list(); ra.tie_total = ts->fix_list() + 1;
-            ra.lp2 = (float2*)v.lp2.p; ra.logp_out = lo;
-            int sms = 148;
-            cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, current_device());
-            const size_t rsm = (size_t)REFINE_RT * m->n_obs * sizeof(double2);
-            tc_refine_kernel<<<(unsigned)(4 * sms), 256, rsm, s>>>(ra);
-            QCE_CHECK_LAUNCH("tc_refine_kernel");
-            float* wts = bucketed ? nullptr : (float*)v.wts.p;
-            const unsigned sgrid = (unsigned)sms;
-            int* pc = fused_count ? p_cnt : nullptr;
-            if (m->n_comp <= 64) tc_select_kernel<2, true><<<sgrid, 256, 0, s>>>((const float2*)v.lp2.p, nb, m->n_comp, mode, n_top, rho, m->flags, wts, nullptr, b_top, nullptr, nullptr, 0.0, ts->tie_list(), nullptr, 0.0, pc, pair_thresh);
-            else if (m->n_comp <= 256) tc_select_kernel<8, true><<<sgrid, 256, 0, s>>>((const float2*)v.lp2.p, nb, m->n_comp, mode, n_top, rho, m->flags, wts, nullptr, b_top, nullptr, nullptr, 0.0, ts->tie_list(), nullptr, 0.0, pc, pair_thresh);
-            else tc_select_kernel<32, true><<<sgrid, 256, 0, s>>>((const float2*)v.lp2.p, nb, m->n_comp, mode, n_top, rho, m->flags, wts, nullptr, b_top, nullptr, nullptr, 0.0, ts->tie_list(), nullptr, 0.0, pc, pair_thresh);
-            QCE_CHECK_LAUNCH("tc_select_kernel(list)");
+        if (refine) {      // (weight rows / labels overwritten)
+            st = tc_reselect_ties(m, ts, s, b0, nb, mode, n_top, rho, c.logp, bucketed ? nullptr : (float*)c.v.wts.p, b_top,
+                                  fused_count ? p_cnt : nullptr, pair_thresh);
+            if (st) return st;
         }
         if (bucketed) {
             tc_bucket_count_kernel<<<(unsigned)((nb + 1023) / 1024), 1024, 0, s>>>(b_top, nb, m->n_comp, b_cnt);
             tc_bucket_scan_kernel<<<1, 1024, 0, s>>>(b_cnt, m->n_comp, bucket_rows, b_off, b_cur, b_ucomp, b_nu);
             tc_bucket_place_kernel<<<(unsigned)((nb + 1023) / 1024), 1024, 0, s>>>(b_top, nb, m->n_comp, b_off, b_cur, b_perm);
-            tc_bucket_gather_kernel<<<(unsigned)(cap_rows / TILE_M), 256, 0, s>>>((const unsigned char*)v.img.p, b_perm, b_nu, tiles_per_unit,
+            tc_bucket_gather_kernel<<<(unsigned)(cap_rows / TILE_M), 256, 0, s>>>((const unsigned char*)c.v.img.p, b_perm, b_nu, tiles_per_unit,
                                                                                   2 * m->n_obs / 8, m->tc.split_a ? 2 : 1, (unsigned char*)ts->img2.p);
             QCE_CHECK_LAUNCH("tc_bucket kernels");
-            for (int part = 0; part < m->tc.h_parts; ++part) {
-                st = tc_run_split(m, &v, s, cap_rows, 2, part, he, ht, h_true_c64, acc, b_ucomp, b_perm, b_nu, ts->img2.p);
-                if (st) return st;
-            }
+            TcArgs ba = args(cap_rows, c.h_est, c.h_true, h_true_c64, acc);
+            ba.unit_comp = b_ucomp; ba.perm = b_perm; ba.n_units_dev = b_nu; ba.a_img = (const __half*)ts->img2.p;
+            st = tc_combine_parts(m, ba, s);
+            if (st) return st;
             continue;
         }
-        if (pairs && !bucketed) {
+        if (pair_chunk) {
             const unsigned g1 = (unsigned)((nb + 1023) / 1024);
-            const unsigned char* vb = (const unsigned char*)v.bad.p;
             QCE_CUDA_TRY(cudaMemsetAsync(p_perm, 0xFF, (size_t)p_rows * sizeof(int), s));          // -1 = padding slot
             QCE_CUDA_TRY(cudaMemsetAsync(ts->tmp_est.p, 0, (size_t)nb * m->n_ant * 8, s));           // the pair rows are added into zeros
-            if (!fused_count) tc_pair_count_kernel<<<g1, 1024, 0, s>>>((const float*)v.wts.p, vb, nb, m->n_comp, pair_thresh, p_cnt);
+            if (!fused_count) tc_pair_count_kernel<<<g1, 1024, 0, s>>>((const float*)c.v.wts.p, vb, nb, m->n_comp, pair_thresh, p_cnt);
             tc_pair_scan_kernel<<<1, 1024, 0, s>>>(p_cnt, m->n_comp, bucket_rows, (int)(p_units - 1), p_off, p_cur, p_ucomp, p_nu, p_dense);
-            tc_pair_place_kernel<<<g1, 1024, 0, s>>>((const float*)v.wts.p, vb, nb, m->n_comp, pair_thresh, p_off, p_cur, p_dense, p_perm, p_w);
-            tc_bucket_gather_kernel<<<(unsigned)(p_rows / TILE_M), 256, 0, s>>>((const unsigned char*)v.img.p, p_perm, p_nu, tiles_per_unit,
+            tc_pair_place_kernel<<<g1, 1024, 0, s>>>((const float*)c.v.wts.p, vb, nb, m->n_comp, pair_thresh, p_off, p_cur, p_dense, p_perm, p_w);
+            tc_bucket_gather_kernel<<<(unsigned)(p_rows / TILE_M), 256, 0, s>>>((const unsigned char*)c.v.img.p, p_perm, p_nu, tiles_per_unit,
                                                                                 2 * m->n_obs / 8, m->tc.split_a ? 2 : 1, (unsigned char*)ts->img2.p);
             QCE_CHECK_LAUNCH("tc_pair kernels");
             count_launch(fused_count ? 2 : 3);
-            for (int part = 0; part < m->tc.h_parts; ++part) {
-                st = tc_run_split(m, &v, s, p_rows, 2, part, nullptr, nullptr, 0, nullptr, p_ucomp, p_perm, p_nu, ts->img2.p, nullptr, p_w);
-                if (st) return st;
-            }
-            {
-                int sms = 148;
-                cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, current_device());
-                tc_pair_finish_kernel<<<(unsigned)(8 * sms), 256, 0, s>>>((const float2*)ts->tmp_est.p, (double2*)he, ht, h_true_c64, vb, nb, m->n_ant,
-                                                                          p_dense, acc);
-                QCE_CHECK_LAUNCH("tc_pair_finish_kernel");
-            }
+            TcArgs pa = args(p_rows, nullptr, nullptr, 0, nullptr);
+            pa.unit_comp = p_ucomp; pa.perm = p_perm; pa.n_units_dev = p_nu; pa.a_img = (const __half*)ts->img2.p; pa.slot_w = p_w;
+            st = tc_combine_parts(m, pa, s);
+            if (st) return st;
+            tc_pair_finish_kernel<<<(unsigned)(8 * sm_count()), 256, 0, s>>>((const float2*)ts->tmp_est.p, (double2*)c.h_est, c.h_true, h_true_c64, vb, nb,
+                                                                             m->n_ant, p_dense, acc);
+            QCE_CHECK_LAUNCH("tc_pair_finish_kernel");
             // ... or, when the pairs were too many, the weighted launch over all K components (returns at once otherwise)
-            for (int part = 0; part < m->tc.h_parts; ++part) {
-                st = tc_run_split(m, &v, s, nb, 2, part, he, ht, h_true_c64, acc, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, p_dense, 1);
-                if (st) return st;
-            }
+            TcArgs da = args(nb, c.h_est, c.h_true, h_true_c64, acc);
+            da.run_flag = p_dense; da.run_flag_want = 1;
+            st = tc_combine_parts(m, da, s);
+            if (st) return st;
             continue;
         }
-        for (int part = 0; part < m->tc.h_parts; ++part) {
-            st = tc_run_split(m, &v, s, nb, 2, part, he, ht, h_true_c64, acc);
-            if (st) return st;
-        }
+        st = tc_combine_parts(m, args(nb, c.h_est, c.h_true, h_true_c64, acc), s);
+        if (st) return st;
     }
     return QCE_OK;
 }
@@ -2103,11 +2138,8 @@ static bool tc_hard_top1_ok(const qce_model* m) {
 static qce_status tc_run_hard_top1(qce_model* m, TileScratch* ts, cudaStream_t s, int64_t B, double* h_est, const void* h_true, int h_true_c64,
                                    double* acc) {
     const int K = m->n_comp;
-    const int64_t unit_rows = 4 * TILE_M;
-    int64_t chunk = (((int64_t)1 << 27) / K) / unit_rows * unit_rows;
-    if (const char* ce = getenv("QCE_TC_MODE_CHUNK")) chunk = atoll(ce) / unit_rows * unit_rows;      // test hook
-    if (chunk < unit_rows) chunk = unit_rows;
-    if (chunk > B) chunk = (B + unit_rows - 1) / unit_rows * unit_rows;
+    int64_t chunk = tc_chunk_rows(m);
+    if (chunk > B) chunk = (B + TC_UNIT_ROWS - 1) / TC_UNIT_ROWS * TC_UNIT_ROWS;
     const double eps = tc_tie_eps(m);
     const bool refine = eps > 0.0 && (ts->src.r || ts->src.obs_h);
     qce_status st = QCE_OK;
@@ -2117,53 +2149,48 @@ static qce_status tc_run_hard_top1(qce_model* m, TileScratch* ts, cudaStream_t s
         st = grow(ts->bidx, (size_t)chunk * sizeof(int));                        // exact labels of the listed pilots
         if (st) return st;
     }
-    const size_t tile_bytes = (size_t)TILE_M * 2 * m->n_obs * sizeof(__half);
-    const size_t true_row = (size_t)m->n_ant * (h_true_c64 ? 8 : 16);
-    const int cz = m->n_obs / 16, ch = m->n_ant / 16;
-    int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, current_device());
+    const int sms = sm_count();
     for (int64_t b0 = 0; b0 < B; b0 += chunk) {
         const int64_t nb = (B - b0) < chunk ? (B - b0) : chunk;
-        TileScratch v = *ts;
-        v.img.p = (unsigned char*)ts->img.p + (size_t)(b0 / TILE_M) * tile_bytes;
-        v.bad.p = (unsigned char*)ts->bad.p + b0;
-        double* he = h_est ? h_est + (size_t)b0 * m->n_ant * 2 : nullptr;
-        const void* ht = h_true ? (const void*)((const char*)h_true + (size_t)b0 * true_row) : nullptr;
+        const TcChunk c = tc_chunk(m, ts, b0, h_est, nullptr, h_true, h_true_c64);
         TcArgs a;
-        tc_fill_args(m, &v, nb, he, ht, h_true_c64, acc, &a);
+        tc_fill_args(m, &c.v, nb, c.h_est, c.h_true, h_true_c64, acc, &a);
         if (refine) QCE_CUDA_TRY(cudaMemsetAsync(ts->tie_list(), 0, sizeof(int), s));
         else a.tie_buf = nullptr;                                              // nobody is handed to the exact path: every pilot is answered here
-        const bool offs = m->tc.has_offsets;
-        bool hit = false;
-#define QCE_TC_HARD_CASE(Z, H) if (!hit && cz == Z && ch == H) { st = offs ? launch_cfg<Z, Z, H, true, 2, 3, 0>(a, s) : launch_cfg<Z, Z, H, false, 2, 3, 0>(a, s); hit = true; }
-        QCE_TC_HARD_CASE(4, 4) QCE_TC_HARD_CASE(2, 2) QCE_TC_HARD_CASE(1, 1) QCE_TC_HARD_CASE(3, 3) QCE_TC_HARD_CASE(4, 2) QCE_TC_HARD_CASE(2, 1)
-#undef QCE_TC_HARD_CASE
-        if (!hit) { set_error("tensor-core kernel: n_obs=%d n_ant=%d not instantiated", m->n_obs, m->n_ant); return QCE_ERR_UNSUPPORTED; }
+        st = tc_launch_fused(m, a, 3, s);
         if (st) return st;
         if (!refine) continue;
-        RefineArgs ra;
-        ra.No = m->n_obs; ra.K = K; ra.tri = 1;
-        ra.Linv = (const double2*)m->Linv; ra.zoff = (const double2*)m->zoff; ra.logc = m->logc;
-        ra.src = ts->src; ra.row0 = b0; ra.tie_buf = ts->tie_list(); ra.tie_total = ts->fix_list() + 1;
-        ra.lp2 = (float2*)ts->lp2.p; ra.logp_out = nullptr;
-        tc_refine_kernel<<<(unsigned)(4 * sms), 256, (size_t)REFINE_RT * m->n_obs * sizeof(double2), s>>>(ra);
-        QCE_CHECK_LAUNCH("tc_refine_kernel");
         int* top = (int*)ts->bidx.p;
-        const unsigned sgrid = (unsigned)sms;
-        if (K <= 64) tc_select_kernel<2, true><<<sgrid, 256, 0, s>>>((const float2*)ts->lp2.p, nb, K, QCE_MODE_TOP1, 1, 0.0, m->flags, nullptr, nullptr, top, nullptr, nullptr, 0.0, ts->tie_list(), nullptr, 0.0, nullptr, 0.f);
-        else if (K <= 256) tc_select_kernel<8, true><<<sgrid, 256, 0, s>>>((const float2*)ts->lp2.p, nb, K, QCE_MODE_TOP1, 1, 0.0, m->flags, nullptr, nullptr, top, nullptr, nullptr, 0.0, ts->tie_list(), nullptr, 0.0, nullptr, 0.f);
-        else tc_select_kernel<32, true><<<sgrid, 256, 0, s>>>((const float2*)ts->lp2.p, nb, K, QCE_MODE_TOP1, 1, 0.0, m->flags, nullptr, nullptr, top, nullptr, nullptr, 0.0, ts->tie_list(), nullptr, 0.0, nullptr, 0.f);
-        QCE_CHECK_LAUNCH("tc_select_kernel(list)");
+        st = tc_reselect_ties(m, ts, s, b0, nb, QCE_MODE_TOP1, 1, 0.0, nullptr, nullptr, top, nullptr, 0.f);
+        if (st) return st;
         Top1RowsArgs ta;
         ta.No = m->n_obs; ta.N = m->n_ant; ta.K = K;
         ta.W = (const double2*)m->W; ta.hoff = (const double2*)m->hoff;
         ta.src = ts->src; ta.row0 = b0; ta.tie_buf = ts->tie_list(); ta.top = top;
-        ta.h_est = (double2*)he; ta.h_true = ht; ta.h_true_c64 = h_true_c64; ta.acc = acc;
+        ta.h_est = (double2*)c.h_est; ta.h_true = c.h_true; ta.h_true_c64 = h_true_c64; ta.acc = acc;
         tc_top1_rows_kernel<<<(unsigned)sms, 256, (size_t)8 * m->n_obs * sizeof(double2), s>>>(ta);
         QCE_CHECK_LAUNCH("tc_top1_rows_kernel");
         count_launch(3);
     }
     return QCE_OK;
+}
+
+// One estimate of a formatted batch: the fused 'all' launch where the shape has one and nothing is exported, the fused hard top-1
+// where tc_hard_top1_ok picks it, the log-probability -> weights -> combination path otherwise; then the complex128 rows.
+static qce_status tc_estimate(qce_model* m, TileScratch* ts, cudaStream_t s, int64_t B, int mode, int n_top, double rho, double* h_est,
+                              double* logp_out, const void* h_true, int h_true_c64, double* acc) {
+    qce_status st;
+    if (mode == QCE_MODE_ALL && !logp_out && !m->tc.split) {
+        TcArgs a;
+        tc_fill_args(m, ts, B, h_est, h_true, h_true_c64, acc, &a);
+        st = tc_launch_fused(m, a, 0, s);
+    } else if (mode == QCE_MODE_TOP1 && !logp_out && (h_est || acc) && tc_hard_top1_ok(m)) {
+        st = tc_run_hard_top1(m, ts, s, B, h_est, h_true, h_true_c64, acc);
+    } else {
+        st = tc_run_modes(m, ts, s, B, mode, n_top, rho, h_est, logp_out, h_true, h_true_c64, acc);
+    }
+    if (st) return st;
+    return tc_fix_rows(m, ts, s, B, mode, n_top, rho, h_est, logp_out, h_true, h_true_c64, acc);
 }
 
 qce_status tc_estimate_formatted(qce_model* m, cudaStream_t s, int64_t B, double* h_est, const void* h_true, int h_true_c64, double* acc) {
@@ -2174,24 +2201,19 @@ qce_status tc_estimate_formatted(qce_model* m, cudaStream_t s, int64_t B, double
         return QCE_ERR_INVALID;
     }
     if (B == 0) return QCE_OK;
-    qce_status st = m->tc.split ? tc_run_modes(m, ts, s, B, QCE_MODE_ALL, 0, 0.0, h_est, nullptr, h_true, h_true_c64, acc)
-                                : tc_run(m, ts, s, B, h_est, h_true, h_true_c64, acc);
-    if (st) return st;
-    return tc_fix_rows(m, ts, s, B, QCE_MODE_ALL, 0, 0.0, h_est, nullptr, h_true, h_true_c64, acc);
+    return tc_estimate(m, ts, s, B, QCE_MODE_ALL, 0, 0.0, h_est, nullptr, h_true, h_true_c64, acc);
 }
 
 // pilots given as complex128 values (estimate_from_y): format, then estimate
 qce_status launch_dense_tc(qce_model* m, cudaStream_t s, const double* r, int64_t B, int mode, int n_top, double rho,
                            double* h_est, double* logp_out, const void* h_true, int h_true_c64, double* acc) {
     if (B == 0) return QCE_OK;
+    RowSource src;
+    src.r = r;
     TileScratch* ts = nullptr;
-    qce_status st = tc_format_into(m, s, r, B, &ts);
+    qce_status st = tc_format_tiles(m, s, B, src, &ts);
     if (st) return st;
-    if (mode == QCE_MODE_ALL && !logp_out && !m->tc.split) st = tc_run(m, ts, s, B, h_est, h_true, h_true_c64, acc);
-    else if (mode == QCE_MODE_TOP1 && !logp_out && (h_est || acc) && tc_hard_top1_ok(m)) st = tc_run_hard_top1(m, ts, s, B, h_est, h_true, h_true_c64, acc);
-    else st = tc_run_modes(m, ts, s, B, mode, n_top, rho, h_est, logp_out, h_true, h_true_c64, acc);
-    if (st) return st;
-    return tc_fix_rows(m, ts, s, B, mode, n_top, rho, h_est, logp_out, h_true, h_true_c64, acc);
+    return tc_estimate(m, ts, s, B, mode, n_top, rho, h_est, logp_out, h_true, h_true_c64, acc);
 }
 
 // fused Monte-Carlo step: observe (A = I) -> quantise -> estimate -> NMSE accumulators; the quantised pilots never exist in HBM
@@ -2199,29 +2221,12 @@ qce_status launch_dense_tc(qce_model* m, cudaStream_t s, const double* r, int64_
 qce_status launch_pipeline_tc(qce_model* m, const QuantTables* qt, cudaStream_t s, const void* h, int h_is_c64, const double* noise,
                               double noise_scale, int64_t B, int mode, int n_top, double rho, double* h_est, double* acc) {
     if (B == 0) return QCE_OK;
-    if (!tc_instantiated(m) && !m->tc.split) { set_error("tensor-core pipeline: shape not supported"); return QCE_ERR_UNSUPPORTED; }
+    RowSource src;
+    src.obs_h = h; src.obs_noise = noise; src.obs_noise_scale = noise_scale; src.obs_h_c64 = h_is_c64; src.qt = *qt;
     TileScratch* ts = nullptr;
-    qce_status st = tc_scratch(m, s, B, &ts);
+    qce_status st = tc_format_tiles(m, s, B, src, &ts);
     if (st) return st;
-    RowSource obs_src;          // where the complex128 re-evaluation of flagged rows finds the pilots: it observes + quantises them again
-    obs_src.obs_h = h; obs_src.obs_noise = noise; obs_src.obs_noise_scale = noise_scale; obs_src.obs_h_c64 = h_is_c64; obs_src.qt = *qt;
-    const int64_t tiles = (B + TILE_M - 1) / TILE_M;
-    const size_t smem = (size_t)(m->tc.split_a ? 2 : 1) * (2 * m->n_obs / 8) * 128 + ((qt->n_bits > 1) ? (size_t)(2 * qt->n_thr + 1) * sizeof(double) : 0);
-    const unsigned grid = (unsigned)(tiles * (TILE_M / 8));
-    const double inv_scale = 1.0 / m->tc.eff_scale;
-#define QCE_FMT(C64, SPL) tc_format_kernel<true, C64, SPL><<<grid, 256, smem, s>>>(h, (const double2*)noise, noise_scale, *qt, B, m->n_obs, inv_scale, \
-                                                                                 (__half*)ts->img.p, (unsigned char*)ts->bad.p, ts->fix_list())
-    if (h_is_c64) { if (m->tc.split_a) QCE_FMT(true, true); else QCE_FMT(true, false); }
-    else { if (m->tc.split_a) QCE_FMT(false, true); else QCE_FMT(false, false); }
-#undef QCE_FMT
-    QCE_CHECK_LAUNCH("tc_format_kernel(observe)");
-    ts->owner = m; ts->rows = B;
-    ts->src = obs_src;
-    if (mode == QCE_MODE_ALL && !m->tc.split) st = tc_run(m, ts, s, B, h_est, h, h_is_c64, acc);
-    else if (mode == QCE_MODE_TOP1 && (h_est || acc) && tc_hard_top1_ok(m)) st = tc_run_hard_top1(m, ts, s, B, h_est, h, h_is_c64, acc);
-    else st = tc_run_modes(m, ts, s, B, mode, n_top, rho, h_est, nullptr, h, h_is_c64, acc);
-    if (st) return st;
-    return tc_fix_rows(m, ts, s, B, mode, n_top, rho, h_est, nullptr, h, h_is_c64, acc);
+    return tc_estimate(m, ts, s, B, mode, n_top, rho, h_est, nullptr, h, h_is_c64, acc);
 }
 
 }  // namespace qce

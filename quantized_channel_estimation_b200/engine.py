@@ -28,8 +28,8 @@ def parse_mode(n_summands_or_proba):
 
 
 def tc_shape_ok(n_obs, n_ant, on_grid=False):
-    """Shapes the tensor-core kernels are instantiated for (mirrors tc_instantiated / tc_split_shape / tc_supported in
-    qce_dense_tc.cu).  ``on_grid``: the pilots lie on an integer grid (``data_scale > 0``: 1 bit, or uniform b bit).  n_obs = 256
+    """Shapes the tensor-core kernels are instantiated for (mirrors QCE_TC_FUSED_SHAPES / QCE_TC_SPLIT_SHAPES and tc_supported
+    in qce_dense_tc.cu).  ``on_grid``: the pilots lie on an integer grid (``data_scale > 0``: 1 bit, or uniform b bit).  n_obs = 256
     (one pilot per antenna on 256 antennas, or two pilots on 128) takes only such pilots; off the grid it runs on the complex128
     kernel."""
     if n_obs % 16 or n_ant % 16:
