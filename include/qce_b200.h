@@ -146,8 +146,12 @@ qce_status qce_pipeline(qce_model* m, const qce_quantizer* q, void* stream, cons
 /* Two-step form of the tensor-core path (QCE_PREC_TC, QCE_MODE_ALL).  qce_format_pilots converts r (c128 [B][n_obs],
  * values on the quantiser grid declared by data_scale) into the FP16 tile image the estimate kernel stages with bulk
  * copies, and keeps it in the library's per-stream scratch.  qce_estimate_formatted then runs the estimate kernel alone on the
- * first B pilots of that image (same model, same stream); outputs as in qce_estimate.  bench.py uses the pair to time the dominant kernel in
- * isolation; qce_estimate with QCE_PREC_TC is exactly format + estimate. */
+ * first B pilots of that image (same model, same stream); outputs as in qce_estimate, B rows of each.  bench.py uses the pair to time the
+ * dominant kernel in isolation; qce_estimate with QCE_PREC_TC is exactly format + estimate.
+ * Lifetime of r_dev: pilots the formatter cannot represent (off the grid, NaN) are re-read from r_dev in complex128 by every
+ * qce_estimate_formatted call on the image, so r_dev must stay valid and unchanged until the work of the last such call has completed
+ * on the stream (or until the next qce_format_pilots / tensor-core call on it replaces the image).  Such rows at or past B are left
+ * alone by a call on B pilots; qce_last_fix_count still counts every listed row of the image. */
 qce_status qce_format_pilots(qce_model* m, void* stream, const void* r_dev, int64_t B);
 qce_status qce_estimate_formatted(qce_model* m, void* stream, int64_t B, void* h_est_dev, const void* h_true_dev,
                                   double* acc_dev);

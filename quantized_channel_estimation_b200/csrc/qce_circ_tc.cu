@@ -636,11 +636,14 @@ qce_status launch_circ_tc(const qce_circ_model* m, cudaStream_t s, const double*
     }
     // hard selections: pilots whose selection the FP32 log-likelihoods (~1.4e-5 nats rms, profiles/r02_flip_rate.json) cannot
     // decide go on a fix list and are answered by the complex128 kernel.  QCE_TC_TIE_EPS overrides the gap (0: no re-evaluation).
+    // 'all' lists nothing, but its list is still reset: qce_last_fix_count reports this call's 0, not an earlier call's count
     a.fix_buf = nullptr;
     a.tie_eps = getenv("QCE_TC_TIE_EPS") ? atof(getenv("QCE_TC_TIE_EPS")) : 5e-4;
-    if (mode != QCE_MODE_ALL) {
-        qce_status st = circ_fix_list(s, B, &a.fix_buf);
+    {
+        int* list = nullptr;
+        qce_status st = circ_fix_list(s, mode == QCE_MODE_ALL ? 0 : B, &list);
         if (st) return st;
+        if (mode != QCE_MODE_ALL) a.fix_buf = list;
     }
     const qce_status st = m->n_comp == 64 ? launch_circ_tc_k<1>(a, s) : launch_circ_tc_k<2>(a, s);
     if (st || mode == QCE_MODE_ALL || !(h_est || acc)) return st;

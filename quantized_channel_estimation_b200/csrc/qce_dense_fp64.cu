@@ -29,7 +29,8 @@ struct Fp64Args {
     double* acc;
     int mode, n_top, flags;
     double rho;
-    // re-evaluation of listed rows (null: the rows are 0 .. B-1 in order): tile entry i is row rows[i], i < *n_rows_dev
+    // re-evaluation of listed rows (null: the rows are 0 .. B-1 in order): tile entry i is row rows[i], i < *n_rows_dev.  A listed
+    // row >= B (the list of a formatted image longer than the batch, qce_estimate_formatted) is skipped: not staged, written or counted
     const int* rows;
     const int* n_rows_dev;
     // r == null: the pilots are observed + quantised on the fly (A = I), bit-exact to quantize_kernel
@@ -58,6 +59,7 @@ __global__ void __launch_bounds__(256) dense_fp64_kernel(Fp64Args a) {
     double* part = lp + (size_t)TS * a.K;                                      // [8][TS]
     __shared__ double red[3];
     __shared__ int64_t s_row[TS];       // batch row of every tile entry
+    __shared__ bool s_ok[TS];           // the entry is a row of the batch (< B)
 
     const int t = threadIdx.x;
     const int sp = t % SP, rg = t / SP;
@@ -66,15 +68,21 @@ __global__ void __launch_bounds__(256) dense_fp64_kernel(Fp64Args a) {
     const int64_t n_rows = a.n_rows_dev ? (int64_t)__ldg(a.n_rows_dev) : a.B;
     for (int64_t base = (int64_t)blockIdx.x * TS; base < n_rows; base += (int64_t)gridDim.x * TS) {
     const int nvalid = (int)((n_rows - base) < TS ? (n_rows - base) : TS);
-    if (t < TS) s_row[t] = (t < nvalid) ? (a.rows ? (int64_t)a.rows[base + t] : base + t) : 0;
+    bool ok = false;
+    if (t < TS) {
+        const int64_t row = (t < nvalid) ? (a.rows ? (int64_t)a.rows[base + t] : base + t) : 0;
+        ok = t < nvalid && row >= 0 && row < a.B;
+        s_row[t] = ok ? row : 0;
+        s_ok[t] = ok;
+    }
     if (t < 3) red[t] = 0.0;
-    __syncthreads();
+    const int n_ok = __syncthreads_count(ok);      // rows this tile writes and counts
 
     // stage the tile transposed: rT[j][s]
     for (int idx = t; idx < TS * No; idx += 256) {
         int s = idx / No, j = idx % No;
         double2 v = make_double2(0.0, 0.0);
-        if (s < nvalid) {
+        if (s_ok[s]) {
             const int64_t e = s_row[s] * No + j;
             if (a.r) {
                 v = a.r[e];
@@ -131,7 +139,8 @@ __global__ void __launch_bounds__(256) dense_fp64_kernel(Fp64Args a) {
 
     // ---- phase 1.5: per-sample weights
     if (a.logp_out) {
-        for (int idx = t; idx < nvalid * K; idx += 256) a.logp_out[s_row[idx / K] * K + (idx % K)] = lp[idx];
+        for (int idx = t; idx < nvalid * K; idx += 256)
+            if (s_ok[idx / K]) a.logp_out[s_row[idx / K] * K + (idx % K)] = lp[idx];
         __syncthreads();
     }
     if (t < TS) weights_from_logp(lp + (size_t)t * K, K, a.mode, a.n_top, a.rho, a.flags);
@@ -172,7 +181,7 @@ __global__ void __launch_bounds__(256) dense_fp64_kernel(Fp64Args a) {
                 #pragma unroll
                 for (int u = 0; u < 2; ++u) {
                     const int s = 2 * sp + u;
-                    if (s >= nvalid) continue;
+                    if (!s_ok[s]) continue;
                     const double2 v = u ? acc1[m] : acc0[m];
                     const int64_t o = s_row[s] * N + i;
                     if (a.h_est) a.h_est[o] = v;
@@ -203,7 +212,7 @@ __global__ void __launch_bounds__(256) dense_fp64_kernel(Fp64Args a) {
         if (t == 0) {
             atomicAdd(a.acc + 0, red[0]);
             atomicAdd(a.acc + 1, red[1]);
-            atomicAdd(a.acc + 2, (double)nvalid);
+            atomicAdd(a.acc + 2, (double)n_ok);
         }
     }
     __syncthreads();      // red[], s_row[], the tile and lp are rewritten by the next tile of this CTA
